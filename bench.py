@@ -2,8 +2,10 @@
 """bench.py -- headline benchmark of the ray-query hot path (contract: see DESIGN.md section 6).
 
     python bench.py --gpus N --steps K --warmup W [--workload c3|c1|c2|c4|c5|soup1m|...] [--impl reference]
+                    [--dump-outputs DIR]
 
 A "step" is one pass of the hot path (trq_trace) over one batch of synthetic rays of the named BASELINE config.
+Every timed region runs exactly K steps. --dump-outputs writes what the last timed step returned (see dump_outputs).
 Default workload = C3 (the config the north_star target is quoted on): the ~1.0 M-triangle "meshes" scene (coatball +
 teapot subdivided twice inside the Cornell box) traced with the incoherent diffuse-bounce rays spawned from the
 3840x2160 primary hits. The default run also measures BASELINE.json's other configs (`workloads`: c1, c2, c4, c5).
@@ -59,6 +61,7 @@ PATH_WORKLOADS = {"c2": (1920, 1080), "c3path": (3840, 2160)}
 # algorithmic bytes per ray measured once by the instrumented oracle (DESIGN.md section 4); used only if the
 # oracle cannot be run in this process. Recomputed live on a sample otherwise.
 BYTES_PER_RAY_FALLBACK = {"c3path": 1400.0, "c2bounce": 1094.0, "c1": 700.0, "c2": 1094.0, "c3": 1778.0, "c4": 2887.0, "c5": 9184.0, "soup1m": 7039.0}
+DUMP_BYTES = 60_000_000        # --dump-outputs writes at most this much: kept small enough to store and diff two runs
 
 
 def L_ray_dtype():
@@ -161,7 +164,7 @@ class Work:
             s1 = torch.empty(W * Hh, dtype=torch.int32, device=dev); c1 = torch.zeros(1, dtype=torch.int64, device=dev)
             seed_base = rank << 32
             self.launches_per_step = 2
-            self.h0, self.h1, self.r0, self.r1 = h0, h1, r0, r1
+            self.h0, self.h1, self.r0, self.r1, self.s1 = h0, h1, r0, r1, s1
             scene = self.scene
 
             def step():
@@ -218,7 +221,7 @@ class Work:
 
     def close(self):
         self.scene.close()
-        self.d_rays = self.d_hits = self.h0 = self.h1 = self.r0 = self.r1 = None
+        self.d_rays = self.d_hits = self.h0 = self.h1 = self.r0 = self.r1 = self.s1 = None
 
 
 # ----------------------------------------------------------------------------------------------- clocks
@@ -400,6 +403,38 @@ def parity_on(work, idx, nthreads):
     return {"rays": int(sub.size), "ids_bit_exact": bool(ids_ok), "t_bit_exact": bool(t_ok), "barycentrics_bit_exact": bool(uv_ok)}
 
 
+def dump_outputs(work, out_dir):
+    """--dump-outputs: what the last timed step returned to its caller, as DIR/<struct>_<field>.npy, one file per field of
+    the C-ABI structs (trq_hit; for the wavefronts also the trq_ray batches they produce). Float fields are written as
+    float32, integer fields as float64 (exact). Row i of every file belongs to the ray at position ray_index[i] of the
+    step's batch. A batch too large for DUMP_BYTES is sampled with a fixed seed, so runs with the same arguments write
+    the same rays. The wavefronts compact their bounce wave in a different order every step, so that wave is written in
+    source-pixel order."""
+    import torch
+    from tracer_b200 import layout as L
+    if work.path:
+        order = torch.argsort(work.s1[:work.n1])
+        out = {"ray": (L.ray_dtype, torch.cat([work.r0, work.r1[:work.n1][order]])),
+               "hit": (L.hit_dtype, torch.cat([work.h0, work.h1[:work.n1][order]]))}
+    else:
+        out = {"hit": (L.hit_dtype, work.d_hits)}
+
+    def as_float(a):
+        return a.astype(np.float32 if a.dtype.kind == "f" else np.float64)
+
+    per_ray = 8 + sum(as_float(np.zeros(1, dt)[f]).nbytes for dt, _ in out.values() for f in dt.names)
+    n = work.n
+    m = min(n, DUMP_BYTES // per_ray)
+    idx = np.arange(n) if m == n else np.sort(np.random.default_rng(0).choice(n, m, replace=False))
+    sel = torch.from_numpy(idx).to(work.device)
+    os.makedirs(out_dir, exist_ok=True)
+    for name, (dt, rows) in out.items():
+        rec = rows[sel].cpu().numpy().view(dt).reshape(-1)
+        for f in dt.names:
+            np.save(os.path.join(out_dir, f"{name}_{f}.npy"), as_float(rec[f]))
+    np.save(os.path.join(out_dir, "ray_index.npy"), idx.astype(np.float64))
+
+
 def roofline_of(name, bpr, n, kernel_ms, step_ms, launches_per_step, hbm_peak, peak_src, l2_gbs, prof):
     """achieved = algorithmic bytes per launch / kernel time; peak = the ceiling of the level that bounds the workload.
     prof: this workload's entry of profiles/traffic.json (ncu --set full capture of the same launch), or None."""
@@ -536,8 +571,7 @@ def measure_gather(D, work, steps, rank, world):
     n_common = int(-D.max_over_ranks(-float(work.n)))                      # ranks trace slightly different batch sizes
     g_rays = work.d_rays[:n_common].contiguous()
     any_hit, sort, scene, device = work.any_hit, work.sort, work.scene, work.device
-    g_steps = max(3, min(steps, 50))
-    out = {"unit": UNIT, "steps": g_steps, "rays_per_rank": n_common}
+    out = {"unit": UNIT, "steps": steps, "rays_per_rank": n_common}
     # local truth: this rank's own records, 32-byte and 16-byte form
     own32 = scene.hit(g_rays, any=any_hit, sort=sort).clone()
     own16 = scene.hit(g_rays, any=any_hit, sort=sort, hit16=True).clone()
@@ -550,11 +584,11 @@ def measure_gather(D, work, steps, rank, world):
     g_all = torch.empty((world, n_common, 8), dtype=torch.float32, device=device)
     for _ in range(3):
         D.trace_and_gather(scene, g_rays, g_local, g_all, any=any_hit, sort=sort)
-    ms, _, _ = time_steps(D, lambda: D.trace_and_gather(scene, g_rays, g_local, g_all, any=any_hit, sort=sort), g_steps)
+    ms, _, _ = time_steps(D, lambda: D.trace_and_gather(scene, g_rays, g_local, g_all, any=any_hit, sort=sort), steps)
     g_ms = D.max_over_ranks(ms)
     ok = bool(torch.equal(g_all[rank].view(torch.int32), own32.view(torch.int32)))
     ok = bool(-D.max_over_ranks(-float(ok)) == 1.0)
-    out["nccl_overlapped"] = {"value": round(n_common * world * g_steps / g_ms / 1e3, 2) if ok else None, "ms_per_step": round(g_ms / g_steps, 4),
+    out["nccl_overlapped"] = {"value": round(n_common * world * steps / g_ms / 1e3, 2) if ok else None, "ms_per_step": round(g_ms / steps, 4),
                               "chunks": 4, "own_shard_matches": ok, "how": "dist.trace_and_gather: NCCL all-gather per chunk on a second stream"}
     del g_all, g_local
 
@@ -572,7 +606,7 @@ def measure_gather(D, work, steps, rank, world):
         def gstep():
             hg.trace(g_rays, any=any_hit, sort=sort, hit16=h16)
             res["all"], res["counts"] = hg.wait()
-        ms, _, _ = time_steps(D, gstep, g_steps)
+        ms, _, _ = time_steps(D, gstep, steps)
         published = True
         try:
             hg.status()
@@ -585,9 +619,9 @@ def measure_gather(D, work, steps, rank, world):
         full = full and all(bool(torch.equal(p_all[r, :m].contiguous().view(torch.int32), ref[r].view(torch.int32))) for r in range(world))
         full = bool(-D.max_over_ranks(-float(full)) == 1.0)
         rec = 16 if h16 else 32
-        out[key] = {"value": round(n_common * world * g_steps / p_ms / 1e3, 2) if full else None, "ms_per_step": round(p_ms / g_steps, 4),
+        out[key] = {"value": round(n_common * world * steps / p_ms / 1e3, 2) if full else None, "ms_per_step": round(p_ms / steps, 4),
                     "record_bytes": rec, "peer_store_bytes_per_rank_per_step": int(n_common * (world - 1) * rec),
-                    "nvlink_egress_gbs_per_gpu": round(n_common * (world - 1) * rec / (p_ms / g_steps * 1e-3) / 1e9, 1),
+                    "nvlink_egress_gbs_per_gpu": round(n_common * (world - 1) * rec / (p_ms / steps * 1e-3) / 1e9, 1),
                     "all_slots_match": full}
     hg.close()
     out["value"] = out["trq_hit"]["value"]
@@ -625,22 +659,15 @@ def run_gpu_arm(a):
     # ---- timed region: K steps, device events, barrier + synchronize on both sides
     m = measure(D, work, a.steps, a.warmup, flush, sampler)
     value, total_ms, total_rays = m["value"], m["total_ms"], m["total_rays"]
-    # ---- sustained region: the K-step region of a ~1 ms step is too short for clock sampling to mean much, so the same
-    # step keeps running for >= 0.6 s (clocks sampled throughout) and its throughput is reported beside `value`
-    sustained = None
-    if total_ms < 600.0:
-        k = int(min(20000, max(a.steps, np.ceil(600.0 / max(1e-3, m["ms_per_step"])))))
-        ms, t0, t1 = time_steps(D, work.step, k, flush)
-        sampler.mark("timed region + the same step sustained for >= 0.6 s", t0, t1)
-        s_ms = D.max_over_ranks(ms)
-        sustained = {"value": round(total_rays * k / s_ms / 1e3, 2), "unit": UNIT, "steps": k, "seconds": round(s_ms / 1e3, 3)}
-    unhinted = measure_unhinted(D, work, min(a.steps, 5)) if a.workload == "c5" and sort else None
+    if a.dump_outputs and rank == 0:
+        dump_outputs(work, a.dump_outputs)
+    unhinted = measure_unhinted(D, work, a.steps) if a.workload == "c5" and sort else None
     hit_frac = float((work.hits()[:, 7].view(torch.int32) & 1).float().mean())
     d_hits_ref = work.hits().clone()
 
     # ---- e2e: host (pinned) rays in, host hits out, through the C-ABI host-pointer path
     h_hits = torch.empty((n, 8), dtype=torch.float32).pin_memory()
-    e2e_steps = max(3, min(a.steps, 20))
+    e2e_steps = a.steps
     e2e_extra = {}
     if path:
         W, Hh, n1 = work.W, work.Hh, work.n1
@@ -774,10 +801,9 @@ def run_gpu_arm(a):
                 continue
             try:
                 w = Work(wname, D, rank, local_rank, world)
-                steps = a.steps if wname != "c5" else max(3, min(a.steps, 10))
-                r = measure(D, w, steps, a.warmup)
+                r = measure(D, w, a.steps, a.warmup)
                 e = {"config": WORKLOADS[wname], "query": "any-hit" if w.any_hit else "closest-hit", "value": round(r["value"], 2), "unit": UNIT,
-                     "steps": steps, "ms_per_step": round(r["ms_per_step"], 4), "rays_per_step_per_gpu": int(w.n),
+                     "steps": a.steps, "ms_per_step": round(r["ms_per_step"], 4), "rays_per_step_per_gpu": int(w.n),
                      "scaling": "strong" if wname == "c5" else "weak", "gpu_launches": r["launches"],
                      "ray_ordering": "TRQ_SORT_RAYS" if w.sort else "as given", "kernel_config": w.scene.kernel_config()}
                 if rank == 0:
@@ -791,7 +817,7 @@ def run_gpu_arm(a):
                     e["roofline"] = roofline_of(wname, wb, w.n, r["kernel_ms"], r["ms_per_step"], w.launches_per_step, hbm_peak, peak_src, l2_gbs,
                                                 traffic.get(wname + "_sorted" if w.sort and wname + "_sorted" in traffic else wname))
                 if wname == "c5":
-                    e["unhinted"] = measure_unhinted(D, w, min(steps, 5))
+                    e["unhinted"] = measure_unhinted(D, w, a.steps)
                 extras[wname] = e
                 w.close()
                 del w
@@ -818,8 +844,6 @@ def run_gpu_arm(a):
         "gpu_launches": m["launches"],
         "clocks": clocks,
     }
-    if sustained is not None:
-        line["sustained"] = sustained
     if unhinted is not None:
         line["unhinted"] = unhinted
     line.update(e2e_extra)
@@ -859,7 +883,12 @@ def main():
     ap.add_argument("--no-extra", action="store_true", help="skip BASELINE.json's other configs (workloads: c1, c2, c4, c5)")
     ap.add_argument("--extra-deadline", type=float, default=240.0, help="do not start another extra workload after this many seconds")
     ap.add_argument("--cpu-budget", type=float, default=10.0, help="seconds of CPU work for the cpu_baseline sample")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write the records of the last timed step (rank 0) as DIR/*.npy")
     a = ap.parse_args()
+    if a.steps < 1:
+        ap.error("--steps must be at least 1")
+    if a.impl == "reference" and a.dump_outputs:
+        ap.error("--dump-outputs writes the GPU path's records; the reference arm has none to write")
     if a.impl == "reference":
         return run_reference_arm(a)
     return run_gpu_arm(a)

@@ -30,7 +30,7 @@ def port(built):
 def reference_builder(built):
     from oracle.pyoracle import ReferenceBuilder
     if not ReferenceBuilder.available():
-        pytest.skip("oracle/_ref builder not built (no /root/reference on this box)")
+        pytest.skip("oracle/_ref builder not built (the reference's source is not present); tests/test_restated_golden.py checks its stored answers")
     return ReferenceBuilder()
 
 
@@ -38,7 +38,7 @@ def reference_builder(built):
 def reference_setup(built):
     from oracle.pyoracle import ReferenceSetup
     if not ReferenceSetup.available():
-        pytest.skip("oracle/_ref scene set-up not built (no /root/reference on this box)")
+        pytest.skip("oracle/_ref scene set-up not built (the reference's source is not present); tests/test_restated_golden.py checks its stored answers")
     return ReferenceSetup()
 
 
@@ -46,5 +46,5 @@ def reference_setup(built):
 def reference(built):
     from oracle.pyoracle import Reference
     if not Reference.available():
-        pytest.skip("oracle/_ref not built (no /root/reference on this box)")
+        pytest.skip("oracle/_ref not built (the reference's source is not present); tests/test_restated_golden.py checks its stored answers")
     return Reference()
