@@ -47,7 +47,7 @@ typedef enum trq_status {
     TRQ_OK            =  0,
     TRQ_ERR_INVALID   = -1,   /* NULL / inconsistent argument */
     TRQ_ERR_LAYOUT    = -2,   /* scene arrays violate the reference layout contract (bad index, cycle, ...) */
-    TRQ_ERR_DEPTH     = -3,   /* interior depth > 32: the reference's 32-bit trail cannot represent it (Render.hh:140) */
+    TRQ_ERR_DEPTH     = -3,   /* interior depth > 31: the reference's 32-bit trail cannot represent it (Render.hh:140) */
     TRQ_ERR_CUDA      = -4,   /* a CUDA runtime call failed */
     TRQ_ERR_NOMEM     = -5,
     TRQ_ERR_NO_DEVICE = -6    /* no usable CUDA device: there is no CPU fallback */
@@ -152,8 +152,9 @@ int  trq_version(void);
 const char* trq_last_error_string(void);
 int  trq_device_count(void);
 
-/* Uploads the six arrays to `device`, validates the tree (indices in range, 2N-1 nodes
- * reachable, depth <= 32) and derives the packed traversal layout on the device. */
+/* Uploads the six arrays to `device`, validates the tree (indices in range, every node the root
+ * reaches well linked, interior depth <= 31) and derives the packed traversal layout on the device.
+ * Nodes the root does not reach are kept but never read: not by a trace, not by a refit. */
 int  trq_scene_create(const trq_scene_desc* desc, int device, trq_scene** out);
 /* The same for a scene that already lives on the GPU: every array of `desc` is a DEVICE pointer on `device` (for
  * example bvhList from trq_bvh_build_tree_device). The arrays are copied device to device; validation and numbering
@@ -163,7 +164,8 @@ int  trq_scene_create_device(const trq_scene_desc* desc, int device, trq_scene**
 
 /* Refit after the vertices moved (animated meshes): same topology, new boxes. Triangle leaf boxes are recomputed from
  * the new vertices (min / max of the three, AAPLRenderer.mm:575-589), interior boxes bottom-up as the union of their
- * children (AABB::make, BVH.hh:229-231), the packed layout is derived again; all on the device. triList holds the
+ * children (AABB::make, BVH.hh:229-231), the packed layout is derived again; all on the device. Only nodes the root reaches
+ * are refit (a one-leaf scene's root leaf included). triList holds the
  * scene's nVert vertices: a device pointer, or a host pointer with TRQ_HOST_PTRS. Synchronous: waits for traces in
  * flight, returns when the scene is ready for the next trq_trace. */
 int  trq_scene_update_vertices(trq_scene* scene, const void* triList, uint32_t nVert, uint32_t flags);

@@ -15,6 +15,7 @@ import pytest
 from tracer_b200 import layout as L
 
 from .test_gpu_parity import _torch, assert_hits_equal, gpu_trace
+from .util import refit_on_host
 
 pytestmark = pytest.mark.gpu
 
@@ -121,26 +122,6 @@ def test_build_and_create_without_leaving_the_gpu(built, port):
     scene.close()
 
 
-def _refit_on_host(prim, verts):
-    """The same refit with numpy: triangle leaf boxes from the vertices, interior boxes bottom-up."""
-    from tracer_b200._lib import check, lib
-    nodes = prim.bvhList.copy()
-    tri = np.nonzero(nodes["pType"] == L.TRIANGLE)[0]
-    leaves = np.zeros(prim.nTri, dtype=L.bvh_dtype)
-    check(lib.trq_bvh_build_nodes_triangles(verts.ctypes.data, prim.idxList.ctypes.data, prim.nTri, 0, leaves.ctypes.data), "leaves")
-    nodes["mini"][tri] = leaves["mini"][nodes["pIndex"][tri]]
-    nodes["maxi"][tri] = leaves["maxi"][nodes["pIndex"][tri]]
-    # interior nodes were appended in post-order after the leaves (children before parents), the root moved to 0
-    inner = np.nonzero(nodes["pType"] == L.BVH)[0]
-    for i in list(inner[inner != 0]) + [0]:
-        l, r = nodes["left"][i], nodes["right"][i]
-        nodes["mini"][i] = np.minimum(nodes["mini"][l], nodes["mini"][r])
-        nodes["maxi"][i] = np.maximum(nodes["maxi"][l], nodes["maxi"][r])
-    from tracer_b200.scene import Primitive
-    return Primitive(sphereList=prim.sphereList, squareList=prim.squareList, cubeList=prim.cubeList, triList=verts,
-                     idxList=prim.idxList, bvhList=nodes)
-
-
 def test_refit_after_the_vertices_moved(built, port):
     torch = _torch()
     from tracer_b200 import Scene, harness as H
@@ -150,7 +131,7 @@ def test_refit_after_the_vertices_moved(built, port):
         rng = np.random.default_rng(1)
         verts = prim.triList.copy()
         verts["v"] += (rng.random(verts["v"].shape, dtype=np.float32) - np.float32(0.5)) * np.float32(0.02) * np.abs(verts["v"]).max()
-        moved = _refit_on_host(prim, verts)
+        moved = refit_on_host(prim, verts)
         for how in ("host", "device"):
             scene.update_vertices(verts if how == "host" else torch.from_numpy(verts.view(np.uint8).reshape(-1).copy()).cuda())
             for any_hit in (False, True):

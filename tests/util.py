@@ -31,6 +31,36 @@ def bits(a):
     return np.ascontiguousarray(a).view(np.uint32)
 
 
+def refit_on_host(prim, verts):
+    """trq_scene_update_vertices restated with numpy, for a tree in any node numbering: triangle leaf boxes from the
+    moved vertices (trq_bvh_build_nodes_triangles), then the interior nodes reachable from the root, deepest first, as
+    unions of their children. Nodes the root does not reach keep their boxes. -> the refit Primitive."""
+    from tracer_b200._lib import check, lib
+    nodes = prim.bvhList.copy()
+    depth = np.full(nodes.size, -1, dtype=np.int64)
+    depth[0] = 0
+    stack = [0]
+    while stack:
+        i = stack.pop()
+        if nodes["pType"][i] == L.BVH:
+            for c in (int(nodes["left"][i]), int(nodes["right"][i])):
+                depth[c] = depth[i] + 1
+                stack.append(c)
+    tri = np.nonzero((depth >= 0) & (nodes["pType"] == L.TRIANGLE))[0]
+    boxes = np.zeros(prim.nTri, dtype=L.bvh_dtype)
+    if prim.nTri:
+        check(lib.trq_bvh_build_nodes_triangles(verts.ctypes.data, prim.idxList.ctypes.data, prim.nTri, 0, boxes.ctypes.data), "leaves")
+    nodes["mini"][tri] = boxes["mini"][nodes["pIndex"][tri]]
+    nodes["maxi"][tri] = boxes["maxi"][nodes["pIndex"][tri]]
+    inner = np.nonzero((depth >= 0) & (nodes["pType"] == L.BVH))[0]
+    for i in inner[np.argsort(-depth[inner], kind="stable")]:
+        l, r = nodes["left"][i], nodes["right"][i]
+        nodes["mini"][i] = np.minimum(nodes["mini"][l], nodes["mini"][r])
+        nodes["maxi"][i] = np.maximum(nodes["maxi"][l], nodes["maxi"][r])
+    return Primitive(sphereList=prim.sphereList, squareList=prim.squareList, cubeList=prim.cubeList, triList=verts,
+                     idxList=prim.idxList, bvhList=nodes)
+
+
 def assert_records_match_reference(recs, want, hits=None, sphere_uv_atol=None, where=""):
     """Bit-exact comparison of HitRecord dumps on the rays the reference reports as hit."""
     assert np.array_equal(recs["hit"], want["hit"]), f"{where}: hit flags differ"

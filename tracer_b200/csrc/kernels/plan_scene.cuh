@@ -228,11 +228,13 @@ refs_kernel(const RefBVH* __restrict__ N, uint32_t n, const uint32_t* __restrict
 
 // ---- refit (trq_scene_update_vertices): leaf boxes of triangle leaves from the moved vertices (AAPLRenderer.mm:575-589:
 // min / max of the three vertices), then interior boxes bottom-up as unions of their children (AABB::make, AABB.hh:227-239;
-// BVH.hh:229-231), same arrival-counter climb as above.
+// BVH.hh:229-231), same arrival-counter climb as above. Only nodes the root reaches take part (ref[i] != TRQ_REF_DONE_WORD):
+// trq_scene_create keeps unreachable nodes without checking their fields, and a climb from one of them would give a real
+// interior node a third arrival (merged before one child subtree is refit) or leave the arrays.
 __global__ void __launch_bounds__(256)
-refit_leaves_kernel(RefBVH* N, uint32_t n, const RefVertex* __restrict__ verts, const uint32_t* __restrict__ idx) {
+refit_leaves_kernel(RefBVH* N, const uint32_t* __restrict__ ref, uint32_t n, const RefVertex* __restrict__ verts, const uint32_t* __restrict__ idx) {
     const uint32_t i = blockIdx.x * blockDim.x + threadIdx.x;
-    if (i >= n || N[i].pType != TRQ_TRIANGLE) return;
+    if (i >= n || ref[i] == TRQ_REF_DONE_WORD || N[i].pType != TRQ_TRIANGLE) return;
     const uint32_t p = N[i].pIndex;
     const float* a = verts[idx[3 * (size_t)p]].v; const float* b = verts[idx[3 * (size_t)p + 1]].v; const float* c = verts[idx[3 * (size_t)p + 2]].v;
     for (int k = 0; k < 3; ++k) {
@@ -242,9 +244,9 @@ refit_leaves_kernel(RefBVH* N, uint32_t n, const RefVertex* __restrict__ verts, 
 }
 
 __global__ void __launch_bounds__(256)
-refit_interior_kernel(RefBVH* N, uint32_t n, uint32_t* arrivals) {
+refit_interior_kernel(RefBVH* N, const uint32_t* __restrict__ ref, uint32_t n, uint32_t* arrivals) {
     const uint32_t i = blockIdx.x * blockDim.x + threadIdx.x;
-    if (i >= n || N[i].pType == TRQ_BVH || i == 0) return;
+    if (i >= n || i == 0 || ref[i] == TRQ_REF_DONE_WORD || N[i].pType == TRQ_BVH) return;   // node 0: a one-leaf scene
     uint32_t node = N[i].parent;
     for (int guard = 0; guard < 64; ++guard) {
         __threadfence();

@@ -777,7 +777,7 @@ int trq_scene_create_device(const trq_scene_desc* d, int device, trq_scene** out
 int trq_scene_update_vertices(trq_scene* s, const void* triList, uint32_t nVert, uint32_t flags) {
     if (!s || !triList) return trq::fail(TRQ_ERR_INVALID, "trq_scene_update_vertices: NULL argument");
     if (nVert != s->nVert) return trq::fail(TRQ_ERR_INVALID, "trq_scene_update_vertices: %u vertices, the scene has %u", nVert, s->nVert);
-    if (s->nNode < 2 || nVert == 0) return TRQ_OK;
+    if (nVert == 0) return TRQ_OK;                              // (a one-leaf scene is refit too: its leaf is the root)
     DeviceGuard guard(s->device);
     if (!guard.ok) return trq::fail(TRQ_ERR_CUDA, "cudaSetDevice(%d) failed", s->device);
     TRQ_CUDA(cudaDeviceSynchronize());                           // traces in flight still read the old boxes
@@ -789,8 +789,8 @@ int trq_scene_update_vertices(trq_scene* s, const void* triList, uint32_t nVert,
         if (!mem.alloc(&arrivals, n)) return trq::fail(TRQ_ERR_NOMEM, "trq_scene_update_vertices: out of device memory");
         TRQ_CUDA(cudaMemsetAsync(arrivals, 0, (size_t)n * 4));
         const unsigned grid = (n + 255) / 256;
-        plan::refit_leaves_kernel<<<grid, 256>>>(s->d_bvh, n, s->d_verts, s->d_idx);
-        plan::refit_interior_kernel<<<grid, 256>>>(s->d_bvh, n, arrivals);
+        plan::refit_leaves_kernel<<<grid, 256>>>(s->d_bvh, s->d_ref, n, s->d_verts, s->d_idx);
+        plan::refit_interior_kernel<<<grid, 256>>>(s->d_bvh, s->d_ref, n, arrivals);
         pack_scene_kernel<<<grid, 256>>>(s->d_bvh, s->d_ref, n, s->d_verts, s->d_idx, s->d_spheres, s->d_squares,
                                          s->d_nodes, s->d_tris, s->d_sph, s->d_sq, s->d_triN, s->d_topSoA, s->topStride);
         g_launches += 3;
