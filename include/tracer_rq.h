@@ -321,17 +321,23 @@ int  trq_bvh_build_nodes_triangles(const void* triList, const uint32_t* idxList,
 
 /* BVH::buildTree: on entry bvhList[0..nLeaves) are leaves (capacity >= 2*nLeaves-1 nodes);
  * on return the array holds the reference's final order: root at 0, leaves at 1..nLeaves,
- * interiors after, parent/left/right = final indices. Sequential variant (deterministic). */
+ * interiors after, parent/left/right = final indices. Sequential variant (deterministic).
+ * *maxDepthOut = deepest interior level (root = 0). Interior depth above 31 returns TRQ_ERR_DEPTH
+ * with the complete tree in bvhList and its true depth in *maxDepthOut. */
 int  trq_bvh_build_tree(void* bvhList, uint32_t nLeaves, uint32_t* nNodeOut, uint32_t* maxDepthOut);
 
 /* The same build on the GPU (level-synchronous binned SAH, kernels/bvh_build.cuh): same arguments (HOST array in
- * and out), same node array byte for byte -- splits, child order, numbering, boxes -- except when three or more
- * primitives share one centroid (the reference then falls back to std::sort, whose order of equal keys is
- * unspecified). TRQ_ERR_NO_DEVICE without a GPU (use the host builder). */
+ * and out), same node array byte for byte -- splits, child order, numbering, boxes -- except where the reference's
+ * std::sort fallback sorts equal or NaN keys, whose order std::sort leaves unspecified: three or more primitives
+ * sharing one centroid, or a node spanning an infinite centroid extent (a leaf side at +inf, centroids near
+ * +-FLT_MAX) in which two keys on the split axis are equal or NaN. The GPU sorts such a node stably, NaN last.
+ * Interior depth above 31 returns TRQ_ERR_DEPTH with the complete tree and its true depth, as trq_bvh_build_tree
+ * does. TRQ_ERR_NO_DEVICE without a GPU (use the host builder). */
 int  trq_bvh_build_tree_gpu(void* bvhList, uint32_t nLeaves, int device, uint32_t* nNodeOut, uint32_t* maxDepthOut);
 
 /* The same build with the array in DEVICE memory on `device` (leaves in d_bvhList[0..nLeaves), capacity 2*nLeaves-1
- * nodes; the result replaces them): build -> trq_scene_create_device without the tree ever visiting the host. */
+ * nodes; the result replaces them): build -> trq_scene_create_device without the tree ever visiting the host.
+ * Interior depth above 31 returns TRQ_ERR_DEPTH with the complete tree in d_bvhList and its true depth. */
 int  trq_bvh_build_tree_device(void* d_bvhList, uint32_t nLeaves, int device, uint32_t* nNodeOut, uint32_t* maxDepthOut);
 
 #ifdef __cplusplus

@@ -64,20 +64,25 @@ struct DeviceScope {
 };
 
 // dLeaves[0..n) -> dOut[0..2n-1): root at 0, leaves at 1..n in list order, interiors after (BVH.hh:263-268). n >= 2.
+// Interior depth above 31 still builds, refits and reports the whole tree, then returns TRQ_ERR_DEPTH as the host
+// builder does. *maxDepthOut is written only when the tree is complete; the callers set it to 0 first.
 int build_on_device(const RefBVH* dLeaves, uint32_t n, RefBVH* dOut, int device, uint32_t* maxDepthOut) {
     const uint32_t nNode = 2 * n - 1;
     cudaStream_t st = nullptr;                          // legacy default stream: ordered with the caller's cudaMemcpy / kernels
     PoolScratch mem(device, st);
-    uint32_t *idx, *seg, *flag, *scanT, *tileSums, *leftFalse, *rightTrue, *arrivals, *counters;
+    uint32_t *idx, *seg, *flag, *scanT, *tileSums, *fallbackList, *arrivals, *counters;
+    unsigned long long* sortKeys;                       // the fallback's sort keys; outside it, the two swap lists
     float4* cen;
     BNode *tabA, *tabB;
     const uint32_t cap = n / 2 + 1;
     const uint32_t nTiles = blocks((uint64_t)n + 1, kScanTile);
     bool ok = mem.alloc(&idx, n) && mem.alloc(&seg, n) &&
               mem.alloc(&flag, (size_t)n + 1) && mem.alloc(&scanT, (size_t)n + 1) && mem.alloc(&tileSums, nTiles) &&
-              mem.alloc(&leftFalse, n) && mem.alloc(&rightTrue, n) && mem.alloc(&arrivals, nNode) &&
+              mem.alloc(&sortKeys, n) && mem.alloc(&fallbackList, cap) && mem.alloc(&arrivals, nNode) &&
               mem.alloc(&counters, 4) && mem.alloc(&cen, n) && mem.alloc(&tabA, cap) && mem.alloc(&tabB, cap);
     if (!ok) return trq::fail(TRQ_ERR_NOMEM, "BVH build on the GPU: out of device memory");
+    uint32_t* leftFalse = reinterpret_cast<uint32_t*>(sortKeys);
+    uint32_t* rightTrue = leftFalse + n;
 
     BCK(cudaMemsetAsync(dOut, 0, (size_t)nNode * sizeof(RefBVH), st));
     BCK(cudaMemcpyAsync(dOut + 1, dLeaves, (size_t)n * sizeof(RefBVH), cudaMemcpyDeviceToDevice, st));     // leaves at 1..N (BVH.hh:265)
@@ -92,12 +97,14 @@ int build_on_device(const RefBVH* dLeaves, uint32_t n, RefBVH* dOut, int device,
 
     BNode *cur = tabA, *nxt = tabB;
     uint32_t nActive = 1, depth = 0;
-    uint32_t* nNext = counters;          // [0] next-level count, [1] max depth, [2] level-table overflow
+    uint32_t* nNext = counters;          // [0] next-level count, [1] max depth, [2] level-table overflow, [3] fallback nodes
     uint32_t* dMaxDepth = counters + 1;
     uint32_t* dOverflow = counters + 2;
+    uint32_t* nFallback = counters + 3;
     while (nActive > 0) {
-        if (depth > 64) return trq::fail(TRQ_ERR_DEPTH, "BVH build on the GPU: tree deeper than 64 levels");
-        reset_nodes_kernel<<<blocks(nActive, 256), 256, 0, st>>>(cur, nActive);
+        // every split leaves both children strictly smaller than their parent, so level n - 2 is the deepest possible
+        if (depth > n - 2) return trq::fail(TRQ_ERR_LAYOUT, "BVH build on the GPU: internal: level %u of %u leaves", depth, n);
+        reset_nodes_kernel<<<blocks(nActive, 256), 256, 0, st>>>(cur, nActive, nFallback);
         centroid_bounds_kernel<<<blocks(n, 256), 256, 0, st>>>(idx, seg, cen, n, cur);
         choose_axis_kernel<<<blocks(nActive, 256), 256, 0, st>>>(cur, nActive);
         bucket_kernel<<<blocks(n, 256), 256, 0, st>>>(dLeaves, idx, seg, cen, n, cur);
@@ -106,13 +113,14 @@ int build_on_device(const RefBVH* dLeaves, uint32_t n, RefBVH* dOut, int device,
         scan_tiles_kernel<<<nTiles, 1024, 0, st>>>(flag, scanT, n + 1, tileSums);
         scan_sums_kernel<<<1, 1024, 0, st>>>(tileSums, nTiles);
         scan_add_kernel<<<nTiles, 1024, 0, st>>>(scanT, n + 1, tileSums);
-        midpoint_kernel<<<blocks(nActive, 256), 256, 0, st>>>(cur, nActive, scanT);
+        midpoint_kernel<<<blocks(nActive, 256), 256, 0, st>>>(cur, nActive, scanT, fallbackList, nFallback);
         mispl_kernel<<<blocks(n, 256), 256, 0, st>>>(seg, n, cur, flag, scanT, leftFalse, rightTrue);
         swap_kernel<<<blocks(n, 256), 256, 0, st>>>(seg, n, cur, leftFalse, rightTrue, idx);
+        fallback_sort_kernel<<<kSortBlocks, kSortThreads, 0, st>>>(cur, fallbackList, nFallback, cen, idx, sortKeys);   // exits at once without fallback nodes
         BCK(cudaMemsetAsync(nNext, 0, sizeof(uint32_t), st));
         emit_kernel<<<blocks(nActive, 128), 128, 0, st>>>(cur, nActive, idx, cen, dOut, n, nxt, cap, nNext, dOverflow, dMaxDepth, depth);
         reseg_kernel<<<blocks(n, 256), 256, 0, st>>>(seg, n, cur);
-        launches += 14;
+        launches += 15;
         uint32_t lvl[3] = {0, 0, 0};
         BCK(cudaMemcpyAsync(lvl, counters, sizeof lvl, cudaMemcpyDeviceToHost, st));
         BCK(cudaStreamSynchronize(st));
@@ -143,6 +151,7 @@ int check_device(int device, const char* who) {
 }  // namespace
 
 extern "C" int trq_bvh_build_tree_device(void* d_bvhList, uint32_t nLeaves, int device, uint32_t* nNodeOut, uint32_t* maxDepthOut) {
+    if (maxDepthOut) *maxDepthOut = 0;
     if (!d_bvhList || nLeaves == 0) return trq::fail(TRQ_ERR_INVALID, "trq_bvh_build_tree_device: empty leaf list");
     if (nLeaves > 0x3fffffffu) return trq::fail(TRQ_ERR_INVALID, "trq_bvh_build_tree_device: too many leaves");
     int rc = check_device(device, "trq_bvh_build_tree_device");
@@ -166,6 +175,7 @@ extern "C" int trq_bvh_build_tree_device(void* d_bvhList, uint32_t nLeaves, int 
 }
 
 extern "C" int trq_bvh_build_tree_gpu(void* bvhList, uint32_t nLeaves, int device, uint32_t* nNodeOut, uint32_t* maxDepthOut) {
+    if (maxDepthOut) *maxDepthOut = 0;
     if (!bvhList || nLeaves == 0) return trq::fail(TRQ_ERR_INVALID, "trq_bvh_build_tree_gpu: empty leaf list");
     if (nLeaves > 0x3fffffffu) return trq::fail(TRQ_ERR_INVALID, "trq_bvh_build_tree_gpu: too many leaves");
     const uint32_t n = nLeaves, nNode = 2 * n - 1;

@@ -13,8 +13,12 @@
 //     see the list the reference would have;
 //   * the sequential builder numbers interior nodes in post-order; a subtree over k leaves creates exactly k-1 of
 //     them, so a node's index (N + base + span - 2) and both children's indices are known the moment it is split.
-// The one documented difference: the sort+median fallback (BVH.hh:187-195) fires only when >= 3 primitives share
-// one centroid (0/0 in AABB::relative); std::sort's order of equal keys is unspecified, the GPU keeps list order.
+// A node whose centroids all land in bucket 0 takes the sort + median fallback (BVH.hh:187-195): >= 3 primitives on one
+// centroid (0/0 in AABB::relative), or centroids spanning an infinite extent on the split axis (a +inf centroid from a
+// leaf side at +inf, or centroids near -FLT_MAX and +FLT_MAX: x/inf is 0, inf/inf is NaN). The GPU sorts such a node by
+// (key, list position), which is std::sort's one result when the keys are distinct. The documented difference: with
+// equal keys std::sort's order is unspecified (the GPU keeps list order), and with a NaN key `<` is no strict weak
+// ordering, so the reference's order is not defined at all (the GPU puts NaN after +inf).
 #pragma once
 #include <cfloat>
 #include <cuda_runtime.h>
@@ -39,14 +43,19 @@ struct BNode {                                   // one active subtree (a contig
     float bmin[kBuckets][3], bmax[kBuckets][3];
 };
 
-// ---- float atomics on bit patterns (min/max are exact, so the result is order-independent)
+// ---- float atomics on bit patterns (min/max are exact, so the result is order-independent). They agree with the
+// host's fminf / fmaxf: a NaN is ignored, and the branch is on the sign BIT, so -0.0 takes the unsigned path
+// (v >= 0.0f is true for -0.0, whose bits are INT_MIN as a signed int). -0.0 and +0.0 then order as -0.0 < +0.0,
+// which no decision of the builder can see: they are equal in every comparison and give equal areas.
 __device__ __forceinline__ void atomic_min_f(float* a, float v) {
-    if (v >= 0.0f) atomicMin(reinterpret_cast<int*>(a), __float_as_int(v));
-    else           atomicMax(reinterpret_cast<unsigned int*>(a), __float_as_uint(v));
+    if (v != v) return;
+    if (__float_as_int(v) >= 0) atomicMin(reinterpret_cast<int*>(a), __float_as_int(v));
+    else                        atomicMax(reinterpret_cast<unsigned int*>(a), __float_as_uint(v));
 }
 __device__ __forceinline__ void atomic_max_f(float* a, float v) {
-    if (v >= 0.0f) atomicMax(reinterpret_cast<int*>(a), __float_as_int(v));
-    else           atomicMin(reinterpret_cast<unsigned int*>(a), __float_as_uint(v));
+    if (v != v) return;
+    if (__float_as_int(v) >= 0) atomicMax(reinterpret_cast<int*>(a), __float_as_int(v));
+    else                        atomicMin(reinterpret_cast<unsigned int*>(a), __float_as_uint(v));
 }
 
 // AABB::centroid  AABB.hh:22-25
@@ -85,8 +94,9 @@ init_elements_kernel(const RefBVH* __restrict__ leaves, uint32_t n, uint32_t* id
 }
 
 __global__ void __launch_bounds__(256)
-reset_nodes_kernel(BNode* nodes, uint32_t nNodes) {
+reset_nodes_kernel(BNode* nodes, uint32_t nNodes, uint32_t* nFallback) {
     const uint32_t i = blockIdx.x * blockDim.x + threadIdx.x;
+    if (i == 0) *nFallback = 0;
     if (i >= nNodes) return;
     BNode& nd = nodes[i];
     for (int k = 0; k < 3; ++k) { nd.cmin[k] = FLT_MAX; nd.cmax[k] = -FLT_MAX; }       // AABB default (AABB.hh:8-9)
@@ -287,7 +297,7 @@ scan_add_kernel(uint32_t* __restrict__ out, uint32_t n, const uint32_t* __restri
 
 // K6: partition point per node, fallback detection (BVH.hh:187-195), number of Hoare swaps
 __global__ void __launch_bounds__(256)
-midpoint_kernel(BNode* nodes, uint32_t nNodes, const uint32_t* __restrict__ scanT) {
+midpoint_kernel(BNode* nodes, uint32_t nNodes, const uint32_t* __restrict__ scanT, uint32_t* fallbackList, uint32_t* nFallback) {
     const uint32_t i = blockIdx.x * blockDim.x + threadIdx.x;
     if (i >= nNodes) return;
     BNode& nd = nodes[i];
@@ -299,6 +309,7 @@ midpoint_kernel(BNode* nodes, uint32_t nNodes, const uint32_t* __restrict__ scan
     if (mid <= nd.start || mid >= nd.end) {             // every centroid in one bucket set: sort + median split in the reference
         nd.fallback = 1;
         mid = nd.start + span / 2;
+        fallbackList[atomicAdd(nFallback, 1u)] = i;
     } else {
         nd.nSwap = (mid - nd.start) - (scanT[mid] - scanT[nd.start]);     // misplaced (false) elements left of mid
     }
@@ -337,6 +348,53 @@ swap_kernel(const uint32_t* __restrict__ seg, uint32_t n, const BNode* __restric
     idx[a] = ib; idx[b] = ia;
 }
 
+// K8b: the fallback's std::sort of the node's idx range by centroid[dim] (BVH.hh:187-195), one block per listed node.
+// Keys are (order-preserving bits of the centroid, position in the range): all distinct, so the result is the stable
+// sort. The network is bitonic with every comparator sending the smaller key to the lower index (the first step of each
+// merge pairs mirrored positions): positions past the span act as +inf padding that no comparator moves, so the
+// range is sorted in place in the 64-bit scratch `keys` (indexed by list position, like idx).
+constexpr uint32_t kSortThreads = 512;
+constexpr uint32_t kSortBlocks = 256;
+
+__device__ __forceinline__ uint32_t sort_bits(float f) {       // -0.0 -> +0.0 first: they are equal under `<`
+    const uint32_t u = __float_as_uint(f == 0.0f ? 0.0f : f);
+    return (u & 0x80000000u) ? ~u : (u | 0x80000000u);
+}
+
+__global__ void __launch_bounds__(kSortThreads)
+fallback_sort_kernel(const BNode* __restrict__ nodes, const uint32_t* __restrict__ fallbackList, const uint32_t* __restrict__ nFallback,
+                     const float4* __restrict__ cen, uint32_t* idx, unsigned long long* keys) {
+    const uint32_t count = *nFallback;
+    for (uint32_t f = blockIdx.x; f < count; f += gridDim.x) {
+        const BNode& nd = nodes[fallbackList[f]];
+        const uint32_t start = nd.start, span = nd.end - nd.start, dim = nd.dim;
+        unsigned long long* k = keys + start;
+        for (uint32_t t = threadIdx.x; t < span; t += blockDim.x) {
+            const float4 c = cen[idx[start + t]];
+            k[t] = ((unsigned long long)sort_bits(dim == 0 ? c.x : (dim == 1 ? c.y : c.z)) << 32) | t;
+        }
+        __syncthreads();
+        uint32_t pow2 = 1;
+        while (pow2 < span) pow2 <<= 1;
+        for (uint32_t size = 2; size <= pow2; size <<= 1)
+            for (uint32_t j = size >> 1; j > 0; j >>= 1) {
+                for (uint32_t t = threadIdx.x; t < pow2 / 2; t += blockDim.x) {
+                    const uint32_t lo = 2 * (t & ~(j - 1)) + (t & (j - 1));
+                    const uint32_t hi = j == size >> 1 ? lo ^ (size - 1) : lo + j;
+                    if (hi < span) {
+                        const unsigned long long a = k[lo], b = k[hi];
+                        if (b < a) { k[lo] = b; k[hi] = a; }
+                    }
+                }
+                __syncthreads();
+            }
+        for (uint32_t t = threadIdx.x; t < span; t += blockDim.x) k[t] = idx[start + (uint32_t)k[t]];
+        __syncthreads();
+        for (uint32_t t = threadIdx.x; t < span; t += blockDim.x) idx[start + t] = (uint32_t)k[t];
+        __syncthreads();
+    }
+}
+
 // K9: emit the interior node of every active subtree and open its children for the next level (BVH.hh:222-243)
 __global__ void __launch_bounds__(128)
 emit_kernel(BNode* nodes, uint32_t nNodes, const uint32_t* __restrict__ idx, const float4* __restrict__ cen,
@@ -353,8 +411,10 @@ emit_kernel(BNode* nodes, uint32_t nNodes, const uint32_t* __restrict__ idx, con
     if (span == 2) {                                                // BVH.hh:60-77
         const uint32_t ia = idx[nd.start], ib = idx[nd.start + 1];
         const float4 ca = cen[ia], cb = cen[ib];
-        const float lo[3] = {fminf(ca.x, cb.x), fminf(ca.y, cb.y), fminf(ca.z, cb.z)};
-        const float hi[3] = {fmaxf(ca.x, cb.x), fmaxf(ca.y, cb.y), fmaxf(ca.z, cb.z)};
+        // AABB::make(a, b) grows the default box (AABB.hh:8-9): a component that is NaN in both centroids stays
+        // (FLT_MAX, -FLT_MAX), an extent of -inf rather than NaN, and maximumExtent sees the difference
+        const float lo[3] = {fminf(fminf(FLT_MAX, ca.x), cb.x), fminf(fminf(FLT_MAX, ca.y), cb.y), fminf(fminf(FLT_MAX, ca.z), cb.z)};
+        const float hi[3] = {fmaxf(fmaxf(-FLT_MAX, ca.x), cb.x), fmaxf(fmaxf(-FLT_MAX, ca.y), cb.y), fmaxf(fmaxf(-FLT_MAX, ca.z), cb.z)};
         dim = maximum_extent(lo, hi);
         const float ka = dim == 0 ? ca.x : (dim == 1 ? ca.y : ca.z), kb = dim == 0 ? cb.x : (dim == 1 ? cb.y : cb.z);
         if (ka < kb) { childPre[0] = ia; childPre[1] = ib; } else { childPre[0] = ib; childPre[1] = ia; }
