@@ -170,6 +170,32 @@ int  trq_scene_create_device(const trq_scene_desc* desc, int device, trq_scene**
  * flight, returns when the scene is ready for the next trq_trace. */
 int  trq_scene_update_vertices(trq_scene* scene, const void* triList, uint32_t nVert, uint32_t flags);
 
+/* Rebuild: a new topology from the scene's current geometry, on the device, in place -- for motion a refit cannot follow
+ * (a refit tree's boxes stretch and overlap as the geometry moves, and every ray pays for it). triList: the scene's nVert
+ * new vertices (a device pointer, or a host pointer with TRQ_HOST_PTRS), or NULL (nVert 0) to keep the current ones.
+ *   leaf list  every leaf the root reaches, in ascending bvhList index order. For a tree trq_bvh_build_tree(_gpu/_device)
+ *              made these are nodes 1..n in list order, so rebuilding an unchanged scene reproduces its tree byte for byte.
+ *   leaves     a triangle leaf keeps its pIndex; its box is what trq_bvh_build_nodes_triangles gives for that triangle
+ *              from the current vertices (std::min / std::max of the three, then BVH::buildNode with the identity). Every
+ *              other leaf (sphere, square, cube, unknown pType) keeps pType, pIndex and box: moving those primitives is
+ *              not a rebuild's business. All other fields are zero, as trq_bvh_build_node writes them.
+ *   tree       what trq_bvh_build_tree_gpu makes from that leaf list (the host builder's tree except where its std::sort
+ *              fallback meets equal or NaN keys, see there); nNode becomes 2n - 1, so a scene whose bvhList had
+ *              unreachable nodes shrinks.
+ *   state      afterwards the scene is indistinguishable from one trq_scene_create_device made from the new tree: info
+ *              (maxDepth, topNodes, nNode, bytesReferenceLayout, ...), packed arrays, top-of-tree block, and every launch
+ *              configuration's usability and staged node count. A configuration chosen with trq_scene_set_kernel_config
+ *              is kept if it is still usable; otherwise the scene uses the automatic choice for the new tree.
+ *   failure    TRQ_ERR_DEPTH (new interior depth > 31; the message gives it), TRQ_ERR_NOMEM, TRQ_ERR_INVALID (nVert other
+ *              than the scene's): the scene is exactly as before, vertices included.
+ * Synchronous: waits for work in flight on the device, returns when the scene is ready for the next trq_trace. Hits traced
+ * before a rebuild name leaves (trq_hit.leafNode) by the OLD numbering. trq_scene_update_vertices refits the new tree. */
+int  trq_scene_rebuild(trq_scene* scene, const void* triList, uint32_t nVert, uint32_t flags);
+
+/* Copies the scene's node array (trq_scene_info_t.nNode nodes, 64 B each) to `out`: a device pointer on the scene's
+ * device, or a host pointer with TRQ_HOST_PTRS. Synchronous. */
+int  trq_scene_copy_bvh(const trq_scene* scene, void* out, uint32_t flags);
+
 int  trq_scene_destroy(trq_scene* scene);
 
 /* Scene arrays and builder scratch come from a per-device memory pool that keeps what it is given back (so that
@@ -318,6 +344,19 @@ int  trq_bvh_build_node(const float box_min[3], const float box_max[3], const fl
  * identity model, pType = Triangle, pIndex = pIndexBase + i. Writes nTri 64-B nodes. */
 int  trq_bvh_build_nodes_triangles(const void* triList, const uint32_t* idxList, uint32_t nTri,
                                    uint32_t pIndexBase, void* nodes_out);
+
+/* The same leaves built on the GPU, bit for bit (NaN, signed zeros and infinities included): device pointers on `device`,
+ * asynchronous on `stream` (a cudaStream_t, NULL = default stream). nTri == 0 is a no-op. With the vertices already on
+ * the GPU, this + trq_bvh_build_tree_device + trq_scene_create_device make a scene without the host touching an array. */
+int  trq_bvh_build_nodes_triangles_device(const void* d_triList, const uint32_t* d_idxList, uint32_t nTri,
+                                          uint32_t pIndexBase, void* d_nodes_out, int device, void* stream);
+
+/* BVH::buildNode on the GPU for n spheres / squares / cubes (pType TRQ_SPHERE / TRQ_SQUARE / TRQ_CUBE; anything else is
+ * TRQ_ERR_INVALID) given in their reference layout (272 / 272 / 240 B): leaf k = trq_bvh_build_node(list[k].box.mini,
+ * list[k].box.maxi, list[k].model, pType, pIndexBase + k), bit for bit -- the box is boundingBOX for Sphere and Square,
+ * box for Cube (AAPLRenderer.mm:454-468). Device pointers, asynchronous on `stream`; n == 0 is a no-op. */
+int  trq_bvh_build_nodes_device(int32_t pType, const void* d_list, uint32_t n, uint32_t pIndexBase,
+                                void* d_nodes_out, int device, void* stream);
 
 /* BVH::buildTree: on entry bvhList[0..nLeaves) are leaves (capacity >= 2*nLeaves-1 nodes);
  * on return the array holds the reference's final order: root at 0, leaves at 1..nLeaves,

@@ -49,10 +49,10 @@ class Camera(C.Structure):
 # every symbol include/*.h declares; tests/test_abi.py checks the library exports all of them
 ABI_SYMBOLS = [
     "trq_version", "trq_last_error_string", "trq_device_count",
-    "trq_scene_create", "trq_scene_create_device", "trq_scene_update_vertices", "trq_scene_destroy", "trq_device_trim", "trq_scene_info",
+    "trq_scene_create", "trq_scene_create_device", "trq_scene_update_vertices", "trq_scene_rebuild", "trq_scene_copy_bvh", "trq_scene_destroy", "trq_device_trim", "trq_scene_info",
     "trq_kernel_config_count", "trq_kernel_config_name", "trq_scene_set_kernel_config", "trq_scene_kernel_config",
     "trq_trace", "trq_host_sync", "trq_expand_hits", "trq_launch_count", "trq_profile_enable", "trq_profile_read", "trq_probe_bandwidth",
-    "trq_bvh_build_node", "trq_bvh_build_nodes_triangles", "trq_bvh_build_tree", "trq_bvh_build_tree_gpu", "trq_bvh_build_tree_device",
+    "trq_bvh_build_node", "trq_bvh_build_nodes_triangles", "trq_bvh_build_nodes_triangles_device", "trq_bvh_build_nodes_device", "trq_bvh_build_tree", "trq_bvh_build_tree_gpu", "trq_bvh_build_tree_device",
     "trq_cast_rays", "trq_trace_indirect", "trq_spawn_bounce", "trq_spawn_shadow", "trq_spawn_bounce_rng", "trq_spawn_shadow_rng", "trq_rng_frame_begin",
     "trq_mgpu_create", "trq_mgpu_device_count", "trq_mgpu_scene", "trq_mgpu_shard", "trq_mgpu_trace", "trq_mgpu_destroy",
     "trq_gather_create", "trq_gather_connect", "trq_trace_gather", "trq_gather_wait", "trq_gather_status", "trq_gather_destroy",
@@ -72,6 +72,8 @@ lib.trq_launch_count.restype = _u64
 lib.trq_scene_create.argtypes = [C.POINTER(SceneDesc), C.c_int, C.POINTER(_vp)]
 lib.trq_scene_create_device.argtypes = [C.POINTER(SceneDesc), C.c_int, C.POINTER(_vp)]
 lib.trq_scene_update_vertices.argtypes = [_vp, _vp, _u32, _u32]
+lib.trq_scene_rebuild.argtypes = [_vp, _vp, _u32, _u32]
+lib.trq_scene_copy_bvh.argtypes = [_vp, _vp, _u32]
 lib.trq_scene_destroy.argtypes = [_vp]
 lib.trq_device_trim.argtypes = [C.c_int]
 lib.trq_scene_info.argtypes = [_vp, C.POINTER(SceneInfo)]
@@ -109,6 +111,8 @@ lib.trq_spawn_bounce_rng.argtypes = [_vp, _vp, _vp, _u64, _vp, _u64, _vp, _vp, _
 lib.trq_spawn_shadow_rng.argtypes = [_vp, _vp, _vp, _u64, _vp, _u64, _vp, _vp, _u32, _u32, _vp, _vp, _vp, _vp]
 lib.trq_bvh_build_node.argtypes = [_vp, _vp, _vp, _i32, _u32, _vp]
 lib.trq_bvh_build_nodes_triangles.argtypes = [_vp, _vp, _u32, _u32, _vp]
+lib.trq_bvh_build_nodes_triangles_device.argtypes = [_vp, _vp, _u32, _u32, _vp, C.c_int, _vp]
+lib.trq_bvh_build_nodes_device.argtypes = [_i32, _vp, _u32, _u32, _vp, C.c_int, _vp]
 lib.trq_bvh_build_tree.argtypes = [_vp, _u32, C.POINTER(_u32), C.POINTER(_u32)]
 lib.trq_bvh_build_tree_gpu.argtypes = [_vp, _u32, C.c_int, C.POINTER(_u32), C.POINTER(_u32)]
 lib.trq_bvh_build_tree_device.argtypes = [_vp, _u32, C.c_int, C.POINTER(_u32), C.POINTER(_u32)]

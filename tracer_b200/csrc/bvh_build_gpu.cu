@@ -1,9 +1,11 @@
 // tracer_b200/csrc/bvh_build_gpu.cu -- BVH::buildTree (BVH.hh:246-269) on the GPU.
 //   trq_bvh_build_tree_device   leaves and result in DEVICE memory (feeds trq_scene_create_device without a host round trip)
 //   trq_bvh_build_tree_gpu      the same build for a HOST array (copy in, build, copy out)
+//   trq_bvh_build_nodes_triangles_device / trq_bvh_build_nodes_device   BVH::buildNode per primitive (kernels/leaves.cuh)
 // Orchestrates the level-synchronous kernels of kernels/bvh_build.cuh; same node array as trq_bvh_build_tree.
 #include <cuda_runtime.h>
 
+#include <cstddef>
 #include <cstdio>
 #include <cstring>
 #include <map>
@@ -12,9 +14,11 @@
 
 #include "../../include/tracer_rq.h"
 #include "host/error.h"
+#include "host/gpu_build.h"
 #include "host/layout.h"
 #include "host/scratch.h"
 #include "kernels/bvh_build.cuh"
+#include "kernels/leaves.cuh"
 
 using namespace trq;
 using namespace trq::gpubuild;
@@ -63,10 +67,11 @@ struct DeviceScope {
     ~DeviceScope() { if (prev >= 0) cudaSetDevice(prev); }
 };
 
-// dLeaves[0..n) -> dOut[0..2n-1): root at 0, leaves at 1..n in list order, interiors after (BVH.hh:263-268). n >= 2.
+}  // namespace
+
 // Interior depth above 31 still builds, refits and reports the whole tree, then returns TRQ_ERR_DEPTH as the host
 // builder does. *maxDepthOut is written only when the tree is complete; the callers set it to 0 first.
-int build_on_device(const RefBVH* dLeaves, uint32_t n, RefBVH* dOut, int device, uint32_t* maxDepthOut) {
+int trq::build_on_device(const RefBVH* dLeaves, uint32_t n, RefBVH* dOut, int device, uint32_t* maxDepthOut) {
     const uint32_t nNode = 2 * n - 1;
     cudaStream_t st = nullptr;                          // legacy default stream: ordered with the caller's cudaMemcpy / kernels
     PoolScratch mem(device, st);
@@ -141,6 +146,26 @@ int build_on_device(const RefBVH* dLeaves, uint32_t n, RefBVH* dOut, int device,
     return TRQ_OK;
 }
 
+// flag -> exclusive scan (the builder's scan kernels) -> scatter
+int trq::reachable_leaves_on_device(const RefBVH* bvh, const uint32_t* ref, uint32_t nNode, uint32_t nLeaf, const RefVertex* verts,
+                                    const uint32_t* idx, PoolScratch& mem, RefBVH** leavesOut) {
+    cudaStream_t st = nullptr;
+    const uint32_t nTiles = blocks((uint64_t)nNode + 1, kScanTile);
+    uint32_t *flag, *pos, *tileSums;
+    if (!(mem.alloc(&flag, (size_t)nNode + 1) && mem.alloc(&pos, (size_t)nNode + 1) && mem.alloc(&tileSums, nTiles) && mem.alloc(leavesOut, nLeaf)))
+        return trq::fail(TRQ_ERR_NOMEM, "trq_scene_rebuild: out of device memory");
+    leaves::reachable_leaf_flag_kernel<<<blocks((uint64_t)nNode + 1, 256), 256, 0, st>>>(bvh, ref, nNode, flag);
+    scan_tiles_kernel<<<nTiles, 1024, 0, st>>>(flag, pos, nNode + 1, tileSums);
+    scan_sums_kernel<<<1, 1024, 0, st>>>(tileSums, nTiles);
+    scan_add_kernel<<<nTiles, 1024, 0, st>>>(pos, nNode + 1, tileSums);
+    leaves::reachable_leaf_scatter_kernel<<<blocks(nNode, 256), 256, 0, st>>>(bvh, flag, pos, nNode, verts, idx, *leavesOut);
+    trq::note_launches(5);
+    BCK(cudaGetLastError());
+    return TRQ_OK;
+}
+
+namespace {
+
 int check_device(int device, const char* who) {
     int ndev = 0;
     if (cudaGetDeviceCount(&ndev) != cudaSuccess || ndev <= 0) { cudaGetLastError(); return trq::fail(TRQ_ERR_NO_DEVICE, "%s: no CUDA device (use trq_bvh_build_tree on the host)", who); }
@@ -201,4 +226,41 @@ extern "C" int trq_bvh_build_tree_gpu(void* bvhList, uint32_t nLeaves, int devic
     if (rc != TRQ_OK && rc != TRQ_ERR_DEPTH) return rc;
     BCK(cudaMemcpy(host, dOut, (size_t)nNode * sizeof(RefBVH), cudaMemcpyDeviceToHost));
     return rc;
+}
+
+extern "C" int trq_bvh_build_nodes_triangles_device(const void* d_triList, const uint32_t* d_idxList, uint32_t nTri, uint32_t pIndexBase,
+                                                    void* d_nodes_out, int device, void* stream) {
+    if (nTri == 0) return TRQ_OK;
+    if (!d_triList || !d_idxList || !d_nodes_out) return trq::fail(TRQ_ERR_INVALID, "trq_bvh_build_nodes_triangles_device: NULL argument");
+    int rc = check_device(device, "trq_bvh_build_nodes_triangles_device");
+    if (rc != TRQ_OK) return rc;
+    DeviceScope scope(device);
+    if (!scope.ok) return trq::fail(TRQ_ERR_CUDA, "cudaSetDevice(%d) failed", device);
+    leaves::triangle_leaves_kernel<<<blocks(nTri, 256), 256, 0, (cudaStream_t)stream>>>((const RefVertex*)d_triList, d_idxList, nTri,
+                                                                                     pIndexBase, (RefBVH*)d_nodes_out);
+    trq::note_launches(1);
+    BCK(cudaGetLastError());
+    return TRQ_OK;
+}
+
+extern "C" int trq_bvh_build_nodes_device(int32_t pType, const void* d_list, uint32_t n, uint32_t pIndexBase, void* d_nodes_out,
+                                          int device, void* stream) {
+    uint32_t stride, modelAt, boxAt;                      // where BVH::buildNode's arguments sit in each record
+    switch (pType) {
+        case TRQ_SPHERE: stride = sizeof(RefSphere); modelAt = offsetof(RefSphere, model); boxAt = offsetof(RefSphere, boundingBOX); break;
+        case TRQ_SQUARE: stride = sizeof(RefSquare); modelAt = offsetof(RefSquare, model); boxAt = offsetof(RefSquare, boundingBOX); break;
+        case TRQ_CUBE:   stride = sizeof(RefCube);   modelAt = offsetof(RefCube, model);   boxAt = offsetof(RefCube, box); break;
+        default: return trq::fail(TRQ_ERR_INVALID, "trq_bvh_build_nodes_device: pType %d is not TRQ_SPHERE, TRQ_SQUARE or TRQ_CUBE", pType);
+    }
+    if (n == 0) return TRQ_OK;
+    if (!d_list || !d_nodes_out) return trq::fail(TRQ_ERR_INVALID, "trq_bvh_build_nodes_device: NULL argument");
+    int rc = check_device(device, "trq_bvh_build_nodes_device");
+    if (rc != TRQ_OK) return rc;
+    DeviceScope scope(device);
+    if (!scope.ok) return trq::fail(TRQ_ERR_CUDA, "cudaSetDevice(%d) failed", device);
+    leaves::primitive_leaves_kernel<<<blocks(n, 256), 256, 0, (cudaStream_t)stream>>>((const uint8_t*)d_list, n, stride, modelAt, boxAt, pType,
+                                                                                   pIndexBase, (RefBVH*)d_nodes_out);
+    trq::note_launches(1);
+    BCK(cudaGetLastError());
+    return TRQ_OK;
 }

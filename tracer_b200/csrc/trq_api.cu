@@ -15,10 +15,12 @@
 #include <cstring>
 #include <mutex>
 #include <new>
+#include <utility>
 #include <vector>
 
 #include "../../include/tracer_rq.h"
 #include "host/error.h"
+#include "host/gpu_build.h"
 #include "host/layout.h"
 #include "host/scratch.h"
 #include "kernels/plan_scene.cuh"
@@ -126,6 +128,7 @@ struct trq_scene {
     float4* d_topSoA = nullptr;
     uint32_t* d_ref = nullptr;    // packed reference of every bvhList node (kept for refits)
     uint32_t nNode = 0, nVert = 0, topStride = 0;
+    uint32_t listSphere = 0, listSquare = 0, listCube = 0, listTri = 0;   // records in the arrays (info counts leaves)
     SceneDev dev{};
     uint32_t stackDepth = 1;
     bool largeTree = false;       // packed tree > 2 x L2: incoherent batches are worth ordering (automatic TRQ_SORT_RAYS)
@@ -135,6 +138,7 @@ struct trq_scene {
     struct CfgState { uint32_t topCount = 0, stackDepth = 0; size_t smem = 0; int blocksPerSM[2][2] = {}; bool usable = false; };
     CfgState cfg[kNumCfgs];
     int defaultCfg = 0, autoCfg = 0;
+    bool userCfg = false;         // defaultCfg was chosen with trq_scene_set_kernel_config (kept by a rebuild while usable)
     // stream-ordered scratch for TRQ_SORT_RAYS: a private pool that keeps its memory across synchronisations
     // (the device's default pool hands it back at every sync and re-maps 64 MB on the next sorted launch)
     cudaMemPool_t scratchPool = nullptr;     // the per-device pool (not owned)
@@ -548,51 +552,9 @@ int check_desc(const trq_scene_desc* d, trq_scene** out, const char* who) {
     return TRQ_OK;
 }
 
-// The part of scene creation that is the same for host and device input: the six reference arrays are resident
-// (s->d_*), every node has its packed reference in s->d_ref, `info` holds the counts. Allocates and derives the packed
-// layout on the device and sizes the launch configurations.
-int finish_scene(trq_scene* s, const trq_scene_desc* d, trq_scene_info_t info, uint32_t nSqLeaf, uint32_t rootRef,
-                 const float rootMin[3], const float rootMax[3]) {
-    const int device = s->device;
-    StageTimer tm;
-    const size_t nodeBytes = (size_t)info.nInterior * 64, triBytes = (size_t)info.nTri * 16 * TRQ_TRI_STRIDE, sphBytes = (size_t)info.nSphere * 32;
-    const size_t sqBytes = (size_t)nSqLeaf * 16 * TRQ_SQ_STRIDE;
-    if (nodeBytes && pool_malloc((void**)&s->d_nodes, nodeBytes) != cudaSuccess) return trq::fail(TRQ_ERR_CUDA, "cudaMalloc(nodes %zu B) failed", nodeBytes);
-    if (triBytes && pool_malloc((void**)&s->d_tris, triBytes) != cudaSuccess) return trq::fail(TRQ_ERR_CUDA, "cudaMalloc(tris %zu B) failed", triBytes);
-    if (sphBytes && pool_malloc((void**)&s->d_sph, sphBytes) != cudaSuccess) return trq::fail(TRQ_ERR_CUDA, "cudaMalloc(spheres %zu B) failed", sphBytes);
-    if (sqBytes && pool_malloc((void**)&s->d_sq, sqBytes) != cudaSuccess) return trq::fail(TRQ_ERR_CUDA, "cudaMalloc(squares %zu B) failed", sqBytes);
-    const size_t triNBytes = (size_t)info.nTri * 64;
-    if (triNBytes && pool_malloc((void**)&s->d_triN, triNBytes) != cudaSuccess) return trq::fail(TRQ_ERR_CUDA, "cudaMalloc(triangle normals %zu B) failed", triNBytes);
-    if (info.topNodes && pool_malloc((void**)&s->d_topSoA, (size_t)info.topNodes * 64) != cudaSuccess) return trq::fail(TRQ_ERR_CUDA, "cudaMalloc(top-of-tree block) failed");
-    if (pool_malloc((void**)&s->d_queues, kQueueRing * sizeof(QueueHead)) != cudaSuccess) return trq::fail(TRQ_ERR_CUDA, "cudaMalloc(queue heads) failed");
-    if (cudaMemsetAsync(s->d_queues, 0, kQueueRing * sizeof(QueueHead), nullptr) != cudaSuccess) return trq::fail(TRQ_ERR_CUDA, "cudaMemset(queue heads) failed");
-
-    s->nNode = d->nNode; s->nVert = d->nVert; s->topStride = info.topNodes;
-    TRQ_LAP(tm, "allocate packed arrays");
-    {
-        const unsigned block = 256, grid = (d->nNode + block - 1) / block;
-        pack_scene_kernel<<<grid, block>>>(s->d_bvh, s->d_ref, d->nNode, s->d_verts, s->d_idx, s->d_spheres, s->d_squares,
-                                           s->d_nodes, s->d_tris, s->d_sph, s->d_sq, s->d_triN, s->d_topSoA, info.topNodes);
-        g_launches++;
-        cudaError_t e = cudaDeviceSynchronize();
-        if (e != cudaSuccess) return trq::fail(TRQ_ERR_CUDA, "pack_scene_kernel failed: %s", cudaGetErrorString(e));
-    }
-
-    TRQ_LAP(tm, "pack_scene_kernel");
-    s->dev.spheres = s->d_spheres; s->dev.squares = s->d_squares; s->dev.cubes = s->d_cubes;
-    s->dev.verts = s->d_verts; s->dev.idx = s->d_idx; s->dev.bvh = s->d_bvh;
-    s->dev.topSoA = s->d_topSoA; s->dev.topStride = info.topNodes;
-    s->dev.nodes = s->d_nodes; s->dev.tris = s->d_tris; s->dev.sph = s->d_sph; s->dev.sq = s->d_sq; s->dev.triN = s->d_triN;
-    s->dev.rootRef = rootRef;
-    for (int k = 0; k < 3; ++k) { s->dev.rootMin[k] = rootMin[k]; s->dev.rootMax[k] = rootMax[k]; }
-    s->dev.nNode = d->nNode;
-    s->stackDepth = info.maxDepth + 1;
-    // (a leaf of unknown pType, which dispatches to `default: break`, also selects the general kernels)
-    s->leaves = info.nLeaf == info.nTri ? LEAVES_TRI : (info.nLeaf == info.nTri + info.nSphere ? LEAVES_TRI_SPHERE : LEAVES_ALL);
-    s->scratchPool = trq::scratch_pool(device);                // TRQ_SORT_RAYS scratch: stream-ordered, kept between launches
-    if (!s->scratchPool) return trq::fail(TRQ_ERR_CUDA, "cudaMemPoolCreate failed");
-    TRQ_LAP(tm, "scratch pool");
-    // launch configurations: per-CTA shared memory = staged top-of-tree nodes + far-child stack + cold per-ray words
+// Launch configurations for the scene's tree (s->stackDepth, s->leaves set): per-CTA shared memory = staged top-of-tree nodes +
+// far-child stack + cold per-ray words, resident CTAs per SM, usability; and the automatic choice s->autoCfg.
+int size_configs(trq_scene* s, const trq_scene_info_t& info) {
     for (int c = 0; c < kNumCfgs; ++c) {
         const KernelCfg& K = kCfgs[c];
         trq_scene::CfgState& cs = s->cfg[c];
@@ -626,13 +588,65 @@ int finish_scene(trq_scene* s, const trq_scene_desc* d, trq_scene_info_t info, u
         }
     }
     if (!s->cfg[0].usable) return trq::fail(TRQ_ERR_CUDA, "trace_packed_kernel does not fit on an SM (smem %zu)", s->cfg[0].smem);
-    TRQ_LAP(tm, "kernel configurations");
     // Staging pays when the staged block IS the tree (C1: +2-15 %); with the leaf-specialised kernels it no longer does when
     // only the top levels fit (C2 / the reference's Cornell mix: -3 to -6 %), and it loses clearly on 1 M+ triangle scenes
     // (profiles/r02_top_of_tree_experiment.txt): chosen only for trees that fit whole.
     s->autoCfg = 0;
     for (int c = 1; c < kNumCfgs; ++c)
         if (kCfgs[c].top && s->cfg[c].usable && info.nInterior <= s->cfg[c].topCount) { s->autoCfg = c; break; }
+    return TRQ_OK;
+}
+
+// The part of scene creation that is the same for host and device input: the six reference arrays are resident
+// (s->d_*), every node has its packed reference in s->d_ref, `info` holds the counts. Allocates and derives the packed
+// layout on the device and sizes the launch configurations.
+int finish_scene(trq_scene* s, const trq_scene_desc* d, trq_scene_info_t info, uint32_t nSqLeaf, uint32_t rootRef,
+                 const float rootMin[3], const float rootMax[3]) {
+    const int device = s->device;
+    StageTimer tm;
+    const size_t nodeBytes = (size_t)info.nInterior * 64, triBytes = (size_t)info.nTri * 16 * TRQ_TRI_STRIDE, sphBytes = (size_t)info.nSphere * 32;
+    const size_t sqBytes = (size_t)nSqLeaf * 16 * TRQ_SQ_STRIDE;
+    if (nodeBytes && pool_malloc((void**)&s->d_nodes, nodeBytes) != cudaSuccess) return trq::fail(TRQ_ERR_CUDA, "cudaMalloc(nodes %zu B) failed", nodeBytes);
+    if (triBytes && pool_malloc((void**)&s->d_tris, triBytes) != cudaSuccess) return trq::fail(TRQ_ERR_CUDA, "cudaMalloc(tris %zu B) failed", triBytes);
+    if (sphBytes && pool_malloc((void**)&s->d_sph, sphBytes) != cudaSuccess) return trq::fail(TRQ_ERR_CUDA, "cudaMalloc(spheres %zu B) failed", sphBytes);
+    if (sqBytes && pool_malloc((void**)&s->d_sq, sqBytes) != cudaSuccess) return trq::fail(TRQ_ERR_CUDA, "cudaMalloc(squares %zu B) failed", sqBytes);
+    const size_t triNBytes = (size_t)info.nTri * 64;
+    if (triNBytes && pool_malloc((void**)&s->d_triN, triNBytes) != cudaSuccess) return trq::fail(TRQ_ERR_CUDA, "cudaMalloc(triangle normals %zu B) failed", triNBytes);
+    if (info.topNodes && pool_malloc((void**)&s->d_topSoA, (size_t)info.topNodes * 64) != cudaSuccess) return trq::fail(TRQ_ERR_CUDA, "cudaMalloc(top-of-tree block) failed");
+    if (!s->d_queues) {                                        // (a rebuild's staging scene borrows the scene's heads)
+        if (pool_malloc((void**)&s->d_queues, kQueueRing * sizeof(QueueHead)) != cudaSuccess) return trq::fail(TRQ_ERR_CUDA, "cudaMalloc(queue heads) failed");
+        if (cudaMemsetAsync(s->d_queues, 0, kQueueRing * sizeof(QueueHead), nullptr) != cudaSuccess) return trq::fail(TRQ_ERR_CUDA, "cudaMemset(queue heads) failed");
+    }
+
+    s->nNode = d->nNode; s->nVert = d->nVert; s->topStride = info.topNodes;
+    s->listSphere = d->nSphere; s->listSquare = d->nSquare; s->listCube = d->nCube; s->listTri = d->nTri;
+    TRQ_LAP(tm, "allocate packed arrays");
+    {
+        const unsigned block = 256, grid = (d->nNode + block - 1) / block;
+        pack_scene_kernel<<<grid, block>>>(s->d_bvh, s->d_ref, d->nNode, s->d_verts, s->d_idx, s->d_spheres, s->d_squares,
+                                           s->d_nodes, s->d_tris, s->d_sph, s->d_sq, s->d_triN, s->d_topSoA, info.topNodes);
+        g_launches++;
+        cudaError_t e = cudaDeviceSynchronize();
+        if (e != cudaSuccess) return trq::fail(TRQ_ERR_CUDA, "pack_scene_kernel failed: %s", cudaGetErrorString(e));
+    }
+
+    TRQ_LAP(tm, "pack_scene_kernel");
+    s->dev.spheres = s->d_spheres; s->dev.squares = s->d_squares; s->dev.cubes = s->d_cubes;
+    s->dev.verts = s->d_verts; s->dev.idx = s->d_idx; s->dev.bvh = s->d_bvh;
+    s->dev.topSoA = s->d_topSoA; s->dev.topStride = info.topNodes;
+    s->dev.nodes = s->d_nodes; s->dev.tris = s->d_tris; s->dev.sph = s->d_sph; s->dev.sq = s->d_sq; s->dev.triN = s->d_triN;
+    s->dev.rootRef = rootRef;
+    for (int k = 0; k < 3; ++k) { s->dev.rootMin[k] = rootMin[k]; s->dev.rootMax[k] = rootMax[k]; }
+    s->dev.nNode = d->nNode;
+    s->stackDepth = info.maxDepth + 1;
+    // (a leaf of unknown pType, which dispatches to `default: break`, also selects the general kernels)
+    s->leaves = info.nLeaf == info.nTri ? LEAVES_TRI : (info.nLeaf == info.nTri + info.nSphere ? LEAVES_TRI_SPHERE : LEAVES_ALL);
+    s->scratchPool = trq::scratch_pool(device);                // TRQ_SORT_RAYS scratch: stream-ordered, kept between launches
+    if (!s->scratchPool) return trq::fail(TRQ_ERR_CUDA, "cudaMemPoolCreate failed");
+    TRQ_LAP(tm, "scratch pool");
+    int rc = size_configs(s, info);
+    if (rc != TRQ_OK) return rc;
+    TRQ_LAP(tm, "kernel configurations");
     s->defaultCfg = s->autoCfg;
 
     info.bytesReferenceLayout = (uint64_t)d->nSphere * sizeof(RefSphere) + (uint64_t)d->nSquare * sizeof(RefSquare) +
@@ -673,6 +687,45 @@ const char* plan_error_text(uint32_t code) {
         case plan::ERR_UNREACHABLE: return "nodes not reachable from the root";
         default: return "unknown";
     }
+}
+
+// The device half of scene creation, shared by trq_scene_create_device and trq_scene_rebuild: s->d_bvh (d->nNode nodes),
+// s->d_idx and the other arrays are resident. The planning kernels (kernels/plan_scene.cuh) validate the tree and number it
+// into a new s->d_ref, 128 bytes of counters come back, and finish_scene derives the packed layout.
+int plan_and_finish(trq_scene* s, const trq_scene_desc* d, const char* who) {
+    StageTimer tm;
+    const uint32_t n = d->nNode;
+    if (pool_malloc((void**)&s->d_ref, (size_t)n * sizeof(uint32_t)) != cudaSuccess) return trq::fail(TRQ_ERR_CUDA, "%s: cudaMalloc(refs) failed", who);
+    plan::PlanInfo hostInfo;
+    {
+        trq::PoolScratch mem(s->device, nullptr);
+        plan::Counts* cnt; uint32_t *leafTotal, *arrivals, *pre, *topPos, *sortedPre; plan::PlanInfo* dInfo;
+        if (!(mem.alloc(&cnt, n) && mem.alloc(&leafTotal, n) && mem.alloc(&arrivals, n) && mem.alloc(&pre, n) && mem.alloc(&topPos, n) &&
+              mem.alloc(&sortedPre, 2048) && mem.alloc(&dInfo, 1)))
+            return trq::fail(TRQ_ERR_NOMEM, "%s: out of device memory", who);
+        cudaMemsetAsync(arrivals, 0, (size_t)n * 4); cudaMemsetAsync(topPos, 0, (size_t)n * 4);
+        cudaMemsetAsync(cnt, 0, (size_t)n * sizeof(plan::Counts)); cudaMemsetAsync(leafTotal, 0, (size_t)n * 4);
+        cudaMemsetAsync(dInfo, 0, sizeof(plan::PlanInfo)); cudaMemsetAsync(s->d_ref, 0xff, (size_t)n * 4);
+        const unsigned grid = (n + 255) / 256;
+        plan::validate_kernel<<<grid, 256>>>(s->d_bvh, n, d->nSphere, d->nSquare, d->nCube, d->nTri, d->nVert, s->d_idx, dInfo);
+        plan::counts_kernel<<<grid, 256>>>(s->d_bvh, n, cnt, leafTotal, arrivals);
+        plan::number_kernel<<<grid, 256>>>(s->d_bvh, n, cnt, leafTotal, s->d_ref, pre, dInfo);
+        plan::top_block_kernel<<<1, 1024>>>(s->d_bvh, n, pre, topPos, sortedPre, dInfo);
+        plan::refs_kernel<<<grid, 256>>>(s->d_bvh, n, pre, topPos, sortedPre, s->d_ref, dInfo);
+        g_launches += 5;
+        cudaError_t e = cudaMemcpy(&hostInfo, dInfo, sizeof hostInfo, cudaMemcpyDeviceToHost);
+        if (e != cudaSuccess) return trq::fail(TRQ_ERR_CUDA, "%s: planning kernels failed: %s", who, cudaGetErrorString(e));
+    }
+    TRQ_LAP(tm, "plan kernels");
+    if (hostInfo.error)
+        return trq::fail(hostInfo.error == plan::ERR_DEPTH ? TRQ_ERR_DEPTH : TRQ_ERR_LAYOUT, "bvhList: node %u: %s (%u, %u)", hostInfo.errorNode,
+                         plan_error_text(hostInfo.error), hostInfo.errorA, hostInfo.errorB);
+    trq_scene_info_t info{};
+    info.nNode = n; info.nInterior = hostInfo.nInterior; info.nLeaf = hostInfo.nLeaf; info.maxDepth = hostInfo.maxDepth;
+    info.nTri = hostInfo.nTri; info.nSphere = hostInfo.nSphere; info.nSquare = d->nSquare; info.nCube = d->nCube;
+    info.topNodes = hostInfo.nTop;
+    s->maxPIndex = hostInfo.maxPIndex;
+    return finish_scene(s, d, info, hostInfo.nSquare, hostInfo.rootRef, hostInfo.rootMin, hostInfo.rootMax);
 }
 
 }  // namespace
@@ -732,40 +785,8 @@ int trq_scene_create_device(const trq_scene_desc* d, int device, trq_scene** out
     if ((rc = upload_from(&s->d_verts, d->triList, d->nVert, k)) != TRQ_OK) return bail(rc);
     if ((rc = upload_from(&s->d_idx, d->idxList, (size_t)d->nTri * 3, k)) != TRQ_OK) return bail(rc);
     if ((rc = upload_from(&s->d_bvh, d->bvhList, d->nNode, k)) != TRQ_OK) return bail(rc);
-    const uint32_t n = d->nNode;
-    if (pool_malloc((void**)&s->d_ref, (size_t)n * sizeof(uint32_t)) != cudaSuccess) return bail(trq::fail(TRQ_ERR_CUDA, "cudaMalloc(refs) failed"));
     TRQ_LAP(tm, "copy six arrays D2D");
-
-    plan::PlanInfo hostInfo;
-    {
-        trq::PoolScratch mem(device, nullptr);
-        plan::Counts* cnt; uint32_t *leafTotal, *arrivals, *pre, *topPos, *sortedPre; plan::PlanInfo* dInfo;
-        if (!(mem.alloc(&cnt, n) && mem.alloc(&leafTotal, n) && mem.alloc(&arrivals, n) && mem.alloc(&pre, n) && mem.alloc(&topPos, n) &&
-              mem.alloc(&sortedPre, 2048) && mem.alloc(&dInfo, 1)))
-            return bail(trq::fail(TRQ_ERR_NOMEM, "trq_scene_create_device: out of device memory"));
-        cudaMemsetAsync(arrivals, 0, (size_t)n * 4); cudaMemsetAsync(topPos, 0, (size_t)n * 4);
-        cudaMemsetAsync(cnt, 0, (size_t)n * sizeof(plan::Counts)); cudaMemsetAsync(leafTotal, 0, (size_t)n * 4);
-        cudaMemsetAsync(dInfo, 0, sizeof(plan::PlanInfo)); cudaMemsetAsync(s->d_ref, 0xff, (size_t)n * 4);
-        const unsigned grid = (n + 255) / 256;
-        plan::validate_kernel<<<grid, 256>>>(s->d_bvh, n, d->nSphere, d->nSquare, d->nCube, d->nTri, d->nVert, s->d_idx, dInfo);
-        plan::counts_kernel<<<grid, 256>>>(s->d_bvh, n, cnt, leafTotal, arrivals);
-        plan::number_kernel<<<grid, 256>>>(s->d_bvh, n, cnt, leafTotal, s->d_ref, pre, dInfo);
-        plan::top_block_kernel<<<1, 1024>>>(s->d_bvh, n, pre, topPos, sortedPre, dInfo);
-        plan::refs_kernel<<<grid, 256>>>(s->d_bvh, n, pre, topPos, sortedPre, s->d_ref, dInfo);
-        g_launches += 5;
-        cudaError_t e = cudaMemcpy(&hostInfo, dInfo, sizeof hostInfo, cudaMemcpyDeviceToHost);
-        if (e != cudaSuccess) return bail(trq::fail(TRQ_ERR_CUDA, "trq_scene_create_device: planning kernels failed: %s", cudaGetErrorString(e)));
-    }
-    TRQ_LAP(tm, "plan kernels");
-    if (hostInfo.error)
-        return bail(trq::fail(hostInfo.error == plan::ERR_DEPTH ? TRQ_ERR_DEPTH : TRQ_ERR_LAYOUT, "bvhList: node %u: %s (%u, %u)", hostInfo.errorNode,
-                              plan_error_text(hostInfo.error), hostInfo.errorA, hostInfo.errorB));
-    trq_scene_info_t info{};
-    info.nNode = n; info.nInterior = hostInfo.nInterior; info.nLeaf = hostInfo.nLeaf; info.maxDepth = hostInfo.maxDepth;
-    info.nTri = hostInfo.nTri; info.nSphere = hostInfo.nSphere; info.nSquare = d->nSquare; info.nCube = d->nCube;
-    info.topNodes = hostInfo.nTop;
-    s->maxPIndex = hostInfo.maxPIndex;
-    if ((rc = finish_scene(s, d, info, hostInfo.nSquare, hostInfo.rootRef, hostInfo.rootMin, hostInfo.rootMax)) != TRQ_OK) return bail(rc);
+    if ((rc = plan_and_finish(s, d, "trq_scene_create_device")) != TRQ_OK) return bail(rc);
     *out = s;
     return TRQ_OK;
 }
@@ -802,6 +823,78 @@ int trq_scene_update_vertices(trq_scene* s, const void* triList, uint32_t nVert,
     return TRQ_OK;
 }
 
+// New topology from the current geometry (header: the leaf list, the records and what a rebuild keeps). Everything new is
+// staged in a second trq_scene that borrows the arrays a rebuild keeps (spheres, squares, cubes, indices, queue heads) and
+// goes through the same planning and packing as trq_scene_create_device; the scene itself changes only once that has
+// succeeded, so a failure leaves it as it was.
+int trq_scene_rebuild(trq_scene* s, const void* triList, uint32_t nVert, uint32_t flags) {
+    if (!s) return trq::fail(TRQ_ERR_INVALID, "trq_scene_rebuild: NULL scene");
+    if (triList ? nVert != s->nVert : (nVert != 0 && nVert != s->nVert))
+        return trq::fail(TRQ_ERR_INVALID, "trq_scene_rebuild: %u vertices, the scene has %u", nVert, s->nVert);
+    DeviceGuard guard(s->device);
+    if (!guard.ok) return trq::fail(TRQ_ERR_CUDA, "cudaSetDevice(%d) failed", s->device);
+    TRQ_CUDA(cudaDeviceSynchronize());                           // traces in flight still read the old arrays
+    trq_scene* t = new (std::nothrow) trq_scene();
+    if (!t) return trq::fail(TRQ_ERR_NOMEM, "trq_scene_rebuild: out of host memory");
+    t->device = s->device; t->numSMs = s->numSMs;
+    t->d_spheres = s->d_spheres; t->d_squares = s->d_squares; t->d_cubes = s->d_cubes; t->d_idx = s->d_idx; t->d_queues = s->d_queues;
+    t->d_verts = s->d_verts;
+    const bool newVerts = triList && nVert;
+    // the arrays a rebuild replaces: the staged ones on failure, the scene's old ones after the commit
+    auto drop = [&] {
+        pool_free(t->d_bvh); pool_free(t->d_ref); pool_free(t->d_nodes); pool_free(t->d_tris); pool_free(t->d_sph); pool_free(t->d_sq);
+        pool_free(t->d_triN); pool_free(t->d_topSoA);
+        if (newVerts) pool_free(t->d_verts);
+        delete t;
+    };
+    auto bail = [&](int code) { drop(); return code; };
+    int rc = TRQ_OK;
+    if (newVerts && (rc = upload_from(&t->d_verts, triList, nVert, (flags & TRQ_HOST_PTRS) ? cudaMemcpyHostToDevice : cudaMemcpyDeviceToDevice)) != TRQ_OK)
+        return bail(rc);
+    const uint32_t n = s->info.nLeaf, nNode = 2 * n - 1;
+    {
+        trq::PoolScratch mem(s->device, nullptr);
+        RefBVH* leaves = nullptr;
+        if ((rc = trq::reachable_leaves_on_device(s->d_bvh, s->d_ref, s->nNode, n, t->d_verts, s->d_idx, mem, &leaves)) != TRQ_OK) return bail(rc);
+        if (pool_malloc((void**)&t->d_bvh, (size_t)nNode * sizeof(RefBVH)) != cudaSuccess)
+            return bail(trq::fail(TRQ_ERR_NOMEM, "trq_scene_rebuild: out of device memory"));
+        if (n == 1) {                                            // the lone leaf is the root (BVH.hh:52-54), parent 0
+            cudaError_t e = cudaMemcpyAsync(t->d_bvh, leaves, sizeof(RefBVH), cudaMemcpyDeviceToDevice, nullptr);
+            if (e != cudaSuccess) return bail(trq::fail(TRQ_ERR_CUDA, "trq_scene_rebuild: %s", cudaGetErrorString(e)));
+        } else {
+            uint32_t depth = 0;
+            rc = trq::build_on_device(leaves, n, t->d_bvh, s->device, &depth);
+            if (rc == TRQ_ERR_DEPTH)
+                return bail(trq::fail(TRQ_ERR_DEPTH, "trq_scene_rebuild: the new tree has interior depth %u, above the 32-bit trail's 31 "
+                                                     "(Render.hh:140); the scene is unchanged", depth));
+            if (rc != TRQ_OK) return bail(rc);
+        }
+    }
+    trq_scene_desc d{};                                          // counts of the arrays the scene holds (no pointer is read)
+    d.nSphere = s->listSphere; d.nSquare = s->listSquare; d.nCube = s->listCube; d.nVert = s->nVert; d.nTri = s->listTri; d.nNode = nNode;
+    if ((rc = plan_and_finish(t, &d, "trq_scene_rebuild")) != TRQ_OK) return bail(rc);
+
+    // commit: swap the replaced arrays, take over the derived state
+    std::swap(s->d_verts, t->d_verts); std::swap(s->d_bvh, t->d_bvh); std::swap(s->d_ref, t->d_ref);
+    std::swap(s->d_nodes, t->d_nodes); std::swap(s->d_tris, t->d_tris); std::swap(s->d_sph, t->d_sph); std::swap(s->d_sq, t->d_sq);
+    std::swap(s->d_triN, t->d_triN); std::swap(s->d_topSoA, t->d_topSoA);
+    s->info = t->info; s->dev = t->dev; s->nNode = t->nNode; s->topStride = t->topStride; s->stackDepth = t->stackDepth;
+    s->largeTree = t->largeTree; s->leaves = t->leaves; s->maxPIndex = t->maxPIndex;
+    for (int c = 0; c < kNumCfgs; ++c) s->cfg[c] = t->cfg[c];
+    s->autoCfg = t->autoCfg;
+    if (!(s->userCfg && s->cfg[s->defaultCfg].usable)) { s->defaultCfg = s->autoCfg; s->userCfg = false; }
+    drop();
+    return TRQ_OK;
+}
+
+int trq_scene_copy_bvh(const trq_scene* s, void* out, uint32_t flags) {
+    if (!s || !out) return trq::fail(TRQ_ERR_INVALID, "trq_scene_copy_bvh: NULL argument");
+    DeviceGuard guard(s->device);
+    if (!guard.ok) return trq::fail(TRQ_ERR_CUDA, "cudaSetDevice(%d) failed", s->device);
+    TRQ_CUDA(cudaMemcpy(out, s->d_bvh, (size_t)s->nNode * sizeof(RefBVH), (flags & TRQ_HOST_PTRS) ? cudaMemcpyDeviceToHost : cudaMemcpyDeviceToDevice));
+    return TRQ_OK;
+}
+
 int trq_scene_destroy(trq_scene* s) {
     if (!s) return TRQ_OK;
     DeviceGuard guard(s->device);
@@ -824,10 +917,12 @@ const char* trq_kernel_config_name(int cfg) { return (cfg >= 0 && cfg < kNumCfgs
 
 int trq_scene_set_kernel_config(trq_scene* s, int cfg, uint32_t* topNodesStaged) {
     if (!s) return trq::fail(TRQ_ERR_INVALID, "trq_scene_set_kernel_config: NULL scene");
+    const bool user = cfg >= 0;
     if (cfg < 0) cfg = s->autoCfg;
     if (cfg >= kNumCfgs) return trq::fail(TRQ_ERR_INVALID, "trq_scene_set_kernel_config: %d configurations", kNumCfgs);
     if (!s->cfg[cfg].usable) return trq::fail(TRQ_ERR_INVALID, "trq_scene_set_kernel_config: configuration %s does not fit this scene (stack depth %u)", kCfgs[cfg].name, s->stackDepth);
     s->defaultCfg = cfg;
+    s->userCfg = user;
     if (topNodesStaged) *topNodesStaged = kCfgs[cfg].top ? s->cfg[cfg].topCount : 0;
     return TRQ_OK;
 }

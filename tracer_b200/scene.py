@@ -82,6 +82,45 @@ class DevicePrimitive:
             return None if a.size == 0 else torch.from_numpy(a.view(np.uint8).reshape(-1).copy()).to(device)
         return cls(up(prim.sphereList), up(prim.squareList), up(prim.cubeList), up(prim.triList), up(prim.idxList), up(prim.bvhList))
 
+    @classmethod
+    def build(cls, sphereList=None, squareList=None, cubeList=None, triList=None, idxList=None, device=0):
+        """BVH::buildNode + BVH::buildTree without leaving the GPU: the leaves are made on `device` in the order of
+        harness.build_primitive (AAPLRenderer.mm:454-468,546-591) -- spheres, cubes, squares, then triangles, each kind
+        numbered from pIndex 0 -- by trq_bvh_build_nodes_device / trq_bvh_build_nodes_triangles_device, and the tree by
+        trq_bvh_build_tree_device. Arguments are torch uint8 CUDA tensors (or None) on `device` in the reference layouts.
+        Returns the DevicePrimitive, ready for Scene(...)."""
+        import torch
+        from . import layout as L
+        prim = cls(sphereList, squareList, cubeList, triList, idxList)
+        dev = torch.device(f"cuda:{int(device)}")
+        for k, t in prim.arrays.items():
+            if t is not None and t.device != dev:
+                raise ValueError(f"{k} is on {t.device}, not {dev}")
+        kinds = ((L.SPHERE, "sphereList"), (L.CUBE, "cubeList"), (L.SQUARE, "squareList"))
+        n = sum(prim.count(k) for _, k in kinds) + prim.count("idxList")
+        if n == 0:
+            raise ValueError("DevicePrimitive.build: no primitives")
+        item = L.bvh_dtype.itemsize
+        bvh = torch.empty((2 * n - 1) * item, dtype=torch.uint8, device=dev)
+        stream = torch.cuda.current_stream(dev)
+        at = 0
+        for p_type, k in kinds:
+            m = prim.count(k)
+            if m:
+                check(lib.trq_bvh_build_nodes_device(p_type, prim.arrays[k].data_ptr(), m, 0, bvh.data_ptr() + at * item, int(device),
+                                                     C.c_void_p(stream.cuda_stream)), "trq_bvh_build_nodes_device")
+                at += m
+        if prim.count("idxList"):
+            check(lib.trq_bvh_build_nodes_triangles_device(prim.arrays["triList"].data_ptr(), prim.arrays["idxList"].data_ptr(),
+                                                           prim.count("idxList"), 0, bvh.data_ptr() + at * item, int(device),
+                                                           C.c_void_p(stream.cuda_stream)), "trq_bvh_build_nodes_triangles_device")
+        stream.synchronize()                     # the tree build runs on the legacy default stream
+        nNode, depth = C.c_uint32(0), C.c_uint32(0)
+        check(lib.trq_bvh_build_tree_device(bvh.data_ptr(), n, int(device), C.byref(nNode), C.byref(depth)), "trq_bvh_build_tree_device")
+        prim.arrays["bvhList"] = bvh
+        prim.maxDepth = depth.value
+        return prim
+
     def count(self, k):
         t = self.arrays[k]
         return 0 if t is None else t.numel() * t.element_size() // dict(self._sizes)[k]
@@ -169,6 +208,9 @@ class Scene:
         else:
             check(lib.trq_scene_create(C.byref(d), int(device), C.byref(self._h)), "trq_scene_create")
         self.device = int(device)
+        self._read_info()
+
+    def _read_info(self):
         info = SceneInfo()
         check(lib.trq_scene_info(self._h, C.byref(info)), "trq_scene_info")
         self.info = {k: getattr(info, k) for k, _ in SceneInfo._fields_}
@@ -214,6 +256,26 @@ class Scene:
         else:
             n = triList.numel() * triList.element_size() // L.vertex_dtype.itemsize
             check(lib.trq_scene_update_vertices(self._h, triList.data_ptr(), n, 0), "trq_scene_update_vertices")
+
+    def rebuild(self, triList=None):
+        """New topology from the current geometry (trq_scene_rebuild), optionally after moving the vertices: numpy
+        `vertex_dtype` array or a torch uint8 CUDA tensor holding all of the scene's vertices; None keeps them. Triangle leaf
+        boxes follow the vertices, other leaves keep theirs. Refreshes `info`; on failure the scene is unchanged."""
+        if triList is None:
+            check(lib.trq_scene_rebuild(self._h, None, 0, 0), "trq_scene_rebuild")
+        elif isinstance(triList, np.ndarray):
+            a = np.ascontiguousarray(triList)
+            check(lib.trq_scene_rebuild(self._h, a.ctypes.data, a.size, L.HOST_PTRS), "trq_scene_rebuild")
+        else:
+            n = triList.numel() * triList.element_size() // L.vertex_dtype.itemsize
+            check(lib.trq_scene_rebuild(self._h, triList.data_ptr(), n, 0), "trq_scene_rebuild")
+        self._read_info()
+
+    def bvh(self):
+        """The scene's node array (trq_scene_copy_bvh) as a numpy `bvh_dtype` array."""
+        nodes = np.empty(self.info["nNode"], dtype=L.bvh_dtype)
+        check(lib.trq_scene_copy_bvh(self._h, nodes.ctypes.data, L.HOST_PTRS), "trq_scene_copy_bvh")
+        return nodes
 
     @staticmethod
     def kernel_configs():
