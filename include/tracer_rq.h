@@ -170,6 +170,32 @@ int  trq_scene_create_device(const trq_scene_desc* desc, int device, trq_scene**
  * flight, returns when the scene is ready for the next trq_trace. */
 int  trq_scene_update_vertices(trq_scene* scene, const void* triList, uint32_t nVert, uint32_t flags);
 
+/* Refit after primitives moved (animated spheres, squares, cubes and meshes): same topology, new boxes. A scene update
+ * is trq_scene_update_vertices for every leaf type.
+ *   changes    each non-NULL sphereList / squareList / cubeList / triList replaces that array of the scene whole; its count
+ *              must equal the scene's list count (the nSphere / nSquare / nCube / nVert the scene was created with, not
+ *              its leaf counts). A NULL pointer with count 0 keeps that array. idxList and bvhList must be NULL with count
+ *              0: they would change the topology. All arrays are device pointers on the scene's device, or all are host
+ *              pointers with TRQ_HOST_PTRS.
+ *   leaves     every leaf the root reaches whose primitive type was replaced gets new bBOX mini / maxi. A sphere, square
+ *              or cube leaf gets, bit for bit, the box trq_bvh_build_node(list[pIndex].box.mini, .maxi, list[pIndex].model,
+ *              pType, pIndex) writes, with `box` the record's boundingBOX (Sphere, Square) or box (Cube)
+ *              (AAPLRenderer.mm:454-468). A triangle leaf gets what trq_scene_update_vertices gives it.
+ *   kept       parent, left, right, axis, pType, pIndex and the padding words of every node, byte for byte. Leaves the root
+ *              does not reach and leaves of unknown pType keep their boxes.
+ *   interior   the interior nodes the root reaches are refit bottom-up as unions of their children, as in
+ *              trq_scene_update_vertices; a one-leaf scene's root leaf is refit like any other leaf.
+ *   derived    the packed layout (sphere centre, radius and material; square ranges, axes and material; interior nodes; the
+ *              top-of-tree block) and the root box are derived again. Everything that reads the lists sees the new records:
+ *              traces (the reference-layout kernel and cubes included), trq_expand_hits, and the bounce and shadow spawns,
+ *              so replacing squareList moves the lights trq_spawn_shadow samples even where the squares have no leaves.
+ *   unchanged  trq_scene_info, the leaf types the traversal kernels are specialised for, the launch configurations and a
+ *              configuration chosen with trq_scene_set_kernel_config.
+ *   failure    TRQ_ERR_INVALID (NULL scene or changes, a count mismatch, a non-NULL idxList / bvhList, a NULL array with a
+ *              non-zero count), TRQ_ERR_NOMEM (no scratch): the scene is exactly as before.
+ * Synchronous: waits for traces in flight, returns when the scene is ready for the next trq_trace. */
+int  trq_scene_update_primitives(trq_scene* scene, const trq_scene_desc* changes, uint32_t flags);
+
 /* Rebuild: a new topology from the scene's current geometry, on the device, in place -- for motion a refit cannot follow
  * (a refit tree's boxes stretch and overlap as the geometry moves, and every ray pays for it). triList: the scene's nVert
  * new vertices (a device pointer, or a host pointer with TRQ_HOST_PTRS), or NULL (nVert 0) to keep the current ones.
@@ -177,8 +203,8 @@ int  trq_scene_update_vertices(trq_scene* scene, const void* triList, uint32_t n
  *              made these are nodes 1..n in list order, so rebuilding an unchanged scene reproduces its tree byte for byte.
  *   leaves     a triangle leaf keeps its pIndex; its box is what trq_bvh_build_nodes_triangles gives for that triangle
  *              from the current vertices (std::min / std::max of the three, then BVH::buildNode with the identity). Every
- *              other leaf (sphere, square, cube, unknown pType) keeps pType, pIndex and box: moving those primitives is
- *              not a rebuild's business. All other fields are zero, as trq_bvh_build_node writes them.
+ *              other leaf (sphere, square, cube, unknown pType) keeps pType, pIndex and box: to move those primitives,
+ *              move them with trq_scene_update_primitives first. All other fields are zero, as trq_bvh_build_node writes them.
  *   tree       what trq_bvh_build_tree_gpu makes from that leaf list (the host builder's tree except where its std::sort
  *              fallback meets equal or NaN keys, see there); nNode becomes 2n - 1, so a scene whose bvhList had
  *              unreachable nodes shrinks.

@@ -65,6 +65,7 @@ ds.hit(r0)
 ds.update_vertices(tri); ds.hit(r0, any=True)
 # the kernels specialised by leaf types: triangles only (ds) and triangles + spheres (C1's spheres), every configuration
 sp = Scene(H.scene_c1(), 0)
+sp.update_primitives(spheres=torch.from_numpy(H.scene_c1().sphereList.view(np.uint8).reshape(-1).copy()).cuda())   # sphere leaf refit
 rs = scene.cast_rays((13, 2, 3), (0, 0, 0), (0, 1, 0), np.float32(20 * np.pi / 180), 96, 54)
 for sc, rr in ((ds, r0), (sp, rs)):
     for c in range(len(Scene.kernel_configs())):

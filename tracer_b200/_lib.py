@@ -49,7 +49,7 @@ class Camera(C.Structure):
 # every symbol include/*.h declares; tests/test_abi.py checks the library exports all of them
 ABI_SYMBOLS = [
     "trq_version", "trq_last_error_string", "trq_device_count",
-    "trq_scene_create", "trq_scene_create_device", "trq_scene_update_vertices", "trq_scene_rebuild", "trq_scene_copy_bvh", "trq_scene_destroy", "trq_device_trim", "trq_scene_info",
+    "trq_scene_create", "trq_scene_create_device", "trq_scene_update_vertices", "trq_scene_update_primitives", "trq_scene_rebuild", "trq_scene_copy_bvh", "trq_scene_destroy", "trq_device_trim", "trq_scene_info",
     "trq_kernel_config_count", "trq_kernel_config_name", "trq_scene_set_kernel_config", "trq_scene_kernel_config",
     "trq_trace", "trq_host_sync", "trq_expand_hits", "trq_launch_count", "trq_profile_enable", "trq_profile_read", "trq_probe_bandwidth",
     "trq_bvh_build_node", "trq_bvh_build_nodes_triangles", "trq_bvh_build_nodes_triangles_device", "trq_bvh_build_nodes_device", "trq_bvh_build_tree", "trq_bvh_build_tree_gpu", "trq_bvh_build_tree_device",
@@ -72,6 +72,7 @@ lib.trq_launch_count.restype = _u64
 lib.trq_scene_create.argtypes = [C.POINTER(SceneDesc), C.c_int, C.POINTER(_vp)]
 lib.trq_scene_create_device.argtypes = [C.POINTER(SceneDesc), C.c_int, C.POINTER(_vp)]
 lib.trq_scene_update_vertices.argtypes = [_vp, _vp, _u32, _u32]
+lib.trq_scene_update_primitives.argtypes = [_vp, C.POINTER(SceneDesc), _u32]
 lib.trq_scene_rebuild.argtypes = [_vp, _vp, _u32, _u32]
 lib.trq_scene_copy_bvh.argtypes = [_vp, _vp, _u32]
 lib.trq_scene_destroy.argtypes = [_vp]

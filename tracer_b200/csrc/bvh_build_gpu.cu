@@ -164,6 +164,21 @@ int trq::reachable_leaves_on_device(const RefBVH* bvh, const uint32_t* ref, uint
     return TRQ_OK;
 }
 
+int trq::refit_primitive_leaves_on_device(RefBVH* bvh, const uint32_t* ref, uint32_t nNode, const RefSphere* spheres, const RefSquare* squares,
+                                          const RefCube* cubes) {
+    leaves::RecordLists lists = {};
+    const void* list[3] = {spheres, squares, cubes};
+    for (int32_t t = TRQ_SPHERE; t <= TRQ_CUBE; ++t) {
+        leaves::RecordList& r = lists.kind[t];
+        r.list = (const uint8_t*)list[t];
+        leaves::record_layout(t, &r.stride, &r.modelAt, &r.boxAt);
+    }
+    leaves::refit_primitive_leaves_kernel<<<blocks(nNode, 256), 256>>>(bvh, ref, nNode, lists);
+    trq::note_launches(1);
+    BCK(cudaGetLastError());
+    return TRQ_OK;
+}
+
 namespace {
 
 int check_device(int device, const char* who) {
@@ -245,13 +260,9 @@ extern "C" int trq_bvh_build_nodes_triangles_device(const void* d_triList, const
 
 extern "C" int trq_bvh_build_nodes_device(int32_t pType, const void* d_list, uint32_t n, uint32_t pIndexBase, void* d_nodes_out,
                                           int device, void* stream) {
-    uint32_t stride, modelAt, boxAt;                      // where BVH::buildNode's arguments sit in each record
-    switch (pType) {
-        case TRQ_SPHERE: stride = sizeof(RefSphere); modelAt = offsetof(RefSphere, model); boxAt = offsetof(RefSphere, boundingBOX); break;
-        case TRQ_SQUARE: stride = sizeof(RefSquare); modelAt = offsetof(RefSquare, model); boxAt = offsetof(RefSquare, boundingBOX); break;
-        case TRQ_CUBE:   stride = sizeof(RefCube);   modelAt = offsetof(RefCube, model);   boxAt = offsetof(RefCube, box); break;
-        default: return trq::fail(TRQ_ERR_INVALID, "trq_bvh_build_nodes_device: pType %d is not TRQ_SPHERE, TRQ_SQUARE or TRQ_CUBE", pType);
-    }
+    uint32_t stride, modelAt, boxAt;
+    if (!leaves::record_layout(pType, &stride, &modelAt, &boxAt))
+        return trq::fail(TRQ_ERR_INVALID, "trq_bvh_build_nodes_device: pType %d is not TRQ_SPHERE, TRQ_SQUARE or TRQ_CUBE", pType);
     if (n == 0) return TRQ_OK;
     if (!d_list || !d_nodes_out) return trq::fail(TRQ_ERR_INVALID, "trq_bvh_build_nodes_device: NULL argument");
     int rc = check_device(device, "trq_bvh_build_nodes_device");

@@ -17,4 +17,9 @@ int build_on_device(const RefBVH* dLeaves, uint32_t n, RefBVH* dOut, int device,
 int reachable_leaves_on_device(const RefBVH* bvh, const uint32_t* ref, uint32_t nNode, uint32_t nLeaf, const RefVertex* verts,
                                const uint32_t* idx, PoolScratch& mem, RefBVH** leavesOut);
 
+// The leaf refit of trq_scene_update_primitives: every leaf the root reaches whose kind has a non-NULL list (the scene's
+// replaced records) gets the box trq_bvh_build_node gives for its record; only mini / maxi are written.
+int refit_primitive_leaves_on_device(RefBVH* bvh, const uint32_t* ref, uint32_t nNode, const RefSphere* spheres, const RefSquare* squares,
+                                     const RefCube* cubes);
+
 }  // namespace trq

@@ -1,5 +1,6 @@
 // tracer_b200/csrc/kernels/leaves.cuh -- BVH::buildNode (BVH.hh:271-314) on the GPU: the leaf records of
-// trq_bvh_build_nodes_triangles / trq_bvh_build_node, bit for bit, and the leaf list of a scene rebuild.
+// trq_bvh_build_nodes_triangles / trq_bvh_build_node, bit for bit, the leaf list of a scene rebuild, and the leaf refit
+// of trq_scene_update_primitives.
 //
 // The host restatement (csrc/host/bvh_build.cpp) is compiled without contraction and calls glibc's fminf / fmaxf, which
 // return the OTHER argument when one is NaN and the FIRST argument when the two compare equal (-0.0 vs +0.0). The
@@ -8,6 +9,7 @@
 // which make no promise about which zero they return.
 #pragma once
 #include <cfloat>
+#include <cstddef>
 #include <cuda_runtime.h>
 #include <stdint.h>
 
@@ -74,17 +76,51 @@ triangle_leaves_kernel(const RefVertex* __restrict__ verts, const uint32_t* __re
     if (i < nTri) triangle_leaf(verts, idx, i, pIndexBase + i, &out[i]);
 }
 
-// Sphere / Square / Cube records: `stride` bytes each, the model matrix at byte modelAt and the AABB at byte boxAt.
+// Where BVH::buildNode's arguments sit in a Sphere / Square / Cube record (AAPLRenderer.mm:454-468): `stride` bytes each,
+// the model matrix at byte modelAt and the AABB at byte boxAt (boundingBOX, or box for a Cube). False for any other pType.
+inline bool record_layout(int32_t pType, uint32_t* stride, uint32_t* modelAt, uint32_t* boxAt) {
+    switch (pType) {
+        case TRQ_SPHERE: *stride = sizeof(RefSphere); *modelAt = offsetof(RefSphere, model); *boxAt = offsetof(RefSphere, boundingBOX); return true;
+        case TRQ_SQUARE: *stride = sizeof(RefSquare); *modelAt = offsetof(RefSquare, model); *boxAt = offsetof(RefSquare, boundingBOX); return true;
+        case TRQ_CUBE:   *stride = sizeof(RefCube);   *modelAt = offsetof(RefCube, model);   *boxAt = offsetof(RefCube, box); return true;
+        default: return false;
+    }
+}
+
+__device__ __forceinline__ void primitive_leaf(const uint8_t* rec, uint32_t modelAt, uint32_t boxAt, int32_t pType, uint32_t pIndex, RefBVH* out) {
+    const RefAABB box = *reinterpret_cast<const RefAABB*>(rec + boxAt);
+    float m[16];
+    for (int k = 0; k < 16; ++k) m[k] = reinterpret_cast<const float*>(rec + modelAt)[k];
+    build_node(box.mini, box.maxi, m, pType, pIndex, out);
+}
+
 __global__ void __launch_bounds__(256)
 primitive_leaves_kernel(const uint8_t* __restrict__ list, uint32_t n, uint32_t stride, uint32_t modelAt, uint32_t boxAt, int32_t pType,
                         uint32_t pIndexBase, RefBVH* out) {
     const uint32_t i = blockIdx.x * blockDim.x + threadIdx.x;
-    if (i >= n) return;
-    const uint8_t* rec = list + (size_t)i * stride;
-    const RefAABB box = *reinterpret_cast<const RefAABB*>(rec + boxAt);
-    float m[16];
-    for (int k = 0; k < 16; ++k) m[k] = reinterpret_cast<const float*>(rec + modelAt)[k];
-    build_node(box.mini, box.maxi, m, pType, pIndexBase + i, &out[i]);
+    if (i < n) primitive_leaf(list + (size_t)i * stride, modelAt, boxAt, pType, pIndexBase + i, &out[i]);
+}
+
+// ---- leaf refit of trq_scene_update_primitives: the record list of each kind, indexed by pType (TRQ_SPHERE, TRQ_SQUARE,
+// TRQ_CUBE); list == nullptr keeps the leaves of that kind.
+struct RecordList { const uint8_t* list; uint32_t stride, modelAt, boxAt; };
+struct RecordLists { RecordList kind[3]; };
+
+// Every leaf the root reaches (ref[i] != TRQ_REF_DONE_WORD) whose kind was replaced gets the box trq_bvh_build_node gives
+// for its record list[pIndex]. Only mini / maxi are written: links, pType, pIndex and the padding words stay as they are.
+__global__ void __launch_bounds__(256)
+refit_primitive_leaves_kernel(RefBVH* N, const uint32_t* __restrict__ ref, uint32_t n, RecordLists lists) {
+    const uint32_t i = blockIdx.x * blockDim.x + threadIdx.x;
+    if (i >= n || ref[i] == TRQ_REF_DONE_WORD) return;
+    const int32_t t = N[i].pType;
+    if (t != TRQ_SPHERE && t != TRQ_SQUARE && t != TRQ_CUBE) return;
+    // (constant indices: a dynamic index would copy the parameter block to local memory)
+    const RecordList r = t == TRQ_SPHERE ? lists.kind[TRQ_SPHERE] : t == TRQ_SQUARE ? lists.kind[TRQ_SQUARE] : lists.kind[TRQ_CUBE];
+    if (!r.list) return;
+    const uint32_t p = N[i].pIndex;
+    RefBVH nb;
+    primitive_leaf(r.list + (size_t)p * r.stride, r.modelAt, r.boxAt, t, p, &nb);
+    for (int k = 0; k < 3; ++k) { N[i].bBOX.mini[k] = nb.bBOX.mini[k]; N[i].bBOX.maxi[k] = nb.bBOX.maxi[k]; }
 }
 
 // ---- leaf list of trq_scene_rebuild: every leaf the root reaches (ref != TRQ_REF_DONE_WORD), in bvhList order

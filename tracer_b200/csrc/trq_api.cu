@@ -728,6 +728,44 @@ int plan_and_finish(trq_scene* s, const trq_scene_desc* d, const char* who) {
     return finish_scene(s, d, info, hostInfo.nSquare, hostInfo.rootRef, hostInfo.rootMin, hostInfo.rootMax);
 }
 
+// The refit of trq_scene_update_vertices and trq_scene_update_primitives (header: what changes and what is kept). `c` is
+// checked: each list that is non-NULL with a non-zero count replaces the scene's records of that kind whole (host pointers
+// with TRQ_HOST_PTRS, device pointers otherwise); idxList / bvhList are not read. Scratch is allocated before the first
+// copy, so running out of memory leaves the scene as it was. The leaf kernels of the replaced kinds run, then the interior
+// nodes bottom-up as unions of their children (BVH.hh:229-231), then the packed layout is derived again; all on the device.
+int refit_scene(trq_scene* s, const trq_scene_desc* c, uint32_t flags, const char* who) {
+    DeviceGuard guard(s->device);
+    if (!guard.ok) return trq::fail(TRQ_ERR_CUDA, "cudaSetDevice(%d) failed", s->device);
+    TRQ_CUDA(cudaDeviceSynchronize());                           // traces in flight still read the old boxes and records
+    const uint32_t n = s->nNode;
+    trq::PoolScratch mem(s->device, nullptr);
+    uint32_t* arrivals;
+    if (!mem.alloc(&arrivals, n)) return trq::fail(TRQ_ERR_NOMEM, "%s: out of device memory", who);
+    const cudaMemcpyKind kind = (flags & TRQ_HOST_PTRS) ? cudaMemcpyHostToDevice : cudaMemcpyDeviceToDevice;
+    const bool sph = c->sphereList && c->nSphere, sq = c->squareList && c->nSquare, cube = c->cubeList && c->nCube, tri = c->triList && c->nVert;
+    if (sph) TRQ_CUDA(cudaMemcpy(s->d_spheres, c->sphereList, (size_t)c->nSphere * sizeof(RefSphere), kind));
+    if (sq) TRQ_CUDA(cudaMemcpy(s->d_squares, c->squareList, (size_t)c->nSquare * sizeof(RefSquare), kind));
+    if (cube) TRQ_CUDA(cudaMemcpy(s->d_cubes, c->cubeList, (size_t)c->nCube * sizeof(RefCube), kind));
+    if (tri) TRQ_CUDA(cudaMemcpy(s->d_verts, c->triList, (size_t)c->nVert * sizeof(RefVertex), kind));
+    TRQ_CUDA(cudaMemsetAsync(arrivals, 0, (size_t)n * 4));
+    const unsigned grid = (n + 255) / 256;
+    if (tri) { plan::refit_leaves_kernel<<<grid, 256>>>(s->d_bvh, s->d_ref, n, s->d_verts, s->d_idx); g_launches++; }
+    if (sph || sq || cube) {
+        const int rc = trq::refit_primitive_leaves_on_device(s->d_bvh, s->d_ref, n, sph ? s->d_spheres : nullptr, sq ? s->d_squares : nullptr,
+                                                             cube ? s->d_cubes : nullptr);
+        if (rc != TRQ_OK) return rc;
+    }
+    plan::refit_interior_kernel<<<grid, 256>>>(s->d_bvh, s->d_ref, n, arrivals);
+    pack_scene_kernel<<<grid, 256>>>(s->d_bvh, s->d_ref, n, s->d_verts, s->d_idx, s->d_spheres, s->d_squares,
+                                     s->d_nodes, s->d_tris, s->d_sph, s->d_sq, s->d_triN, s->d_topSoA, s->topStride);
+    g_launches += 2;
+    RefAABB root;
+    TRQ_CUDA(cudaMemcpy(&root, &s->d_bvh[0].bBOX, sizeof root, cudaMemcpyDeviceToHost));
+    for (int k = 0; k < 3; ++k) { s->dev.rootMin[k] = root.mini[k]; s->dev.rootMax[k] = root.maxi[k]; }
+    TRQ_CUDA(cudaGetLastError());
+    return TRQ_OK;
+}
+
 }  // namespace
 
 extern "C" {
@@ -791,36 +829,30 @@ int trq_scene_create_device(const trq_scene_desc* d, int device, trq_scene** out
     return TRQ_OK;
 }
 
-// Refit after the vertices moved (animated meshes): same topology, new boxes. The triangle leaves' boxes are recomputed
-// from the new vertices (min / max of the three, AAPLRenderer.mm:575-589), the interior boxes bottom-up as unions of
-// their children (BVH.hh:229-231), and the packed layout is derived again -- all on the device. `triList` holds nVert
-// vertices (device pointer, or host with TRQ_HOST_PTRS). Returns after the scene is ready for the next trq_trace.
+// Refit after the vertices moved (animated meshes): the refit with only triList replaced.
 int trq_scene_update_vertices(trq_scene* s, const void* triList, uint32_t nVert, uint32_t flags) {
     if (!s || !triList) return trq::fail(TRQ_ERR_INVALID, "trq_scene_update_vertices: NULL argument");
     if (nVert != s->nVert) return trq::fail(TRQ_ERR_INVALID, "trq_scene_update_vertices: %u vertices, the scene has %u", nVert, s->nVert);
     if (nVert == 0) return TRQ_OK;                              // (a one-leaf scene is refit too: its leaf is the root)
-    DeviceGuard guard(s->device);
-    if (!guard.ok) return trq::fail(TRQ_ERR_CUDA, "cudaSetDevice(%d) failed", s->device);
-    TRQ_CUDA(cudaDeviceSynchronize());                           // traces in flight still read the old boxes
-    TRQ_CUDA(cudaMemcpy(s->d_verts, triList, (size_t)nVert * sizeof(RefVertex), (flags & TRQ_HOST_PTRS) ? cudaMemcpyHostToDevice : cudaMemcpyDeviceToDevice));
-    const uint32_t n = s->nNode;
-    {
-        trq::PoolScratch mem(s->device, nullptr);
-        uint32_t* arrivals;
-        if (!mem.alloc(&arrivals, n)) return trq::fail(TRQ_ERR_NOMEM, "trq_scene_update_vertices: out of device memory");
-        TRQ_CUDA(cudaMemsetAsync(arrivals, 0, (size_t)n * 4));
-        const unsigned grid = (n + 255) / 256;
-        plan::refit_leaves_kernel<<<grid, 256>>>(s->d_bvh, s->d_ref, n, s->d_verts, s->d_idx);
-        plan::refit_interior_kernel<<<grid, 256>>>(s->d_bvh, s->d_ref, n, arrivals);
-        pack_scene_kernel<<<grid, 256>>>(s->d_bvh, s->d_ref, n, s->d_verts, s->d_idx, s->d_spheres, s->d_squares,
-                                         s->d_nodes, s->d_tris, s->d_sph, s->d_sq, s->d_triN, s->d_topSoA, s->topStride);
-        g_launches += 3;
-        RefAABB root;
-        TRQ_CUDA(cudaMemcpy(&root, &s->d_bvh[0].bBOX, sizeof root, cudaMemcpyDeviceToHost));
-        for (int k = 0; k < 3; ++k) { s->dev.rootMin[k] = root.mini[k]; s->dev.rootMax[k] = root.maxi[k]; }
-    }
-    TRQ_CUDA(cudaGetLastError());
-    return TRQ_OK;
+    trq_scene_desc c{};
+    c.triList = triList; c.nVert = nVert;
+    return refit_scene(s, &c, flags, "trq_scene_update_vertices");
+}
+
+// Refit after spheres, squares, cubes and / or vertices moved: every check comes before the scene is touched.
+int trq_scene_update_primitives(trq_scene* s, const trq_scene_desc* c, uint32_t flags) {
+    const char* who = "trq_scene_update_primitives";
+    if (!s || !c) return trq::fail(TRQ_ERR_INVALID, "%s: NULL argument", who);
+    if (c->idxList || c->nTri || c->bvhList || c->nNode)
+        return trq::fail(TRQ_ERR_INVALID, "%s: idxList and bvhList must be NULL with count 0 (they would change the topology)", who);
+    if ((c->nSphere && !c->sphereList) || (c->nSquare && !c->squareList) || (c->nCube && !c->cubeList) || (c->nVert && !c->triList))
+        return trq::fail(TRQ_ERR_INVALID, "%s: NULL array with non-zero count", who);
+    const struct { const void* list; uint32_t n, have; const char* what; } kinds[] = {
+        {c->sphereList, c->nSphere, s->listSphere, "spheres"}, {c->squareList, c->nSquare, s->listSquare, "squares"},
+        {c->cubeList, c->nCube, s->listCube, "cubes"}, {c->triList, c->nVert, s->nVert, "vertices"}};
+    for (const auto& k : kinds)
+        if (k.list && k.n != k.have) return trq::fail(TRQ_ERR_INVALID, "%s: %u %s, the scene has %u", who, k.n, k.what, k.have);
+    return refit_scene(s, c, flags, who);
 }
 
 // New topology from the current geometry (header: the leaf list, the records and what a rebuild keeps). Everything new is

@@ -257,6 +257,38 @@ class Scene:
             n = triList.numel() * triList.element_size() // L.vertex_dtype.itemsize
             check(lib.trq_scene_update_vertices(self._h, triList.data_ptr(), n, 0), "trq_scene_update_vertices")
 
+    def update_primitives(self, spheres=None, squares=None, cubes=None, triList=None):
+        """Refit after primitives moved (trq_scene_update_primitives, same topology): each argument given replaces that list
+        of the scene whole (same count as the scene was created with); None keeps it. Either all numpy arrays of
+        `sphere_dtype` / `square_dtype` / `cube_dtype` / `vertex_dtype`, or all torch uint8 CUDA tensors holding those
+        layouts on the scene's device. Triangle leaves are refit as by update_vertices."""
+        given = {k: a for k, a in (("sphereList", spheres), ("squareList", squares), ("cubeList", cubes), ("triList", triList))
+                 if a is not None}
+        host = [isinstance(a, np.ndarray) for a in given.values()]
+        if any(host) and not all(host):
+            raise TypeError("update_primitives: give either numpy arrays or CUDA tensors, not both")
+        d = SceneDesc()
+        if all(host):
+            dtypes = dict(sphereList=L.sphere_dtype, squareList=L.square_dtype, cubeList=L.cube_dtype, triList=L.vertex_dtype)
+            keep = []                            # the arrays must outlive the call
+            for k, a in given.items():
+                if a.dtype != dtypes[k]:
+                    raise TypeError(f"{k}: expected dtype {dtypes[k]}, got {a.dtype}")
+                a = np.ascontiguousarray(a)
+                keep.append(a)
+                setattr(d, k, a.ctypes.data)
+                setattr(d, _COUNT[k], a.size)
+            check(lib.trq_scene_update_primitives(self._h, C.byref(d), L.HOST_PTRS), "trq_scene_update_primitives")
+        else:
+            prim = DevicePrimitive(**given)
+            for k, t in given.items():
+                if t.device.index != self.device:
+                    raise ValueError(f"update_primitives: {k} is on {t.device}, the scene on cuda:{self.device}")
+            for k in given:
+                setattr(d, k, prim.arrays[k].data_ptr())
+                setattr(d, _COUNT[k], prim.count(k))
+            check(lib.trq_scene_update_primitives(self._h, C.byref(d), 0), "trq_scene_update_primitives")
+
     def rebuild(self, triList=None):
         """New topology from the current geometry (trq_scene_rebuild), optionally after moving the vertices: numpy
         `vertex_dtype` array or a torch uint8 CUDA tensor holding all of the scene's vertices; None keeps them. Triangle leaf
@@ -378,6 +410,9 @@ class Scene:
         check(lib.trq_expand_hits(self._h, rays.data_ptr(), hits.data_ptr(), n, 0, recs.data_ptr(), C.c_void_p(st)),
               "trq_expand_hits")
         return recs
+
+
+_COUNT = dict(sphereList="nSphere", squareList="nSquare", cubeList="nCube", triList="nVert")
 
 
 def _sort_flag(sort):
