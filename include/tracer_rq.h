@@ -69,7 +69,13 @@ typedef struct trq_scene_desc {
 
 /* 32 B. Prefix-compatible with struct Ray (origin@0, direction@16); `tmax` is Scene::hit's
  * test_t (FLT_MAX for closest-hit of primary/bounce rays, light distance for shadow rays).
- * `direction` is used as given (Scene::hit never normalises; Ray's ctor already did). */
+ * `direction` is used as given (Scene::hit never normalises; Ray's ctor already did), and no field is restricted:
+ * every value has the oracle's answer, bit for bit. A -0.0 direction component gives 1/d = -inf; a NaN origin component is
+ * dropped by every box test's fminf / fmaxf, so an all-NaN origin enters every box (at t = FLT_MIN, ties going right) and
+ * visits the whole tree; a NaN tmax accepts leaves until one sets a finite range and otherwise ends as a miss; tmax <= 0 or
+ * -inf misses; a direction need not be unit length (t is then in units of |direction|).
+ * Spawned rays (trq_spawn_bounce / trq_spawn_shadow) use offset_ray, whose int(256 n) follows x86: truncation toward zero,
+ * and INT32_MIN when n is NaN or |256 n| >= 2^31; the offset is added to the float's bits modulo 2^32. */
 typedef struct trq_ray {
     float    ox, oy, oz, tmax;
     float    dx, dy, dz;

@@ -257,14 +257,17 @@ int orq_cube_hit(const orq_cube* c, const float o_[3], const float d_[3], float 
 }
 
 /* ---------------------------------------------------------------- offset_ray  (Math.hh:57-74) */
-static inline int32_t f2i(float f) { int32_t i; memcpy(&i, &f, 4); return i; }
-static inline float i2f(int32_t i) { float f; memcpy(&f, &i, 4); return f; }
+static inline uint32_t f2u(float f) { uint32_t i; memcpy(&i, &f, 4); return i; }
+static inline float u2f(uint32_t i) { float f; memcpy(&f, &i, 4); return f; }
+/* (int32_t)v as x86 computes it (cvttss2si): truncation, INT32_MIN for NaN and outside [-2^31, 2^31). The cast itself is
+ * undefined there in C, so the rule is spelled out. */
+static inline int32_t x86_f2i(float v) { return (v != v || v >= 0x1p31f || v < -0x1p31f) ? INT32_MIN : (int32_t)v; }
 
 void orq_offset_ray(const float p[3], const float n[3], float out[3]) {
     const float origin = 1.0f / 32.0f, float_scale = 1.0f / 65536.0f, int_scale = 256.0f;
     for (int k = 0; k < 3; ++k) {
-        int32_t of_i = (int32_t)(int_scale * n[k]);                        /* :64 (truncation) */
-        float p_i = i2f(f2i(p[k]) + ((p[k] < 0.0f) ? -of_i : of_i));       /* :66-69 */
+        uint32_t of_i = (uint32_t)x86_f2i(int_scale * n[k]);                /* :64 (truncation) */
+        float p_i = u2f(f2u(p[k]) + ((p[k] < 0.0f) ? 0u - of_i : of_i));    /* :66-69, modulo 2^32 */
         out[k] = fabsf(p[k]) < origin ? p[k] + float_scale * n[k] : p_i;   /* :71-73 */
     }
 }

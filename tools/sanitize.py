@@ -11,7 +11,7 @@ import numpy as np
 sys.path.insert(0, os.path.dirname(os.path.dirname(os.path.abspath(__file__))))
 import torch  # noqa: E402
 
-from tracer_b200 import Scene, harness as H  # noqa: E402
+from tracer_b200 import Scene, harness as H, rays_to_torch  # noqa: E402
 from tracer_b200.scene import BVHBuilder  # noqa: E402
 
 prim = H.scene_reference_cornell()
@@ -41,6 +41,18 @@ r1, s1, c1 = scene.spawn_bounce(r0, h0, seed_base=3)
 h1 = scene.hit_indirect(r1, c1)
 sh, s2, c2 = scene.spawn_shadow(r1, h1, 5, 6, seed_base=5, count_in=c1)
 scene.hit_indirect(sh, c2, any=True)
+# NaN-origin rays on a depth-31 comb fill the far-child stack to its bound; spawns from degenerate normals (NaN, huge)
+from tests.test_special_rays_cpu import aimed_rays, comb_right, degenerate_scene, nan_origin_rays  # noqa: E402
+cs = Scene(comb_right(), 0)
+cr = rays_to_torch(nan_origin_rays(np.random.default_rng(1), 1024), "cuda:0")
+cs.hit(cr); cs.hit(cr, any=True); cs.hit(cr, reflayout=True)
+cs.close()
+dp, dt = degenerate_scene()
+dscene = Scene(dp, 0)
+dr = rays_to_torch(aimed_rays(np.random.default_rng(2), dt, 4096), "cuda:0")
+dh = dscene.hit(dr)
+dscene.expand(dr, dh); dscene.spawn_bounce(dr, dh); dscene.spawn_shadow(dr, dh, 0, 1)
+dscene.close()
 # the RNG-texture producers (row f-4) and the single-rank gather path (tile counts in the trace, sender kernel, gather_wait_kernel)
 tex = torch.randint(-2**31, 2**31 - 1, (r0.shape[0], 4), dtype=torch.int32, device=r0.device)
 r2, s3, c3 = scene.spawn_bounce(r0, h0, rng_state=tex)

@@ -74,14 +74,18 @@ struct RngSlot {
     ~RngSlot() { if (slot) rng.store(slot); }
 };
 
-// Math.hh:57-74
+// (int32_t)v as x86 computes it (cvttss2si), spelled out because the cast is undefined for NaN and out-of-range values:
+// truncation toward zero, INT32_MIN for NaN and for values outside [-2^31, 2^31). The device uses the same rule.
+inline int32_t x86_f2i(float v) { return (v != v || v >= 0x1p31f || v < -0x1p31f) ? INT32_MIN : (int32_t)v; }
+
+// Math.hh:57-74; the negation and the add into the float's bits wrap modulo 2^32
 inline V3 offset_ray(V3 p, V3 n) {
     const float origin = 1.0f / 32.0f, float_scale = 1.0f / 65536.0f, int_scale = 256.0f;
     float pin[3] = {p.x, p.y, p.z}, nin[3] = {n.x, n.y, n.z}, out[3];
     for (int k = 0; k < 3; ++k) {
-        int32_t of_i = (int32_t)(int_scale * nin[k]);
-        int32_t pi; std::memcpy(&pi, &pin[k], 4);
-        pi += (pin[k] < 0) ? -of_i : of_i;
+        uint32_t of_i = (uint32_t)x86_f2i(int_scale * nin[k]);
+        uint32_t pi; std::memcpy(&pi, &pin[k], 4);
+        pi += (pin[k] < 0) ? 0u - of_i : of_i;
         float p_i; std::memcpy(&p_i, &pi, 4);
         out[k] = fabsf(pin[k]) < origin ? pin[k] + float_scale * nin[k] : p_i;
     }

@@ -55,26 +55,16 @@ __device__ __forceinline__ void rng_release(const Pcg32Dev& rng, uint32_t* rngSt
     if (rngState) *reinterpret_cast<uint4*>(rngState + 4 * (size_t)pixel) = rng.store();
 }
 
-// Math.hh:57-74
-__device__ __forceinline__ f3 offset_ray_dev(const f3& p, const f3& n) {
+// Math.hh:57-74. of_i = int(256 n) with the host's conversion (host_f2i: NaN and |256 n| >= 2^31 give INT32_MIN); the
+// negation and the add into the float's bits wrap modulo 2^32, as on the host.
+__device__ __forceinline__ float offset_component(float p, float n) {
     const float origin = 1.0f / 32.0f, float_scale = 1.0f / 65536.0f, int_scale = 256.0f;
-    f3 out;
-    {
-        const int of_i = (int)fmul(int_scale, n.x);
-        const float p_i = __int_as_float(__float_as_int(p.x) + ((p.x < 0.0f) ? -of_i : of_i));
-        out.x = fabsf(p.x) < origin ? fadd(p.x, fmul(float_scale, n.x)) : p_i;
-    }
-    {
-        const int of_i = (int)fmul(int_scale, n.y);
-        const float p_i = __int_as_float(__float_as_int(p.y) + ((p.y < 0.0f) ? -of_i : of_i));
-        out.y = fabsf(p.y) < origin ? fadd(p.y, fmul(float_scale, n.y)) : p_i;
-    }
-    {
-        const int of_i = (int)fmul(int_scale, n.z);
-        const float p_i = __int_as_float(__float_as_int(p.z) + ((p.z < 0.0f) ? -of_i : of_i));
-        out.z = fabsf(p.z) < origin ? fadd(p.z, fmul(float_scale, n.z)) : p_i;
-    }
-    return out;
+    const uint32_t of_i = (uint32_t)host_f2i(fmul(int_scale, n));
+    const float p_i = __uint_as_float(__float_as_uint(p) + ((p < 0.0f) ? 0u - of_i : of_i));
+    return fabsf(p) < origin ? fadd(p, fmul(float_scale, n)) : p_i;
+}
+__device__ __forceinline__ f3 offset_ray_dev(const f3& p, const f3& n) {
+    return make_f3(offset_component(p.x, n.x), offset_component(p.y, n.y), offset_component(p.z, n.z));
 }
 
 // Sampling.hh:18-34

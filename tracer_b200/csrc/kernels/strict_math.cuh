@@ -21,6 +21,12 @@ __device__ __forceinline__ float fmul(float a, float b) { return __fmul_rn(a, b)
 __device__ __forceinline__ float fdiv(float a, float b) { return __fdiv_rn(a, b); }
 __device__ __forceinline__ float fsqrt(float a) { return __fsqrt_rn(a); }
 
+// (int32_t)v as the host computes it (x86 cvttss2si): truncation toward zero, and INT32_MIN for NaN and for values outside
+// [-2^31, 2^31). CUDA's (int)v saturates instead and maps NaN to 0, so offset_ray would move a point the host does not.
+__device__ __forceinline__ int32_t host_f2i(float v) {
+    return (v != v || v >= 0x1p31f || v < -0x1p31f) ? INT32_MIN : __float2int_rz(v);
+}
+
 __device__ __forceinline__ f3 make_f3(float x, float y, float z) { f3 r; r.x = x; r.y = y; r.z = z; return r; }
 __device__ __forceinline__ f3 ld3(const float* p) { return make_f3(p[0], p[1], p[2]); }
 __device__ __forceinline__ f3 add3(f3 a, f3 b) { return make_f3(fadd(a.x, b.x), fadd(a.y, b.y), fadd(a.z, b.z)); }
