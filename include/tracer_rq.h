@@ -327,9 +327,13 @@ int  trq_mgpu_destroy(trq_mgpu* m);
 /* ---- multi-GPU: hit gather through NVLink peer memory (one process per GPU, one node) -----------------------
  * Rays shard across ranks with no collective (SURVEY.md section 8e). A consumer that wants EVERY rank's hits whole
  * (the all-gather of trq_hit[N/R] of section 8e) gets them while the traversal is still running: the trace kernel
- * counts finished records per 4096-record tile, and a sender kernel that shares the SMs with it ships every complete
- * tile into slot [rank] of every other rank's buffer over NVLink with coalesced stores -- compute and all-gather
- * overlap tile by tile -- then publishes (count, step) with system-scope release stores. No NCCL call.
+ * counts finished records per tile of 2^TRQ_GATHER_TILE_SHIFT records (environment, 8..16, default 11: 2048 records),
+ * and a sender kernel that shares the SMs with it ships every complete tile into slot [rank] of every other rank's
+ * buffer over NVLink -- compute and all-gather overlap tile by tile -- then publishes (count, step) with system-scope
+ * release stores. No NCCL call. The sender is by default the TMA one (bulk copies through 24 KB of shared memory, in
+ * 12 KB chunks). The LSU sender (coalesced 16-byte loads and stores, no shared memory) runs instead when
+ * TRQ_GATHER_TMA=0, or when those 24 KB do not fit in the SM beside the resident trace CTAs, which happens for
+ * deep trees (a larger far-child stack per ray). Both give the same bytes.
  *   1. every rank: trq_gather_create -> 64-byte handle; exchange the handles (any transport, e.g. MPI /
  *      torch.distributed all_gather) into a world*64-byte array in rank order; trq_gather_connect.
  *   2. per step: trq_trace_gather(rays of this rank) then trq_gather_wait -> hitsAll, counts[r]; rank r's records

@@ -304,8 +304,8 @@ struct TraceParams {
     const uint32_t* order;         // optional queue order (TRQ_SORT_RAYS): queue slot -> ray index; NULL = identity
     const uint32_t* orderFlag;     // optional (automatic mode): the probe's counters; `order` applies only if batch_is_incoherent()
     const unsigned long long* nPtr;    // optional device-resident batch size (trq_trace_indirect); n is then the capacity
-    // trq_trace_gather: every finished record also counts towards its tile of TRQ_GATHER_TILE consecutive records
-    // (tileDone[index >> shift], after a fence), so that gather_send_kernel -- running beside this kernel -- can ship each
+    // trq_trace_gather: every finished record also counts towards its tile of 2^tileShift consecutive records
+    // (tileDone[index >> shift], after a fence), so that the sender kernel -- running beside this kernel -- can ship each
     // tile to the peer GPUs the moment it is complete. NULL otherwise.
     uint32_t*           tileDone;
     uint32_t            tileShift;     // log2(records per tile)

@@ -1168,8 +1168,10 @@ int trq_spawn_shadow_rng(trq_scene* s, const trq_ray* rays, const trq_hit* hits,
 // Peer-memory hit gather (SURVEY.md section 8e: a consumer that wants every rank's hits whole). One process per GPU;
 // every rank owns a buffer [phase][rank][capacity] of trq_hit plus a small header (flags, counts), exported through
 // CUDA IPC. trq_trace_gather traces this rank's rays into slot [rank] of its own buffer and, BESIDE the trace kernel,
-// runs gather_send_kernel on a second stream: the trace counts finished records per 4096-record tile, the sender ships
-// each complete tile into slot [rank] of EVERY other rank's buffer over NVLink with coalesced 16-byte stores. The
+// runs a sender kernel on a second stream: the trace counts finished records per tile of 2^TRQ_GATHER_TILE_SHIFT
+// records (default 2^11 = 2048), the sender ships each complete tile into slot [rank] of EVERY other rank's buffer over
+// NVLink (gather_send_tma_kernel with TMA bulk copies; gather_send_kernel with coalesced 16-byte stores when
+// TRQ_GATHER_TMA=0 or when the TMA sender's staging does not fit beside the trace CTAs). The
 // all-gather runs under the traversal, tile by tile, with no NCCL call; the sender's last CTA publishes (count, step)
 // with system-scope release stores. trq_gather_wait enqueues a small kernel that acquires all ranks' step numbers.
 // Three phases (step mod 3): a peer can start writing phase p again at step k + 3 only after it has seen this rank's
@@ -1314,20 +1316,28 @@ int trq_trace_gather(trq_scene* s, trq_gather* g, const trq_ray* rays, uint64_t 
     const bool any = (flags & TRQ_TRACE_ANY) != 0, hit16 = (flags & TRQ_HIT16) != 0;
     const void* fn = kCfgs[0].fn[s->leaves][any ? 1 : 0][hit16 ? 1 : 0];
     bool bumped = false, useTma = false;
+    size_t chosen = 228 * 1024;
     if (n) {
         static const size_t kCarveKB[] = {0, 8, 16, 32, 64, 100, 132, 164, 196, 228};
         const size_t need = (size_t)s->cfg[0].blocksPerSM[any ? 1 : 0][hit16 ? 1 : 0] * (s->cfg[0].smem + kSmemBlockReserve);
-        size_t chosen = 228 * 1024;
         for (size_t kb : kCarveKB) if (kb * 1024 >= need) { chosen = kb * 1024; break; }
         static const int tmaEnv = [] { const char* e = getenv("TRQ_GATHER_TMA"); return e ? atoi(e) : 1; }();
         // the TMA sender stages through 24 KB of shared memory; beside a trace that leaves less than that even at the largest
         // carve-out (very deep trees) the LSU sender, which needs none, is the one that can run concurrently
         useTma = tmaEnv != 0 && 228 * 1024 >= need + kSmemBlockReserve + 512 + (size_t)TRQ_SEND_TMA_STAGES * TRQ_SEND_TMA_CHUNK + 256;
         const size_t senderSmem = useTma ? (size_t)TRQ_SEND_TMA_STAGES * TRQ_SEND_TMA_CHUNK + 256 : 0;
-        if (chosen - need < kSmemBlockReserve + 512 + senderSmem && chosen < 228 * 1024) {
+        const bool bump = chosen - need < kSmemBlockReserve + 512 + senderSmem && chosen < 228 * 1024;
+        if (bump)
             for (size_t kb : kCarveKB) if (kb * 1024 > chosen) { chosen = kb * 1024; break; }
-            bumped = cudaFuncSetAttribute(fn, cudaFuncAttributePreferredSharedMemoryCarveout, (int)((chosen * 100 + kSmemPerSM - 1) / kSmemPerSM)) == cudaSuccess;
-        }
+        const int carveout = (int)((chosen * 100 + kSmemPerSM - 1) / kSmemPerSM);
+        // The sender may reach an SM before the trace does: it starts with the caller's stream at evStart, and with
+        // TRQ_SORT_RAYS the ordering kernels still run ahead of the trace. An SM takes its carve-out from the first CTA it
+        // gets, and the sender's own need (24 KB, or none) leaves no room for a trace CTA. With a sender CTA on every SM
+        // (nTiles >= numSMs) the trace then has nowhere to run and every sender waits for the timeout. The sender asks for
+        // the trace's carve-out, so a trace CTA fits beside it whichever kernel arrives first.
+        TRQ_CUDA(cudaFuncSetAttribute(useTma ? (const void*)gather_send_tma_kernel : (const void*)gather_send_kernel,
+                                      cudaFuncAttributePreferredSharedMemoryCarveout, carveout));
+        if (bump) bumped = cudaFuncSetAttribute(fn, cudaFuncAttributePreferredSharedMemoryCarveout, carveout) == cudaSuccess;
     }
     const int rc = launch_trace(s, rays, n, flags, own, st, nullptr, g->d_tileDone, tileShift);     // first: its CTAs take their places
     if (bumped) cudaFuncSetAttribute(fn, cudaFuncAttributePreferredSharedMemoryCarveout, cudaSharedmemCarveoutDefault);
