@@ -248,8 +248,13 @@ int  trq_scene_set_kernel_config(trq_scene* scene, int cfg, uint32_t* topNodesSt
 int  trq_scene_kernel_config(const trq_scene* scene);
 
 /* Scene::hit for n rays. Device pointers unless TRQ_HOST_PTRS; asynchronous on `stream`
- * (a cudaStream_t, NULL = default stream) for device pointers. Re-entrant across streams and host threads (any number
- * of launches in flight on any number of streams; each draws its own work-queue head).
+ * (a cudaStream_t, NULL = default stream) for device pointers. Re-entrant across streams and host threads, and
+ * capturable into CUDA graphs. Work-queue heads: a launch captured into a graph allocates, zeroes and frees a head of its
+ * own at every replay, so graphs captured at any time may be replayed concurrently with each other and with eager
+ * calls. Eager launches of a scene take heads from a ring of 4096 that the kernel re-arms: launch k and launch k + 4096
+ * of one scene share a head and must not run at the same time, so with many streams keep fewer than 4096 launches of a
+ * scene issued beside a long-running one (a single stream always satisfies this).
+ * A batch of more than 2^31 rays is traced as consecutive launches of at most 2^31 rays each.
  * `hits` is trq_hit[n], or trq_hit16[n] with TRQ_HIT16. Device rays / hits must be aligned to their record size
  * (32 bytes; 16 for trq_hit16): every record is moved with one access. */
 int  trq_trace(trq_scene* scene, const trq_ray* rays, uint64_t n, uint32_t flags,
@@ -277,7 +282,8 @@ typedef struct trq_camera {
  * rays[y*W + x], tmax = FLT_MAX. Only aperture 0 (the reference's prepareCamera, Tracer.mm:380). */
 int  trq_cast_rays(trq_scene* scene, const trq_camera* camera, uint32_t W, uint32_t H, trq_ray* rays, void* stream);
 
-/* Scene::hit with the batch size read from device memory: traces min(*d_count, capacity) rays. */
+/* Scene::hit with the batch size read from device memory: traces min(*d_count, capacity) rays. One launch covers the
+ * whole capacity, so a capacity above 2^31 is refused (TRQ_ERR_INVALID) whatever *d_count holds. */
 int  trq_trace_indirect(trq_scene* scene, const trq_ray* rays, const uint64_t* d_count, uint64_t capacity,
                         uint32_t flags, trq_hit* hits, void* stream);
 
@@ -343,7 +349,9 @@ int  trq_mgpu_destroy(trq_mgpu* m);
  *      reuse the phase before it has seen this rank finish step k+2). Every rank must call both every step.
  *   3. all ranks synchronise (barrier) before any of them calls trq_gather_destroy.
  * trq_gather_status (after synchronising the stream) reports a peer that never published (timeout 10 s,
- * TRQ_GATHER_TIMEOUT_MS) instead of hanging the GPU. */
+ * TRQ_GATHER_TIMEOUT_MS) instead of hanging the GPU.
+ * A step is one kernel launch: the capacity is at most 2^31 rays (trq_gather_create refuses more), and trq_trace_gather
+ * refuses n above the capacity. */
 typedef struct trq_gather trq_gather;
 #define TRQ_GATHER_HANDLE_BYTES 64
 int  trq_gather_create(trq_scene* scene, uint32_t rank, uint32_t world, uint64_t capacity, trq_gather** out,

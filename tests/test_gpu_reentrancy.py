@@ -1,7 +1,7 @@
-"""GPU: trq_trace is re-entrant -- many launches in flight on many streams, and more launches than the queue-head ring
-holds. Every launch draws its own work-queue head and the kernel's last CTA re-arms it (no memset, no follow-up pass),
-so a head is zero whenever a launch picks it up -- whatever kind of launch used it before (round-1 regression: heads left
-dirty by one kernel variant made the next variant skip rays)."""
+"""GPU: trq_trace is re-entrant -- many launches in flight on many streams, and thousands of launches of mixed kinds on
+one scene, more than the queue-head ring holds. Every eager launch draws its own work-queue head and the kernel's last CTA
+re-arms it, so a head is zero whenever a launch picks it up -- whatever kind of launch used it before (round-1 regression:
+heads left dirty by one kernel variant made the next variant skip rays; graph replays: tests/test_gpu_work_queue.py)."""
 import threading
 
 import numpy as np

@@ -80,7 +80,8 @@ struct CompactHit {
 };
 
 // Work-queue head of one trace launch: `head` is the next unclaimed queue slot; `done` counts CTAs that have left the
-// kernel. The last CTA to leave zeroes both, so a head is always zero between launches (no memset, no resolve pass).
+// kernel. The last CTA to leave zeroes both, so a head of the eager ring is zero between launches (no memset, no resolve
+// pass); a launch captured into a CUDA graph zeroes a head of its own instead (trq_api.cu launch_trace).
 struct QueueHead {
     unsigned long long head;
     unsigned int       done;

@@ -74,8 +74,9 @@ struct DeviceGuard {
     ~DeviceGuard() { if (prev >= 0) cudaSetDevice(prev); }
 };
 
-constexpr int kQueueRing = 4096;           // queue heads handed out round-robin; each is zero between launches (the kernel
-                                           // re-arms it), so only > 4096 launches IN FLIGHT at once could alias one
+constexpr int kQueueRing = 4096;           // queue heads of eager launches, handed out round-robin; each is zero between launches
+                                           // (the kernel's last CTA re-arms it). Launch k and launch k + 4096 share one: they
+                                           // must not run at the same time (trq_trace in include/tracer_rq.h)
 constexpr int kStageBufs = 4;
 constexpr int kProfRing = 64;
 constexpr uint32_t kTopMax = 2047;         // interior nodes numbered breadth-first at the front (11 full levels)
@@ -104,6 +105,11 @@ const KernelCfg kCfgs[] = {
 constexpr int kNumCfgs = (int)(sizeof(kCfgs) / sizeof(kCfgs[0]));
 #ifndef TRQ_DEFAULT_CHUNK_RAYS
 #define TRQ_DEFAULT_CHUNK_RAYS (512ll << 10)
+#endif
+// Largest batch one kernel launch takes (the kernels keep a 32-bit ray index per lane); trq_trace splits larger ones.
+// Smaller values build test variants that exercise the split on small batches.
+#ifndef TRQ_MAX_RAYS_PER_LAUNCH
+#define TRQ_MAX_RAYS_PER_LAUNCH (1ull << 31)
 #endif
 
 }  // namespace
@@ -141,8 +147,8 @@ struct trq_scene {
     bool userCfg = false;         // defaultCfg was chosen with trq_scene_set_kernel_config (kept by a rebuild while usable)
     // stream-ordered scratch for TRQ_SORT_RAYS: a private pool that keeps its memory across synchronisations
     // (the device's default pool hands it back at every sync and re-maps 64 MB on the next sorted launch)
-    cudaMemPool_t scratchPool = nullptr;     // the per-device pool (not owned)
-    // ray-queue heads
+    cudaMemPool_t scratchPool = nullptr;     // the per-device pool (not owned); also holds the queue heads of captured launches
+    // ray-queue heads of eager launches
     QueueHead* d_queues = nullptr;
     std::atomic<uint32_t> queueNext{0};
     // staging for TRQ_HOST_PTRS
@@ -305,7 +311,7 @@ int launch_trace(trq_scene* s, const trq_ray* d_rays, uint64_t n, uint32_t flags
     if (n == 0) return TRQ_OK;
     const bool hit16 = (flags & TRQ_HIT16) != 0;
     const size_t recBytes = hit16 ? sizeof(trq_hit16) : sizeof(trq_hit);
-    constexpr uint64_t kMaxPerLaunch = 1ull << 31;             // the kernels keep a 32-bit ray index per lane
+    constexpr uint64_t kMaxPerLaunch = TRQ_MAX_RAYS_PER_LAUNCH;
     if (n > kMaxPerLaunch) {
         if (nPtr || tileDone) return trq::fail(TRQ_ERR_INVALID, "trq_trace_indirect / trq_trace_gather: more than 2^31 rays");
         for (uint64_t off = 0; off < n; off += kMaxPerLaunch) {
@@ -359,8 +365,18 @@ int launch_trace(trq_scene* s, const trq_ray* d_rays, uint64_t n, uint32_t flags
         if (grid > need) grid = need;
         TraceParams P{};
         P.rays = d_rays; P.hits = d_hits; P.n = n;
-        // the head is zero: heads are zeroed at creation and every launch's last CTA re-arms the one it used
-        P.queue = s->d_queues + (s->queueNext.fetch_add(1) % kQueueRing);
+        // Work-queue head. An eager launch takes the next one of the ring (zero: heads are zeroed at creation and every launch's
+        // last CTA re-arms the one it used). A launch captured into a CUDA graph is fixed in the graph and may be replayed at
+        // any later time, beside any other launch: it gets a head of its own, allocated, zeroed and freed in stream order
+        // around the kernel at every replay. (A per-launch memset for eager launches too costs ~1 % on C1 / C2.)
+        cudaStreamCaptureStatus capture = cudaStreamCaptureStatusNone;
+        TRQ_CUDA(cudaStreamIsCapturing(st, &capture));
+        QueueHead* ownHead = nullptr;
+        if (capture != cudaStreamCaptureStatusNone) {
+            TRQ_CUDA(cudaMallocFromPoolAsync((void**)&ownHead, sizeof(QueueHead), s->scratchPool, st));
+            TRQ_CUDA(cudaMemsetAsync(ownHead, 0, sizeof(QueueHead), st));
+        }
+        P.queue = ownHead ? ownHead : s->d_queues + (s->queueNext.fetch_add(1) % kQueueRing);
         P.stackDepth = cs.stackDepth; P.refillMin = refillMin; P.leafBatch = leafBatch;
         P.topCount = K.top ? cs.topCount : 0;
         P.order = nullptr; P.nPtr = nPtr;
@@ -397,6 +413,7 @@ int launch_trace(trq_scene* s, const trq_ray* d_rays, uint64_t n, uint32_t flags
         void* args[2] = {(void*)&s->dev, (void*)&P};
         TRQ_CUDA(cudaLaunchKernel(K.fn[s->leaves][any ? 1 : 0][hit16 ? 1 : 0], dim3((unsigned)grid), dim3((unsigned)K.block), args, cs.smem, st));
         g_launches++;
+        if (ownHead) TRQ_CUDA(cudaFreeAsync(ownHead, st));
         if (scratch) TRQ_CUDA(cudaFreeAsync(scratch, st));
         if (prof) TRQ_CUDA(cudaEventRecord(prof[1], st));
     }
