@@ -5,7 +5,7 @@
 // the GPU (trq_scene_create_device: the output of trq_bvh_build_tree_device, or a caller's own device builder) the same
 // plan is computed here without a device-to-host copy of the tree, and must give the SAME references:
 //   leaves     numbered per kind in depth-first order, left child first;
-//   interior   the first kTopMax of a breadth-first walk come first in that order (the block a kernel may stage in shared
+//   interior   the first packed::kTopMax of a breadth-first walk come first in that order (the block a kernel may stage in shared
 //              memory), the others follow in depth-first (pre-)order.
 // Depth-first positions need no traversal: with cnt[x] = (interior nodes, triangle / sphere / square leaves) below x,
 //   pre(x)   = depth(x) + sum over ancestors a with x in right(a) of cnt[left(a)].interior
@@ -17,12 +17,11 @@
 
 #include "../../../include/tracer_rq.h"
 #include "../host/layout.h"
+#include "packed_layout.cuh"
 #include "scene_dev.cuh"
 
 namespace trq {
 namespace plan {
-
-constexpr uint32_t kTopMaxDev = 2047;              // == kTopMax in trq_api.cu
 
 enum : uint32_t { ERR_NONE = 0, ERR_CHILD_RANGE, ERR_CHILDREN, ERR_PARENT_LINK, ERR_ROOT_PARENT, ERR_LEAF_INDEX, ERR_VERTEX_INDEX,
                   ERR_DEPTH, ERR_UNREACHABLE };
@@ -136,7 +135,7 @@ number_kernel(const RefBVH* __restrict__ N, uint32_t n, const Counts* __restrict
     }
 }
 
-// One CTA: breadth-first walk of the interior nodes from the root, level by level, left to right, until kTopMaxDev nodes
+// One CTA: breadth-first walk of the interior nodes from the root, level by level, left to right, until packed::kTopMax nodes
 // are listed (the queue order of plan_layout's walk). topPos[node] = position + 1; sortedPre = their pre-order positions,
 // ascending (refs_kernel counts how many of them precede a node).
 __global__ void __launch_bounds__(1024)
@@ -150,11 +149,11 @@ top_block_kernel(const RefBVH* __restrict__ N, uint32_t n, const uint32_t* __res
     if (t == 0) { total = 0; nFront = (N[0].pType == TRQ_BVH) ? 1u : 0u; frontier[0][0] = 0u; }
     __syncthreads();
     int cur = 0;
-    while (nFront > 0 && total < kTopMaxDev) {
+    while (nFront > 0 && total < packed::kTopMax) {
         const uint32_t nf = nFront, base = total;
         // list this level (clipped to the capacity)
         for (uint32_t k = t; k < nf; k += 1024) {
-            if (base + k < kTopMaxDev) { topPos[frontier[cur][k]] = base + k + 1; keys[base + k] = pre[frontier[cur][k]]; }
+            if (base + k < packed::kTopMax) { topPos[frontier[cur][k]] = base + k + 1; keys[base + k] = pre[frontier[cur][k]]; }
         }
         // children that are interior, in order: exclusive scan of (left interior) + (right interior)
         for (uint32_t k = t; k < 2048; k += 1024) {
@@ -169,8 +168,8 @@ top_block_kernel(const RefBVH* __restrict__ N, uint32_t n, const uint32_t* __res
             scan[t] += v0; scan[t + 1024] += v1;
             __syncthreads();
         }
-        const uint32_t listed = (base + nf < kTopMaxDev) ? nf : (kTopMaxDev - base);
-        const uint32_t room = kTopMaxDev - (base + listed);         // what the next level may still add
+        const uint32_t listed = (base + nf < packed::kTopMax) ? nf : (packed::kTopMax - base);
+        const uint32_t room = packed::kTopMax - (base + listed);         // what the next level may still add
         for (uint32_t k = t; k < nf; k += 1024) {
             const RefBVH& b = N[frontier[cur][k]];
             uint32_t pos = scan[k] - ((interior(b.left) ? 1u : 0u) + (interior(b.right) ? 1u : 0u));

@@ -22,12 +22,12 @@
 //                           memory while the traversal is still running (gather_send_kernel: the LSU fallback)
 //   sort_*_kernel           optional ordering of the work queue (TRQ_SORT_RAYS)
 //   expand_hits_kernel      trq_hit -> HitRecord fields (p, gn, sn, uv, f, material)
-//   pack_scene_kernel       reference-layout arrays -> packed traversal layout, on the device
 #pragma once
 #include <cfloat>
 
 #include "../../../include/tracer_rq.h"
 #include "intersect.cuh"
+#include "packed_layout.cuh"
 #include "scene_dev.cuh"
 
 namespace trq {
@@ -38,17 +38,6 @@ __device__ __forceinline__ uint64_t live_count(uint64_t n, const unsigned long l
     if (nPtr == nullptr) return n;
     const unsigned long long m = *nPtr;
     return m < n ? (uint64_t)m : n;
-}
-
-// ---------------------------------------------------------------------------------------------
-// loads
-__device__ __forceinline__ float4 ldg4(const float4* p) { return __ldg(p); }
-
-// 256-bit read-only load (LDG.E.256 on sm_100): two float4 from a 32-byte aligned address.
-__device__ __forceinline__ void ldg8(const float4* p, float4& a, float4& b) {
-    asm volatile("ld.global.nc.v8.f32 {%0,%1,%2,%3,%4,%5,%6,%7}, [%8];"
-                 : "=f"(a.x), "=f"(a.y), "=f"(a.z), "=f"(a.w), "=f"(b.x), "=f"(b.y), "=f"(b.z), "=f"(b.w)
-                 : "l"(p));
 }
 
 // 256-bit store (STG.E.256 on sm_100): one request for a whole 32-byte record.
@@ -285,8 +274,6 @@ sort_scatter_kernel(const uint32_t* __restrict__ keys, uint64_t n, const unsigne
 
 // ---------------------------------------------------------------------------------------------
 // v1: packed layout, persistent warps, shared-memory far-child stack, records finished in the kernel.
-#define TRQ_TRI_STRIDE 4u      // float4 per packed triangle: 64-byte records (48 used) so that a test is two requests, never three
-#define TRQ_SQ_STRIDE  4u      // float4 per packed square
 
 // Output record formats of the packed kernel
 enum : int { OUT_HIT32 = 0, OUT_HIT16 = 1 };
@@ -376,7 +363,8 @@ __device__ __noinline__ void finish_other(const float4* __restrict__ sph, const 
     const f3 o = make_f3(ox, oy, oz), d = make_f3(dx, dy, dz);
     float4 o0 = make_float4(0.f, 0.f, 0.f, 0.f), o1 = o0;
     if (kind == REF_SPHERE) {
-        const float4 s0 = ldg4(sph + (size_t)slot * 2u), s1 = ldg4(sph + (size_t)slot * 2u + 1);
+        float4 s0, s1;
+        packed::load_sphere(sph, slot, s0, s1);
         const f3 p = add3(o, scale3(d, t));
         const f3 gn = divs3(sub3(p, make_f3(s0.x, s0.y, s0.z)), s0.w);
         const uint32_t front = front_face(d, gn) ? TRQ_HIT_FLAG_FRONT : 0u;
@@ -387,10 +375,8 @@ __device__ __noinline__ void finish_other(const float4* __restrict__ sph, const 
         o0 = make_float4(t, __uint_as_float((uint32_t)TRQ_SPHERE), s1.y, s1.x);
         o1 = make_float4(uvx, uvy, s1.z, __uint_as_float(TRQ_HIT_FLAG_HIT | front));
     } else if (SQCUBE && kind == REF_SQUARE) {
-        const float4* qp = sq + (size_t)slot * TRQ_SQ_STRIDE;
-        float4 q0, q1;
-        ldg8(qp, q0, q1);
-        const float4 q2 = ldg4(qp + 2);
+        float4 q0, q1, q2;
+        packed::load_square(sq, slot, q0, q1, q2);
         const uint32_t axes = __float_as_uint(q1.y);
         const unsigned ai = axes & 3u, aj = (axes >> 8) & 3u, ak = (axes >> 16) & 3u;
         const float a = fadd(get3(o, ai), fmul(t, get3(d, ai)));                   // Square.hh:88,91 with the accepted t
@@ -424,33 +410,6 @@ enum : uint32_t { COLD_TEST_T = 0, COLD_BEST, COLD_U, COLD_V, COLD_AUX, COLD_RAY
 __device__ unsigned long long g_stats[8];
 #endif
 
-// Top-of-tree staging (TOP kernels): TMA bulk copies (cp.async.bulk, completion on an mbarrier) bring the first topCount
-// packed nodes -- the top levels of the tree in breadth-first order -- into shared memory when the CTA starts. Source and
-// destination are quarter-major ([4][n] float4: all q0, then all q1, ...): with the node-major 64-byte stride every q0
-// would sit in banks 0-3 / 16-19 and a warp's LDS.128 would serialise 4 ways.
-__device__ __forceinline__ void stage_top_of_tree(float4* dst, const float4* src, uint32_t count, uint32_t srcStride, unsigned long long* mbar) {
-    const uint32_t mb = (uint32_t)__cvta_generic_to_shared(mbar);
-    if (threadIdx.x == 0) {
-        asm volatile("mbarrier.init.shared::cta.b64 [%0], 1;" :: "r"(mb));
-        asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
-    }
-    __syncthreads();
-    if (count == 0) return;
-    if (threadIdx.x == 0) {
-        const uint32_t bytes = count * 16u;
-        asm volatile("mbarrier.arrive.expect_tx.shared::cta.b64 _, [%0], %1;" :: "r"(mb), "r"(4u * bytes) : "memory");
-#pragma unroll
-        for (uint32_t q = 0; q < 4; ++q)
-            asm volatile("cp.async.bulk.shared::cluster.global.mbarrier::complete_tx::bytes [%0], [%1], %2, [%3];"
-                         :: "r"((uint32_t)__cvta_generic_to_shared(dst + (size_t)q * count)), "l"(src + (size_t)q * srcStride), "r"(bytes), "r"(mb) : "memory");
-    }
-    uint32_t ready = 0;
-    while (!ready) {
-        asm volatile("{\n\t.reg .pred p;\n\tmbarrier.try_wait.parity.shared::cta.b64 p, [%1], 0;\n\tselp.u32 %0, 1, 0, p;\n\t}"
-                     : "=r"(ready) : "r"(mb) : "memory");
-    }
-}
-
 // ANY: Scene::hit(any = true). OUT: record format. BLOCK x MINB: CTA size and resident CTAs per SM.
 // TOP: the first P.topCount interior nodes are read from shared memory instead of L1/L2.
 // LEAVES: which leaf types the tree has. The code of the absent ones is compiled out: a triangle-only kernel has no
@@ -462,7 +421,7 @@ __global__ void __launch_bounds__(BLOCK, MINB)
 trace_packed_kernel(const SceneDev S, const TraceParams P) {
     extern __shared__ __align__(128) uint32_t smem_u32[];
     __shared__ unsigned long long topBarrier;
-    const uint32_t topWords = TOP ? P.topCount * 16u : 0u;
+    const uint32_t topWords = TOP ? packed::staged_words(P.topCount) : 0u;
     const float4* const topNodes = reinterpret_cast<const float4*>(smem_u32);        // [4][topCount]
     uint32_t* const stk = smem_u32 + topWords + threadIdx.x;                         // [stackDepth][BLOCK]
     uint32_t* const cold = smem_u32 + topWords + P.stackDepth * BLOCK + threadIdx.x; // [COLD_WORDS][BLOCK]
@@ -471,7 +430,7 @@ trace_packed_kernel(const SceneDev S, const TraceParams P) {
     constexpr int TAG = ((((BLOCK * 8 + MINB) * 2 + (ANY ? 1 : 0)) * 2 + OUT) * 2 + (TOP ? 1 : 0)) * 4 + LEAVES;
     constexpr bool TRIS = LEAVES == LEAVES_TRI, SQCUBE = LEAVES == LEAVES_ALL;
 
-    if (TOP) stage_top_of_tree(reinterpret_cast<float4*>(smem_u32), S.topSoA, P.topCount, S.topStride, &topBarrier);
+    if (TOP) packed::stage_top_of_tree(reinterpret_cast<float4*>(smem_u32), S.topSoA, P.topCount, S.topStride, &topBarrier);
 
     const uint64_t N = live_count(P.n, P.nPtr);
     const bool useOrder = P.order != nullptr && (P.orderFlag == nullptr || batch_is_incoherent(P.orderFlag));
@@ -496,10 +455,8 @@ trace_packed_kernel(const SceneDev S, const TraceParams P) {
                 const f3 d = make_f3(coldf[COLD_DX * BLOCK], coldf[COLD_DY * BLOCK], coldf[COLD_DZ * BLOCK]);
                 if (TRQ_REF_KIND(best) == REF_TRI) {
                     // Triangle.hh:73-82: interpolated normal, checkFace; ids from the finish record
-                    const float4* np = S.triN + (size_t)TRQ_REF_INDEX(best) * 4u;
-                    float4 q0, q1;
-                    ldg8(np, q0, q1);
-                    const float4 q2 = ldg4(np + 2);
+                    float4 q0, q1, q2;
+                    packed::load_tri_finish(S.triN, TRQ_REF_INDEX(best), q0, q1, q2);
                     const float w = fsub(fsub(1.0f, u), v);
                     const f3 gn = add3(add3(scale3(make_f3(q1.x, q1.y, q1.z), u), scale3(make_f3(q2.x, q2.y, q2.z), v)),
                                        scale3(make_f3(q0.x, q0.y, q0.z), w));
@@ -594,14 +551,8 @@ trace_packed_kernel(const SceneDev S, const TraceParams P) {
                     if (active && TRQ_REF_KIND(cur) == REF_INTERIOR) {
                         const uint32_t ni = TRQ_REF_INDEX(cur);
                         float4 q0, q1, q2, q3;
-                        if (TOP && ni < P.topCount) {                         // top of the tree: four LDS.128 from this CTA's copy
-                            const float4* tp = topNodes + ni;
-                            q0 = tp[0]; q1 = tp[P.topCount]; q2 = tp[2u * P.topCount]; q3 = tp[3u * P.topCount];
-                        } else {
-                            const float4* np = S.nodes + (size_t)ni * 4u;
-                            ldg8(np, q0, q1);
-                            ldg8(np + 2, q2, q3);
-                        }
+                        if (TOP && ni < P.topCount) packed::load_staged_node(topNodes, P.topCount, ni, q0, q1, q2, q3);   // this CTA's copy
+                        else                        packed::load_node(S.nodes, ni, q0, q1, q2, q3);
                         float tl = range_y, tr = range_y;                     // :157
                         const bool lt = box_entry(make_f3(q0.x, q0.y, q0.z), make_f3(q1.x, q1.y, q1.z), ro, rinv, range_y, tl);   // :159
                         const bool rt = box_entry(make_f3(q2.x, q2.y, q2.z), make_f3(q3.x, q3.y, q3.z), ro, rinv, range_y, tr);   // :160
@@ -628,20 +579,18 @@ trace_packed_kernel(const SceneDev S, const TraceParams P) {
                 ray.d = make_f3(coldf[COLD_DX * BLOCK], coldf[COLD_DY * BLOCK], coldf[COLD_DZ * BLOCK]);
                 bool h = false; float t = 0.0f, u = 0.0f, v = 0.0f; uint32_t a = 0;
                 if (kind == REF_TRI) {
-                    const float4* tp = S.tris + (size_t)TRQ_REF_INDEX(cur) * TRQ_TRI_STRIDE;
-                    float4 t0, t1;
-                    ldg8(tp, t0, t1);                                       // one 256-bit + one 128-bit request per test
-                    const float4 t2 = ldg4(tp + 2);
+                    float4 t0, t1, t2;
+                    packed::load_tri(S.tris, TRQ_REF_INDEX(cur), t0, t1, t2);
                     h = tri_hit(make_f3(t0.x, t0.y, t0.z), make_f3(t1.x, t1.y, t1.z), make_f3(t2.x, t2.y, t2.z),
                                 ray, FLT_MIN, range_y, t, u, v);
                 }
                 else if (!TRIS && kind == REF_SPHERE) {
-                    const float4 s0 = ldg4(S.sph + (size_t)TRQ_REF_INDEX(cur) * 2u);
+                    const float4 s0 = packed::load_sphere_test(S.sph, TRQ_REF_INDEX(cur));
                     h = sphere_hit(make_f3(s0.x, s0.y, s0.z), s0.w, ray, FLT_MIN, range_y, t);
                 } else if (SQCUBE && kind == REF_SQUARE) {
                     // Square::hit_test (Square.hh:82-92) on the packed record; the rejections are pure comparisons, and-ed
                     float4 q0, q1;
-                    ldg8(S.sq + (size_t)TRQ_REF_INDEX(cur) * TRQ_SQ_STRIDE, q0, q1);
+                    packed::load_square_test(S.sq, TRQ_REF_INDEX(cur), q0, q1);
                     const uint32_t axes = __float_as_uint(q1.y);
                     const unsigned ai = axes & 3u, aj = (axes >> 8) & 3u, ak = (axes >> 16) & 3u;
                     const float tt = fdiv(fsub(q1.x, get3(ro, ak)), get3(ray.d, ak));
@@ -882,15 +831,6 @@ resolve_hits_kernel(SceneDev S, const trq_ray* __restrict__ rays, trq_hit* hits,
     io[0] = o0; io[1] = o1;
 }
 
-// trq_hit -> trq_hit16 (for the paths that do not produce it directly: the reference-layout kernel)
-__global__ void __launch_bounds__(256)
-pack_hit16_kernel(const trq_hit* __restrict__ hits, float4* __restrict__ out, uint64_t n, const unsigned long long* __restrict__ nPtr) {
-    const uint64_t i = (uint64_t)blockIdx.x * blockDim.x + threadIdx.x;
-    if (i >= live_count(n, nPtr)) return;
-    const float4* in = reinterpret_cast<const float4*>(hits + i);
-    out[i] = pack_hit16(in[0], in[1]);
-}
-
 // Waits (on the stream) until every rank has published `step`; gives up after timeoutNs and raises *status.
 __global__ void gather_wait_kernel(const unsigned long long* flags, uint32_t world, unsigned long long step,
                                    unsigned long long timeoutNs, volatile unsigned int* status) {
@@ -935,62 +875,6 @@ expand_hits_kernel(SceneDev S, const trq_ray* __restrict__ rays, const trq_hit* 
         out.front = s.front; out.material = s.material;
     }
     recs[i] = out;
-}
-
-// ---------------------------------------------------------------------------------------------
-// derive the packed layout from the reference-layout buffers (one thread per BVH node)
-__global__ void __launch_bounds__(256)
-pack_scene_kernel(const RefBVH* __restrict__ bvh, const uint32_t* __restrict__ ref, uint32_t nNode,
-                  const RefVertex* __restrict__ verts, const uint32_t* __restrict__ idx,
-                  const RefSphere* __restrict__ spheres, const RefSquare* __restrict__ squares,
-                  float4* __restrict__ nodes, float4* __restrict__ tris, float4* __restrict__ sph, float4* __restrict__ sq,
-                  float4* __restrict__ triN, float4* __restrict__ topSoA, uint32_t topStride) {
-    const uint32_t i = blockIdx.x * blockDim.x + threadIdx.x;
-    if (i >= nNode) return;
-    const uint32_t my = ref[i];
-    const uint32_t kind = TRQ_REF_KIND(my), slot = TRQ_REF_INDEX(my);
-    if (my == TRQ_REF_DONE_WORD) return;                      // unreachable node
-    if (kind == REF_INTERIOR) {
-        const uint32_t l = bvh[i].left, r = bvh[i].right;
-        const RefAABB lb = bvh[l].bBOX, rb = bvh[r].bBOX;
-        float4* out = nodes + (size_t)slot * 4u;
-        out[0] = make_float4(lb.mini[0], lb.mini[1], lb.mini[2], __uint_as_float(ref[l]));
-        out[1] = make_float4(lb.maxi[0], lb.maxi[1], lb.maxi[2], __uint_as_float(ref[r]));
-        out[2] = make_float4(rb.mini[0], rb.mini[1], rb.mini[2], 0.0f);
-        out[3] = make_float4(rb.maxi[0], rb.maxi[1], rb.maxi[2], 0.0f);
-        if (slot < topStride) {                                 // quarter-major copy of the breadth-first top block (smem staging source)
-#pragma unroll
-            for (uint32_t q = 0; q < 4; ++q) topSoA[(size_t)q * topStride + slot] = out[q];
-        }
-    } else if (kind == REF_TRI) {
-        const uint32_t p = bvh[i].pIndex;
-        const f3 v0 = ld3(verts[idx[3 * p]].v), v1 = ld3(verts[idx[3 * p + 1]].v), v2 = ld3(verts[idx[3 * p + 2]].v);
-        const f3 e1 = sub3(v1, v0), e2 = sub3(v2, v0);       // Triangle.hh:43-44
-        float4* out = tris + (size_t)slot * TRQ_TRI_STRIDE;
-        out[0] = make_float4(v0.x, v0.y, v0.z, __uint_as_float(i));
-        out[1] = make_float4(e1.x, e1.y, e1.z, 0.0f);
-        out[2] = make_float4(e2.x, e2.y, e2.z, 0.0f);
-        // what a finished triangle hit needs beyond (t, u, v): the vertex normals for checkFace, and its ids
-        const f3 n0 = ld3(verts[idx[3 * p]].n), n1 = ld3(verts[idx[3 * p + 1]].n), n2 = ld3(verts[idx[3 * p + 2]].n);
-        float4* on = triN + (size_t)slot * 4u;
-        on[0] = make_float4(n0.x, n0.y, n0.z, __uint_as_float(i));
-        on[1] = make_float4(n1.x, n1.y, n1.z, __uint_as_float(p));
-        on[2] = make_float4(n2.x, n2.y, n2.z, 0.0f);
-        on[3] = make_float4(0.0f, 0.0f, 0.0f, 0.0f);
-    } else if (kind == REF_SPHERE) {
-        const RefSphere* s = &spheres[bvh[i].pIndex];
-        float4* out = sph + (size_t)slot * 2u;
-        out[0] = make_float4(s->center[0], s->center[1], s->center[2], s->radius);
-        out[1] = make_float4(__uint_as_float(i), __uint_as_float(bvh[i].pIndex), __uint_as_float(s->material), 0.0f);
-    } else if (kind == REF_SQUARE) {
-        const RefSquare* q = &squares[bvh[i].pIndex];
-        float4* out = sq + (size_t)slot * TRQ_SQ_STRIDE;
-        const uint32_t axes = (uint32_t)q->axis_i | ((uint32_t)q->axis_j << 8) | ((uint32_t)q->axis_k << 16);
-        out[0] = make_float4(q->range_i[0], q->range_i[1], q->range_j[0], q->range_j[1]);
-        out[1] = make_float4(q->value_k, __uint_as_float(axes), __uint_as_float(q->material), __uint_as_float(i));
-        out[2] = make_float4(__uint_as_float(bvh[i].pIndex), 0.0f, 0.0f, 0.0f);
-        out[3] = make_float4(0.0f, 0.0f, 0.0f, 0.0f);
-    }
 }
 
 }  // namespace trq

@@ -79,7 +79,6 @@ constexpr int kQueueRing = 4096;           // queue heads of eager launches, han
                                            // must not run at the same time (trq_trace in include/tracer_rq.h)
 constexpr int kStageBufs = 4;
 constexpr int kProfRing = 64;
-constexpr uint32_t kTopMax = 2047;         // interior nodes numbered breadth-first at the front (11 full levels)
 constexpr size_t kSmemPerSM = 228u * 1024u, kSmemPerBlockMax = 227u * 1024u, kSmemBlockReserve = 1024u;
 constexpr size_t kSmemDynamicMax = kSmemPerBlockMax - 1024u;   // dynamic part: the kernel also has a few static bytes (mbarrier)
 
@@ -112,38 +111,56 @@ constexpr int kNumCfgs = (int)(sizeof(kCfgs) / sizeof(kCfgs[0]));
 #define TRQ_MAX_RAYS_PER_LAUNCH (1ull << 31)
 #endif
 
+// Scene arrays come from the per-device pool that keeps its memory (host/scratch.h): a scene created after another one of
+// similar size was destroyed gets its memory back without a cudaMalloc (about 1 ms each for these sizes: 15 of the 22 ms
+// of a 1 M-triangle trq_scene_create_device before). trq_device_trim() hands cached memory back to the driver.
+cudaError_t pool_malloc(void** p, size_t bytes) {
+    int dev = 0;
+    cudaError_t e = cudaGetDevice(&dev);
+    if (e != cudaSuccess) return e;
+    cudaMemPool_t pool = trq::scratch_pool(dev);
+    return pool ? cudaMallocFromPoolAsync(p, bytes, pool, nullptr) : cudaMalloc(p, bytes);
+}
+void pool_free(void* p) { if (p) cudaFreeAsync(p, nullptr); }
+
+// One launch configuration for one tree: staged top-of-tree nodes, dynamic shared memory, resident CTAs per SM [any][format]
+struct CfgState { uint32_t topCount = 0, stackDepth = 0; size_t smem = 0; int blocksPerSM[2][2] = {}; bool usable = false; };
+
+// The records a rebuild keeps: device copies of the reference-layout lists (struct Primitive) and their lengths.
+struct SceneRecords {
+    RefSphere* spheres = nullptr; RefSquare* squares = nullptr; RefCube* cubes = nullptr; RefVertex* verts = nullptr; uint32_t* idx = nullptr;
+    uint32_t nSphere = 0, nSquare = 0, nCube = 0, nVert = 0, nTri = 0;   // records in the lists (info counts leaves)
+    void release() { pool_free(spheres); pool_free(squares); pool_free(cubes); pool_free(verts); pool_free(idx); *this = SceneRecords(); }
+};
+
+// The tree and everything derived from it: what a rebuild replaces whole.
+struct PackedTree {
+    RefBVH*   bvh = nullptr;
+    uint32_t* ref = nullptr;      // packed reference of every bvhList node (kept for refits)
+    float4 *nodes = nullptr, *tris = nullptr, *sph = nullptr, *sq = nullptr, *triN = nullptr, *topSoA = nullptr;   // packed_layout.cuh
+    trq_scene_info_t info{};
+    uint32_t nSqLeaf = 0;         // square leaves (info.nSquare counts records)
+    uint32_t rootRef = 0, stackDepth = 1;
+    float rootMin[3] = {}, rootMax[3] = {};
+    bool largeTree = false;       // packed tree > 2 x L2: incoherent batches are worth ordering (automatic TRQ_SORT_RAYS)
+    int leaves = 0;               // LEAVES_*: which leaf types the tree has (selects the kernels without the other types' code)
+    uint32_t maxPIndex = 0;       // largest leaf pIndex (trq_hit16 packs it into 28 bits)
+    CfgState cfg[kNumCfgs];
+    int autoCfg = 0;
+    void release() {
+        pool_free(bvh); pool_free(ref); pool_free(nodes); pool_free(tris); pool_free(sph); pool_free(sq); pool_free(triN); pool_free(topSoA);
+        *this = PackedTree();
+    }
+};
+
 }  // namespace
 
 struct trq_scene {
     int device = 0;
     int numSMs = 0;
-    trq_scene_info_t info{};
-    // reference-layout device copies (struct Primitive)
-    RefSphere* d_spheres = nullptr;
-    RefSquare* d_squares = nullptr;
-    RefCube*   d_cubes = nullptr;
-    RefVertex* d_verts = nullptr;
-    uint32_t*  d_idx = nullptr;
-    RefBVH*    d_bvh = nullptr;
-    // packed layout
-    float4* d_nodes = nullptr;
-    float4* d_tris = nullptr;
-    float4* d_sph = nullptr;
-    float4* d_sq = nullptr;
-    float4* d_triN = nullptr;
-    float4* d_topSoA = nullptr;
-    uint32_t* d_ref = nullptr;    // packed reference of every bvhList node (kept for refits)
-    uint32_t nNode = 0, nVert = 0, topStride = 0;
-    uint32_t listSphere = 0, listSquare = 0, listCube = 0, listTri = 0;   // records in the arrays (info counts leaves)
-    SceneDev dev{};
-    uint32_t stackDepth = 1;
-    bool largeTree = false;       // packed tree > 2 x L2: incoherent batches are worth ordering (automatic TRQ_SORT_RAYS)
-    int leaves = 0;               // LEAVES_*: which leaf types the tree has (selects the kernels without the other types' code)
-    uint32_t maxPIndex = 0;       // largest leaf pIndex (trq_hit16 packs it into 28 bits)
-    // per launch configuration: staged top-of-tree nodes, dynamic shared memory, resident CTAs per SM [any][format]
-    struct CfgState { uint32_t topCount = 0, stackDepth = 0; size_t smem = 0; int blocksPerSM[2][2] = {}; bool usable = false; };
-    CfgState cfg[kNumCfgs];
-    int defaultCfg = 0, autoCfg = 0;
+    SceneRecords rec;
+    PackedTree tree;
+    int defaultCfg = 0;
     bool userCfg = false;         // defaultCfg was chosen with trq_scene_set_kernel_config (kept by a rebuild while usable)
     // stream-ordered scratch for TRQ_SORT_RAYS: a private pool that keeps its memory across synchronisations
     // (the device's default pool hands it back at every sync and re-maps 64 MB on the next sorted launch)
@@ -168,24 +185,21 @@ struct trq_scene {
 
 namespace {
 
-// Scene arrays come from the per-device pool that keeps its memory (host/scratch.h): a scene created after another one of
-// similar size was destroyed gets its memory back without a cudaMalloc (about 1 ms each for these sizes: 15 of the 22 ms
-// of a 1 M-triangle trq_scene_create_device before). trq_device_trim() hands cached memory back to the driver.
-cudaError_t pool_malloc(void** p, size_t bytes) {
-    int dev = 0;
-    cudaError_t e = cudaGetDevice(&dev);
-    if (e != cudaSuccess) return e;
-    cudaMemPool_t pool = trq::scratch_pool(dev);
-    return pool ? cudaMallocFromPoolAsync(p, bytes, pool, nullptr) : cudaMalloc(p, bytes);
+// The kernels' view of a scene (a kernel parameter)
+SceneDev scene_dev(const trq_scene* s) {
+    const SceneRecords& r = s->rec;
+    const PackedTree& t = s->tree;
+    SceneDev d{r.spheres, r.squares, r.cubes, r.verts, r.idx, t.bvh, t.nodes, t.topSoA, t.info.topNodes, t.tris, t.sph, t.sq, t.triN, t.rootRef};
+    for (int k = 0; k < 3; ++k) { d.rootMin[k] = t.rootMin[k]; d.rootMax[k] = t.rootMax[k]; }
+    d.nNode = t.info.nNode;
+    return d;
 }
-void pool_free(void* p) { if (p) cudaFreeAsync(p, nullptr); }
 
 void free_scene(trq_scene* s) {
     if (!s) return;
     cudaDeviceSynchronize();                                   // launches on any stream may still read the arrays
-    pool_free(s->d_spheres); pool_free(s->d_squares); pool_free(s->d_cubes);
-    pool_free(s->d_verts); pool_free(s->d_idx); pool_free(s->d_bvh);
-    pool_free(s->d_nodes); pool_free(s->d_tris); pool_free(s->d_sph); pool_free(s->d_sq); pool_free(s->d_triN); pool_free(s->d_topSoA); pool_free(s->d_ref);
+    s->rec.release();
+    s->tree.release();
     pool_free(s->d_queues);
     for (int b = 0; b < kStageBufs; ++b) {
         cudaFree(s->d_stageRays[b]); cudaFree(s->d_stageHits[b]);
@@ -197,24 +211,34 @@ void free_scene(trq_scene* s) {
 }
 
 template <typename T>
-int upload(T** dst, const void* src, size_t count) {
+int upload(T** dst, const void* src, size_t count, cudaMemcpyKind kind) {
     *dst = nullptr;
     if (count == 0) return TRQ_OK;
     TRQ_CUDA(pool_malloc((void**)dst, count * sizeof(T)));
-    TRQ_CUDA(cudaMemcpy(*dst, src, count * sizeof(T), cudaMemcpyHostToDevice));
+    TRQ_CUDA(cudaMemcpyAsync(*dst, src, count * sizeof(T), kind, nullptr));
+    return TRQ_OK;
+}
+
+int upload_records(SceneRecords& r, const trq_scene_desc* d, cudaMemcpyKind kind) {
+    int rc;
+    if ((rc = upload(&r.spheres, d->sphereList, d->nSphere, kind)) != TRQ_OK) return rc;
+    if ((rc = upload(&r.squares, d->squareList, d->nSquare, kind)) != TRQ_OK) return rc;
+    if ((rc = upload(&r.cubes, d->cubeList, d->nCube, kind)) != TRQ_OK) return rc;
+    if ((rc = upload(&r.verts, d->triList, d->nVert, kind)) != TRQ_OK) return rc;
+    if ((rc = upload(&r.idx, d->idxList, (size_t)d->nTri * 3, kind)) != TRQ_OK) return rc;
+    r.nSphere = d->nSphere; r.nSquare = d->nSquare; r.nCube = d->nCube; r.nVert = d->nVert; r.nTri = d->nTri;
     return TRQ_OK;
 }
 
 // Walk the tree once on the host: validate the layout contract and assign every reachable node its packed reference.
-// Leaves are numbered per kind in depth-first order (left child first). Interior nodes: the first kTopMax of a
+// Leaves are numbered per kind in depth-first order (left child first). Interior nodes: the first packed::kTopMax of a
 // breadth-first walk come first, in that order (the block a kernel may stage in shared memory); the rest follow in
-// depth-first order.
-int plan_layout(const trq_scene_desc* d, std::vector<uint32_t>& ref, trq_scene_info_t& info, uint32_t& maxPIndex) {
+// depth-first order. Sets t's counts, root and maxPIndex.
+int plan_layout(const trq_scene_desc* d, std::vector<uint32_t>& ref, PackedTree& t) {
     const RefBVH* N = (const RefBVH*)d->bvhList;
     const uint32_t n = d->nNode;
     ref.assign(n, TRQ_REF_DONE_WORD);
-    uint32_t nTriLeaf = 0, nSphLeaf = 0, nSqLeaf = 0, nLeaf = 0, maxDepth = 0;
-    maxPIndex = 0;
+    uint32_t nTriLeaf = 0, nSphLeaf = 0, nSqLeaf = 0, nLeaf = 0, maxDepth = 0, maxPIndex = 0;
     std::vector<uint32_t> interiorDfs;                       // interior nodes in depth-first order
     struct Item { uint32_t node, depth; };
     std::vector<Item> stack;
@@ -276,12 +300,12 @@ int plan_layout(const trq_scene_desc* d, std::vector<uint32_t>& ref, trq_scene_i
     uint32_t nTop = 0;
     if (nInterior) {
         std::vector<uint32_t> bfs;
-        bfs.reserve(kTopMax);
+        bfs.reserve(packed::kTopMax);
         bfs.push_back(0u);
         for (size_t head = 0; head < bfs.size(); ++head) {
             const RefBVH& b = N[bfs[head]];
-            if (bfs.size() < kTopMax && N[b.left].pType == TRQ_BVH) bfs.push_back(b.left);
-            if (bfs.size() < kTopMax && N[b.right].pType == TRQ_BVH) bfs.push_back(b.right);
+            if (bfs.size() < packed::kTopMax && N[b.left].pType == TRQ_BVH) bfs.push_back(b.left);
+            if (bfs.size() < packed::kTopMax && N[b.right].pType == TRQ_BVH) bfs.push_back(b.right);
         }
         nTop = (uint32_t)bfs.size();
         for (uint32_t k = 0; k < nTop; ++k) ref[bfs[k]] = TRQ_MAKE_REF(REF_INTERIOR, k) | 0x10000000u;   // bit 28: numbered (cleared below)
@@ -291,10 +315,13 @@ int plan_layout(const trq_scene_desc* d, std::vector<uint32_t>& ref, trq_scene_i
             else ref[i] = TRQ_MAKE_REF(REF_INTERIOR, next++);
         }
     }
+    trq_scene_info_t& info = t.info;
     info.nNode = n; info.nInterior = nInterior; info.nLeaf = nLeaf; info.maxDepth = maxDepth;
     info.nTri = nTriLeaf; info.nSphere = nSphLeaf;
     info.nSquare = d->nSquare; info.nCube = d->nCube;
     info.topNodes = nTop;
+    t.nSqLeaf = nSqLeaf; t.maxPIndex = maxPIndex; t.rootRef = ref[0];
+    for (int k = 0; k < 3; ++k) { t.rootMin[k] = N[0].bBOX.mini[k]; t.rootMax[k] = N[0].bBOX.maxi[k]; }
     return TRQ_OK;
 }
 
@@ -302,7 +329,7 @@ int plan_layout(const trq_scene_desc* d, std::vector<uint32_t>& ref, trq_scene_i
 int pick_cfg(const trq_scene* s) {
     static const int env = [] { const char* e = getenv("TRQ_CFG"); return e ? atoi(e) : -1; }();
     int c = (env >= 0 && env < kNumCfgs) ? env : s->defaultCfg;
-    if (!s->cfg[c].usable) c = 0;
+    if (!s->tree.cfg[c].usable) c = 0;
     return c;
 }
 
@@ -322,6 +349,7 @@ int launch_trace(trq_scene* s, const trq_ray* d_rays, uint64_t n, uint32_t flags
         return TRQ_OK;
     }
     const bool any = (flags & TRQ_TRACE_ANY) != 0;
+    const SceneDev dev = scene_dev(s);
     cudaEvent_t* prof = nullptr;
     if (s->profile) {
         std::lock_guard<std::mutex> lock(s->profMutex);
@@ -336,10 +364,10 @@ int launch_trace(trq_scene* s, const trq_ray* d_rays, uint64_t n, uint32_t flags
         const unsigned block = 128;
         const uint64_t grid = (n + block - 1) / block;
         if (grid > 0x7fffffffull) return trq::fail(TRQ_ERR_INVALID, "trq_trace: batch too large");
-        if (any) trace_reflayout_kernel<true><<<(unsigned)grid, block, 0, st>>>(s->dev, d_rays, (trq_hit*)d_hits, n, nPtr);
-        else     trace_reflayout_kernel<false><<<(unsigned)grid, block, 0, st>>>(s->dev, d_rays, (trq_hit*)d_hits, n, nPtr);
+        if (any) trace_reflayout_kernel<true><<<(unsigned)grid, block, 0, st>>>(dev, d_rays, (trq_hit*)d_hits, n, nPtr);
+        else     trace_reflayout_kernel<false><<<(unsigned)grid, block, 0, st>>>(dev, d_rays, (trq_hit*)d_hits, n, nPtr);
         if (prof) TRQ_CUDA(cudaEventRecord(prof[1], st));
-        resolve_hits_kernel<<<(unsigned)((n + 255) / 256), 256, 0, st>>>(s->dev, d_rays, (trq_hit*)d_hits, n, nPtr);
+        resolve_hits_kernel<<<(unsigned)((n + 255) / 256), 256, 0, st>>>(dev, d_rays, (trq_hit*)d_hits, n, nPtr);
         g_launches += 2;
     } else {
         static const uint32_t refillMin = [] {
@@ -357,7 +385,7 @@ int launch_trace(trq_scene* s, const trq_ray* d_rays, uint64_t n, uint32_t flags
         // takes (nearly) all of an SM's shared memory could be locked out by a resident sender CTA that waits for it
         const int c = tileDone ? 0 : pick_cfg(s);
         const KernelCfg& K = kCfgs[c];
-        const trq_scene::CfgState& cs = s->cfg[c];
+        const CfgState& cs = s->tree.cfg[c];
         int perSM = cs.blocksPerSM[any ? 1 : 0][hit16 ? 1 : 0];                  // queried once, in trq_scene_create
         if (blocksPerSMOverride > 0 && blocksPerSMOverride < perSM) perSM = blocksPerSMOverride;
         uint64_t grid = (uint64_t)perSM * (uint64_t)s->numSMs;             // persistent: a multiple of the SM count
@@ -392,7 +420,7 @@ int launch_trace(trq_scene* s, const trq_ray* d_rays, uint64_t n, uint32_t flags
         const int autoEnv = autoStr ? atoi(autoStr) : -1;
         const bool sortRays = sortEnv >= 0 ? (sortEnv != 0) : ((flags & TRQ_SORT_RAYS) != 0);
         const bool autoSort = !sortRays && sortEnv < 0 && !(flags & TRQ_NO_SORT) && !tileDone && n >= (1ull << 20) &&
-                              (autoEnv >= 0 ? autoEnv != 0 : s->largeTree);
+                              (autoEnv >= 0 ? autoEnv != 0 : s->tree.largeTree);
         uint32_t* scratch = nullptr;
         if ((sortRays && n >= 65536) || autoSort) {
             const size_t words = (size_t)TRQ_SORT_BINS + 4 + 2 * (size_t)n;      // hist | ctrl | keys | order
@@ -402,16 +430,16 @@ int launch_trace(trq_scene* s, const trq_ray* d_rays, uint64_t n, uint32_t flags
             unsigned gb = (unsigned)((n + 255) / 256);
             if (gb > (unsigned)s->numSMs * 32u) gb = (unsigned)s->numSMs * 32u;   // grid-stride beyond that
             uint32_t* decide = autoSort ? ctrl : nullptr;
-            if (autoSort) { sort_probe_kernel<<<256, 256, 0, st>>>(s->dev, d_rays, n, nPtr, ctrl); g_launches++; }
-            sort_count_kernel<<<gb, 256, 0, st>>>(s->dev, d_rays, n, nPtr, keys, hist, decide);
+            if (autoSort) { sort_probe_kernel<<<256, 256, 0, st>>>(dev, d_rays, n, nPtr, ctrl); g_launches++; }
+            sort_count_kernel<<<gb, 256, 0, st>>>(dev, d_rays, n, nPtr, keys, hist, decide);
             sort_scan_kernel<<<1, 1024, 0, st>>>(hist, decide);
             sort_scatter_kernel<<<gb, 256, 0, st>>>(keys, n, nPtr, hist, order, decide);
             g_launches += 3;
             P.order = order;
             P.orderFlag = decide;
         }
-        void* args[2] = {(void*)&s->dev, (void*)&P};
-        TRQ_CUDA(cudaLaunchKernel(K.fn[s->leaves][any ? 1 : 0][hit16 ? 1 : 0], dim3((unsigned)grid), dim3((unsigned)K.block), args, cs.smem, st));
+        void* args[2] = {(void*)&dev, (void*)&P};
+        TRQ_CUDA(cudaLaunchKernel(K.fn[s->tree.leaves][any ? 1 : 0][hit16 ? 1 : 0], dim3((unsigned)grid), dim3((unsigned)K.block), args, cs.smem, st));
         g_launches++;
         if (ownHead) TRQ_CUDA(cudaFreeAsync(ownHead, st));
         if (scratch) TRQ_CUDA(cudaFreeAsync(scratch, st));
@@ -488,7 +516,7 @@ int trace_host(trq_scene* s, const trq_ray* rays, uint64_t n, uint32_t flags, vo
     std::lock_guard<std::mutex> lock(s->stageMutex);
     // a sorted chunk is only as coherent as it is large: C5 e2e 461 / 605 / 599 / 504 Mrays/s at 512K / 1M / 2M / 4M rays
     // (the same chunk size for a tree much larger than L2 without the hint: the automatic mode looks at batches of >= 2^20 rays)
-    const bool mayOrder = (flags & TRQ_SORT_RAYS) || (s->largeTree && !(flags & TRQ_NO_SORT));
+    const bool mayOrder = (flags & TRQ_SORT_RAYS) || (s->tree.largeTree && !(flags & TRQ_NO_SORT));
     const uint64_t want = mayOrder ? 2 * chunkRays : chunkRays;
     const uint64_t chunk = n < want ? n : want;
     int rc = ensure_staging(s, chunk);
@@ -550,15 +578,6 @@ void trq_debug_stats(unsigned long long* out, int reset) {
 
 namespace {
 
-template <typename T>
-int upload_from(T** dst, const void* src, size_t count, cudaMemcpyKind kind) {
-    *dst = nullptr;
-    if (count == 0) return TRQ_OK;
-    TRQ_CUDA(pool_malloc((void**)dst, count * sizeof(T)));
-    TRQ_CUDA(cudaMemcpyAsync(*dst, src, count * sizeof(T), kind, nullptr));
-    return TRQ_OK;
-}
-
 int check_desc(const trq_scene_desc* d, trq_scene** out, const char* who) {
     if (!d || !out) return trq::fail(TRQ_ERR_INVALID, "%s: NULL argument", who);
     *out = nullptr;
@@ -569,13 +588,13 @@ int check_desc(const trq_scene_desc* d, trq_scene** out, const char* who) {
     return TRQ_OK;
 }
 
-// Launch configurations for the scene's tree (s->stackDepth, s->leaves set): per-CTA shared memory = staged top-of-tree nodes +
-// far-child stack + cold per-ray words, resident CTAs per SM, usability; and the automatic choice s->autoCfg.
-int size_configs(trq_scene* s, const trq_scene_info_t& info) {
+// Launch configurations for the tree (t.stackDepth, t.leaves set): per-CTA shared memory = staged top-of-tree nodes +
+// far-child stack + cold per-ray words, resident CTAs per SM, usability; and the automatic choice t.autoCfg.
+int size_configs(PackedTree& t) {
     for (int c = 0; c < kNumCfgs; ++c) {
         const KernelCfg& K = kCfgs[c];
-        trq_scene::CfgState& cs = s->cfg[c];
-        cs.stackDepth = s->stackDepth;
+        CfgState& cs = t.cfg[c];
+        cs.stackDepth = t.stackDepth;
         const size_t perRay = ((size_t)cs.stackDepth + COLD_WORDS) * K.block * sizeof(uint32_t);
         size_t budget = kSmemPerSM / (size_t)K.minb - kSmemBlockReserve;
         if (budget > kSmemDynamicMax) budget = kSmemDynamicMax;
@@ -583,17 +602,17 @@ int size_configs(trq_scene* s, const trq_scene_info_t& info) {
         if (K.top) {
             const char* topStr = getenv("TRQ_TOP_NODES");               // read per scene: the sweeps create one scene per value
             const int topEnv = topStr ? atoi(topStr) : -1;
-            if (budget > perRay) cs.topCount = (uint32_t)((budget - perRay) / 64);
-            if (cs.topCount > info.topNodes) cs.topCount = info.topNodes;
+            if (budget > perRay) cs.topCount = (uint32_t)((budget - perRay) / packed::kNodeBytes);
+            if (cs.topCount > t.info.topNodes) cs.topCount = t.info.topNodes;
             if (topEnv >= 0 && (uint32_t)topEnv < cs.topCount) cs.topCount = (uint32_t)topEnv;
         }
-        cs.smem = perRay + (size_t)cs.topCount * 64;
+        cs.smem = perRay + (size_t)cs.topCount * packed::kNodeBytes;
         cs.usable = cs.smem <= kSmemDynamicMax && !(K.top && cs.topCount == 0 && c != 0);
         if (!cs.usable) continue;
         cudaError_t e = cudaSuccess;
         for (int a = 0; a < 2 && e == cudaSuccess; ++a)
             for (int f = 0; f < 2 && e == cudaSuccess; ++f) {
-                const void* fn = K.fn[s->leaves][a][f];
+                const void* fn = K.fn[t.leaves][a][f];
                 if (cs.smem > 48 * 1024) e = cudaFuncSetAttribute(fn, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)kSmemDynamicMax);
                 if (e == cudaSuccess) e = cudaOccupancyMaxActiveBlocksPerMultiprocessor(&cs.blocksPerSM[a][f], fn, K.block, cs.smem);
                 if (e == cudaSuccess && cs.blocksPerSM[a][f] < 1) cs.usable = false;
@@ -604,79 +623,59 @@ int size_configs(trq_scene* s, const trq_scene_info_t& info) {
             cs.usable = false;
         }
     }
-    if (!s->cfg[0].usable) return trq::fail(TRQ_ERR_CUDA, "trace_packed_kernel does not fit on an SM (smem %zu)", s->cfg[0].smem);
+    if (!t.cfg[0].usable) return trq::fail(TRQ_ERR_CUDA, "trace_packed_kernel does not fit on an SM (smem %zu)", t.cfg[0].smem);
     // Staging pays when the staged block IS the tree (C1: +2-15 %); with the leaf-specialised kernels it no longer does when
     // only the top levels fit (C2 / the reference's Cornell mix: -3 to -6 %), and it loses clearly on 1 M+ triangle scenes
     // (profiles/r02_top_of_tree_experiment.txt): chosen only for trees that fit whole.
-    s->autoCfg = 0;
+    t.autoCfg = 0;
     for (int c = 1; c < kNumCfgs; ++c)
-        if (kCfgs[c].top && s->cfg[c].usable && info.nInterior <= s->cfg[c].topCount) { s->autoCfg = c; break; }
+        if (kCfgs[c].top && t.cfg[c].usable && t.info.nInterior <= t.cfg[c].topCount) { t.autoCfg = c; break; }
     return TRQ_OK;
 }
 
-// The part of scene creation that is the same for host and device input: the six reference arrays are resident
-// (s->d_*), every node has its packed reference in s->d_ref, `info` holds the counts. Allocates and derives the packed
-// layout on the device and sizes the launch configurations.
-int finish_scene(trq_scene* s, const trq_scene_desc* d, trq_scene_info_t info, uint32_t nSqLeaf, uint32_t rootRef,
-                 const float rootMin[3], const float rootMax[3]) {
-    const int device = s->device;
+// Derives t's packed arrays from its nodes and the records, on the device (creation and refit).
+void launch_pack(const PackedTree& t, const SceneRecords& r) {
+    const unsigned block = 256, grid = (t.info.nNode + block - 1) / block;
+    pack_scene_kernel<<<grid, block>>>(t.bvh, t.ref, t.info.nNode, r.verts, r.idx, r.spheres, r.squares,
+                                       t.nodes, t.tris, t.sph, t.sq, t.triN, t.topSoA, t.info.topNodes);
+    g_launches++;
+}
+
+// The part of building a tree that is the same for every path: t.bvh and t.ref are resident, t's counts, root and maxPIndex
+// are set (plan_layout or plan_tree). Allocates the packed arrays, derives them on the device and sizes the launch
+// configurations.
+int pack_tree(PackedTree& t, const SceneRecords& r, int device) {
     StageTimer tm;
-    const size_t nodeBytes = (size_t)info.nInterior * 64, triBytes = (size_t)info.nTri * 16 * TRQ_TRI_STRIDE, sphBytes = (size_t)info.nSphere * 32;
-    const size_t sqBytes = (size_t)nSqLeaf * 16 * TRQ_SQ_STRIDE;
-    if (nodeBytes && pool_malloc((void**)&s->d_nodes, nodeBytes) != cudaSuccess) return trq::fail(TRQ_ERR_CUDA, "cudaMalloc(nodes %zu B) failed", nodeBytes);
-    if (triBytes && pool_malloc((void**)&s->d_tris, triBytes) != cudaSuccess) return trq::fail(TRQ_ERR_CUDA, "cudaMalloc(tris %zu B) failed", triBytes);
-    if (sphBytes && pool_malloc((void**)&s->d_sph, sphBytes) != cudaSuccess) return trq::fail(TRQ_ERR_CUDA, "cudaMalloc(spheres %zu B) failed", sphBytes);
-    if (sqBytes && pool_malloc((void**)&s->d_sq, sqBytes) != cudaSuccess) return trq::fail(TRQ_ERR_CUDA, "cudaMalloc(squares %zu B) failed", sqBytes);
-    const size_t triNBytes = (size_t)info.nTri * 64;
-    if (triNBytes && pool_malloc((void**)&s->d_triN, triNBytes) != cudaSuccess) return trq::fail(TRQ_ERR_CUDA, "cudaMalloc(triangle normals %zu B) failed", triNBytes);
-    if (info.topNodes && pool_malloc((void**)&s->d_topSoA, (size_t)info.topNodes * 64) != cudaSuccess) return trq::fail(TRQ_ERR_CUDA, "cudaMalloc(top-of-tree block) failed");
-    if (!s->d_queues) {                                        // (a rebuild's staging scene borrows the scene's heads)
-        if (pool_malloc((void**)&s->d_queues, kQueueRing * sizeof(QueueHead)) != cudaSuccess) return trq::fail(TRQ_ERR_CUDA, "cudaMalloc(queue heads) failed");
-        if (cudaMemsetAsync(s->d_queues, 0, kQueueRing * sizeof(QueueHead), nullptr) != cudaSuccess) return trq::fail(TRQ_ERR_CUDA, "cudaMemset(queue heads) failed");
-    }
-
-    s->nNode = d->nNode; s->nVert = d->nVert; s->topStride = info.topNodes;
-    s->listSphere = d->nSphere; s->listSquare = d->nSquare; s->listCube = d->nCube; s->listTri = d->nTri;
+    trq_scene_info_t& info = t.info;
+    const packed::Sizes b = packed::sizes(info.nInterior, info.nTri, info.nSphere, t.nSqLeaf, info.topNodes);
+    if (b.nodes && pool_malloc((void**)&t.nodes, b.nodes) != cudaSuccess) return trq::fail(TRQ_ERR_CUDA, "cudaMalloc(nodes %zu B) failed", b.nodes);
+    if (b.tris && pool_malloc((void**)&t.tris, b.tris) != cudaSuccess) return trq::fail(TRQ_ERR_CUDA, "cudaMalloc(tris %zu B) failed", b.tris);
+    if (b.sph && pool_malloc((void**)&t.sph, b.sph) != cudaSuccess) return trq::fail(TRQ_ERR_CUDA, "cudaMalloc(spheres %zu B) failed", b.sph);
+    if (b.sq && pool_malloc((void**)&t.sq, b.sq) != cudaSuccess) return trq::fail(TRQ_ERR_CUDA, "cudaMalloc(squares %zu B) failed", b.sq);
+    if (b.triN && pool_malloc((void**)&t.triN, b.triN) != cudaSuccess) return trq::fail(TRQ_ERR_CUDA, "cudaMalloc(triangle normals %zu B) failed", b.triN);
+    if (b.top && pool_malloc((void**)&t.topSoA, b.top) != cudaSuccess) return trq::fail(TRQ_ERR_CUDA, "cudaMalloc(top-of-tree block) failed");
     TRQ_LAP(tm, "allocate packed arrays");
-    {
-        const unsigned block = 256, grid = (d->nNode + block - 1) / block;
-        pack_scene_kernel<<<grid, block>>>(s->d_bvh, s->d_ref, d->nNode, s->d_verts, s->d_idx, s->d_spheres, s->d_squares,
-                                           s->d_nodes, s->d_tris, s->d_sph, s->d_sq, s->d_triN, s->d_topSoA, info.topNodes);
-        g_launches++;
-        cudaError_t e = cudaDeviceSynchronize();
-        if (e != cudaSuccess) return trq::fail(TRQ_ERR_CUDA, "pack_scene_kernel failed: %s", cudaGetErrorString(e));
-    }
-
+    launch_pack(t, r);
+    cudaError_t e = cudaDeviceSynchronize();
+    if (e != cudaSuccess) return trq::fail(TRQ_ERR_CUDA, "pack_scene_kernel failed: %s", cudaGetErrorString(e));
     TRQ_LAP(tm, "pack_scene_kernel");
-    s->dev.spheres = s->d_spheres; s->dev.squares = s->d_squares; s->dev.cubes = s->d_cubes;
-    s->dev.verts = s->d_verts; s->dev.idx = s->d_idx; s->dev.bvh = s->d_bvh;
-    s->dev.topSoA = s->d_topSoA; s->dev.topStride = info.topNodes;
-    s->dev.nodes = s->d_nodes; s->dev.tris = s->d_tris; s->dev.sph = s->d_sph; s->dev.sq = s->d_sq; s->dev.triN = s->d_triN;
-    s->dev.rootRef = rootRef;
-    for (int k = 0; k < 3; ++k) { s->dev.rootMin[k] = rootMin[k]; s->dev.rootMax[k] = rootMax[k]; }
-    s->dev.nNode = d->nNode;
-    s->stackDepth = info.maxDepth + 1;
+    t.stackDepth = info.maxDepth + 1;
     // (a leaf of unknown pType, which dispatches to `default: break`, also selects the general kernels)
-    s->leaves = info.nLeaf == info.nTri ? LEAVES_TRI : (info.nLeaf == info.nTri + info.nSphere ? LEAVES_TRI_SPHERE : LEAVES_ALL);
-    s->scratchPool = trq::scratch_pool(device);                // TRQ_SORT_RAYS scratch: stream-ordered, kept between launches
-    if (!s->scratchPool) return trq::fail(TRQ_ERR_CUDA, "cudaMemPoolCreate failed");
-    TRQ_LAP(tm, "scratch pool");
-    int rc = size_configs(s, info);
+    t.leaves = info.nLeaf == info.nTri ? LEAVES_TRI : (info.nLeaf == info.nTri + info.nSphere ? LEAVES_TRI_SPHERE : LEAVES_ALL);
+    int rc = size_configs(t);
     if (rc != TRQ_OK) return rc;
     TRQ_LAP(tm, "kernel configurations");
-    s->defaultCfg = s->autoCfg;
 
-    info.bytesReferenceLayout = (uint64_t)d->nSphere * sizeof(RefSphere) + (uint64_t)d->nSquare * sizeof(RefSquare) +
-                                (uint64_t)d->nCube * sizeof(RefCube) + (uint64_t)d->nVert * sizeof(RefVertex) +
-                                (uint64_t)d->nTri * 12 + (uint64_t)d->nNode * sizeof(RefBVH);
-    info.bytesPacked = nodeBytes + triBytes + sphBytes + sqBytes + triNBytes;
+    info.bytesReferenceLayout = (uint64_t)r.nSphere * sizeof(RefSphere) + (uint64_t)r.nSquare * sizeof(RefSquare) +
+                                (uint64_t)r.nCube * sizeof(RefCube) + (uint64_t)r.nVert * sizeof(RefVertex) +
+                                (uint64_t)r.nTri * 12 + (uint64_t)info.nNode * sizeof(RefBVH);
+    info.bytesPacked = b.nodes + b.tris + b.sph + b.sq + b.triN;
     {
         int l2 = 0;
         if (cudaDeviceGetAttribute(&l2, cudaDevAttrL2CacheSize, device) != cudaSuccess) { cudaGetLastError(); l2 = 0; }
-        s->largeTree = l2 > 0 && (uint64_t)(nodeBytes + triBytes + sphBytes + sqBytes) > 2ull * (uint64_t)l2;   // what traversal touches
+        t.largeTree = l2 > 0 && (uint64_t)(b.nodes + b.tris + b.sph + b.sq) > 2ull * (uint64_t)l2;   // what traversal touches
     }
     info.device = device;
-    s->info = info;
     return TRQ_OK;
 }
 
@@ -689,6 +688,16 @@ int open_scene(int device, trq_scene** sOut, const char* who) {
     s->device = device;
     if (cudaDeviceGetAttribute(&s->numSMs, cudaDevAttrMultiProcessorCount, device) != cudaSuccess) { delete s; return trq::fail(TRQ_ERR_CUDA, "cudaDeviceGetAttribute failed"); }
     *sOut = s;
+    return TRQ_OK;
+}
+
+// What a scene keeps whatever its tree: the zeroed ray-queue heads of eager launches and the TRQ_SORT_RAYS scratch pool
+// (stream-ordered, kept between launches). Runs on the scene's device before the creation's first synchronisation.
+int open_queues(trq_scene* s) {
+    if (pool_malloc((void**)&s->d_queues, kQueueRing * sizeof(QueueHead)) != cudaSuccess) return trq::fail(TRQ_ERR_CUDA, "cudaMalloc(queue heads) failed");
+    if (cudaMemsetAsync(s->d_queues, 0, kQueueRing * sizeof(QueueHead), nullptr) != cudaSuccess) return trq::fail(TRQ_ERR_CUDA, "cudaMemset(queue heads) failed");
+    s->scratchPool = trq::scratch_pool(s->device);
+    if (!s->scratchPool) return trq::fail(TRQ_ERR_CUDA, "cudaMemPoolCreate failed");
     return TRQ_OK;
 }
 
@@ -706,29 +715,28 @@ const char* plan_error_text(uint32_t code) {
     }
 }
 
-// The device half of scene creation, shared by trq_scene_create_device and trq_scene_rebuild: s->d_bvh (d->nNode nodes),
-// s->d_idx and the other arrays are resident. The planning kernels (kernels/plan_scene.cuh) validate the tree and number it
-// into a new s->d_ref, 128 bytes of counters come back, and finish_scene derives the packed layout.
-int plan_and_finish(trq_scene* s, const trq_scene_desc* d, const char* who) {
+// Device planning, shared by trq_scene_create_device and trq_scene_rebuild: t.bvh (nNode nodes over the records r) is
+// resident. The planning kernels (kernels/plan_scene.cuh) validate the tree and number it into a new t.ref, and 128 bytes of
+// counters come back with t's counts, root and maxPIndex.
+int plan_tree(PackedTree& t, uint32_t n, const SceneRecords& r, int device, const char* who) {
     StageTimer tm;
-    const uint32_t n = d->nNode;
-    if (pool_malloc((void**)&s->d_ref, (size_t)n * sizeof(uint32_t)) != cudaSuccess) return trq::fail(TRQ_ERR_CUDA, "%s: cudaMalloc(refs) failed", who);
+    if (pool_malloc((void**)&t.ref, (size_t)n * sizeof(uint32_t)) != cudaSuccess) return trq::fail(TRQ_ERR_CUDA, "%s: cudaMalloc(refs) failed", who);
     plan::PlanInfo hostInfo;
     {
-        trq::PoolScratch mem(s->device, nullptr);
+        trq::PoolScratch mem(device, nullptr);
         plan::Counts* cnt; uint32_t *leafTotal, *arrivals, *pre, *topPos, *sortedPre; plan::PlanInfo* dInfo;
         if (!(mem.alloc(&cnt, n) && mem.alloc(&leafTotal, n) && mem.alloc(&arrivals, n) && mem.alloc(&pre, n) && mem.alloc(&topPos, n) &&
               mem.alloc(&sortedPre, 2048) && mem.alloc(&dInfo, 1)))
             return trq::fail(TRQ_ERR_NOMEM, "%s: out of device memory", who);
         cudaMemsetAsync(arrivals, 0, (size_t)n * 4); cudaMemsetAsync(topPos, 0, (size_t)n * 4);
         cudaMemsetAsync(cnt, 0, (size_t)n * sizeof(plan::Counts)); cudaMemsetAsync(leafTotal, 0, (size_t)n * 4);
-        cudaMemsetAsync(dInfo, 0, sizeof(plan::PlanInfo)); cudaMemsetAsync(s->d_ref, 0xff, (size_t)n * 4);
+        cudaMemsetAsync(dInfo, 0, sizeof(plan::PlanInfo)); cudaMemsetAsync(t.ref, 0xff, (size_t)n * 4);
         const unsigned grid = (n + 255) / 256;
-        plan::validate_kernel<<<grid, 256>>>(s->d_bvh, n, d->nSphere, d->nSquare, d->nCube, d->nTri, d->nVert, s->d_idx, dInfo);
-        plan::counts_kernel<<<grid, 256>>>(s->d_bvh, n, cnt, leafTotal, arrivals);
-        plan::number_kernel<<<grid, 256>>>(s->d_bvh, n, cnt, leafTotal, s->d_ref, pre, dInfo);
-        plan::top_block_kernel<<<1, 1024>>>(s->d_bvh, n, pre, topPos, sortedPre, dInfo);
-        plan::refs_kernel<<<grid, 256>>>(s->d_bvh, n, pre, topPos, sortedPre, s->d_ref, dInfo);
+        plan::validate_kernel<<<grid, 256>>>(t.bvh, n, r.nSphere, r.nSquare, r.nCube, r.nTri, r.nVert, r.idx, dInfo);
+        plan::counts_kernel<<<grid, 256>>>(t.bvh, n, cnt, leafTotal, arrivals);
+        plan::number_kernel<<<grid, 256>>>(t.bvh, n, cnt, leafTotal, t.ref, pre, dInfo);
+        plan::top_block_kernel<<<1, 1024>>>(t.bvh, n, pre, topPos, sortedPre, dInfo);
+        plan::refs_kernel<<<grid, 256>>>(t.bvh, n, pre, topPos, sortedPre, t.ref, dInfo);
         g_launches += 5;
         cudaError_t e = cudaMemcpy(&hostInfo, dInfo, sizeof hostInfo, cudaMemcpyDeviceToHost);
         if (e != cudaSuccess) return trq::fail(TRQ_ERR_CUDA, "%s: planning kernels failed: %s", who, cudaGetErrorString(e));
@@ -737,12 +745,13 @@ int plan_and_finish(trq_scene* s, const trq_scene_desc* d, const char* who) {
     if (hostInfo.error)
         return trq::fail(hostInfo.error == plan::ERR_DEPTH ? TRQ_ERR_DEPTH : TRQ_ERR_LAYOUT, "bvhList: node %u: %s (%u, %u)", hostInfo.errorNode,
                          plan_error_text(hostInfo.error), hostInfo.errorA, hostInfo.errorB);
-    trq_scene_info_t info{};
+    trq_scene_info_t& info = t.info;
     info.nNode = n; info.nInterior = hostInfo.nInterior; info.nLeaf = hostInfo.nLeaf; info.maxDepth = hostInfo.maxDepth;
-    info.nTri = hostInfo.nTri; info.nSphere = hostInfo.nSphere; info.nSquare = d->nSquare; info.nCube = d->nCube;
+    info.nTri = hostInfo.nTri; info.nSphere = hostInfo.nSphere; info.nSquare = r.nSquare; info.nCube = r.nCube;
     info.topNodes = hostInfo.nTop;
-    s->maxPIndex = hostInfo.maxPIndex;
-    return finish_scene(s, d, info, hostInfo.nSquare, hostInfo.rootRef, hostInfo.rootMin, hostInfo.rootMax);
+    t.nSqLeaf = hostInfo.nSquare; t.maxPIndex = hostInfo.maxPIndex; t.rootRef = hostInfo.rootRef;
+    for (int k = 0; k < 3; ++k) { t.rootMin[k] = hostInfo.rootMin[k]; t.rootMax[k] = hostInfo.rootMax[k]; }
+    return TRQ_OK;
 }
 
 // The refit of trq_scene_update_vertices and trq_scene_update_primitives (header: what changes and what is kept). `c` is
@@ -754,31 +763,32 @@ int refit_scene(trq_scene* s, const trq_scene_desc* c, uint32_t flags, const cha
     DeviceGuard guard(s->device);
     if (!guard.ok) return trq::fail(TRQ_ERR_CUDA, "cudaSetDevice(%d) failed", s->device);
     TRQ_CUDA(cudaDeviceSynchronize());                           // traces in flight still read the old boxes and records
-    const uint32_t n = s->nNode;
+    PackedTree& t = s->tree;
+    const SceneRecords& r = s->rec;
+    const uint32_t n = t.info.nNode;
     trq::PoolScratch mem(s->device, nullptr);
     uint32_t* arrivals;
     if (!mem.alloc(&arrivals, n)) return trq::fail(TRQ_ERR_NOMEM, "%s: out of device memory", who);
     const cudaMemcpyKind kind = (flags & TRQ_HOST_PTRS) ? cudaMemcpyHostToDevice : cudaMemcpyDeviceToDevice;
     const bool sph = c->sphereList && c->nSphere, sq = c->squareList && c->nSquare, cube = c->cubeList && c->nCube, tri = c->triList && c->nVert;
-    if (sph) TRQ_CUDA(cudaMemcpy(s->d_spheres, c->sphereList, (size_t)c->nSphere * sizeof(RefSphere), kind));
-    if (sq) TRQ_CUDA(cudaMemcpy(s->d_squares, c->squareList, (size_t)c->nSquare * sizeof(RefSquare), kind));
-    if (cube) TRQ_CUDA(cudaMemcpy(s->d_cubes, c->cubeList, (size_t)c->nCube * sizeof(RefCube), kind));
-    if (tri) TRQ_CUDA(cudaMemcpy(s->d_verts, c->triList, (size_t)c->nVert * sizeof(RefVertex), kind));
+    if (sph) TRQ_CUDA(cudaMemcpy(r.spheres, c->sphereList, (size_t)c->nSphere * sizeof(RefSphere), kind));
+    if (sq) TRQ_CUDA(cudaMemcpy(r.squares, c->squareList, (size_t)c->nSquare * sizeof(RefSquare), kind));
+    if (cube) TRQ_CUDA(cudaMemcpy(r.cubes, c->cubeList, (size_t)c->nCube * sizeof(RefCube), kind));
+    if (tri) TRQ_CUDA(cudaMemcpy(r.verts, c->triList, (size_t)c->nVert * sizeof(RefVertex), kind));
     TRQ_CUDA(cudaMemsetAsync(arrivals, 0, (size_t)n * 4));
     const unsigned grid = (n + 255) / 256;
-    if (tri) { plan::refit_leaves_kernel<<<grid, 256>>>(s->d_bvh, s->d_ref, n, s->d_verts, s->d_idx); g_launches++; }
+    if (tri) { plan::refit_leaves_kernel<<<grid, 256>>>(t.bvh, t.ref, n, r.verts, r.idx); g_launches++; }
     if (sph || sq || cube) {
-        const int rc = trq::refit_primitive_leaves_on_device(s->d_bvh, s->d_ref, n, sph ? s->d_spheres : nullptr, sq ? s->d_squares : nullptr,
-                                                             cube ? s->d_cubes : nullptr);
+        const int rc = trq::refit_primitive_leaves_on_device(t.bvh, t.ref, n, sph ? r.spheres : nullptr, sq ? r.squares : nullptr,
+                                                             cube ? r.cubes : nullptr);
         if (rc != TRQ_OK) return rc;
     }
-    plan::refit_interior_kernel<<<grid, 256>>>(s->d_bvh, s->d_ref, n, arrivals);
-    pack_scene_kernel<<<grid, 256>>>(s->d_bvh, s->d_ref, n, s->d_verts, s->d_idx, s->d_spheres, s->d_squares,
-                                     s->d_nodes, s->d_tris, s->d_sph, s->d_sq, s->d_triN, s->d_topSoA, s->topStride);
-    g_launches += 2;
+    plan::refit_interior_kernel<<<grid, 256>>>(t.bvh, t.ref, n, arrivals);
+    g_launches++;
+    launch_pack(t, r);
     RefAABB root;
-    TRQ_CUDA(cudaMemcpy(&root, &s->d_bvh[0].bBOX, sizeof root, cudaMemcpyDeviceToHost));
-    for (int k = 0; k < 3; ++k) { s->dev.rootMin[k] = root.mini[k]; s->dev.rootMax[k] = root.maxi[k]; }
+    TRQ_CUDA(cudaMemcpy(&root, &t.bvh[0].bBOX, sizeof root, cudaMemcpyDeviceToHost));
+    for (int k = 0; k < 3; ++k) { t.rootMin[k] = root.mini[k]; t.rootMax[k] = root.maxi[k]; }
     TRQ_CUDA(cudaGetLastError());
     return TRQ_OK;
 }
@@ -791,31 +801,24 @@ int trq_scene_create(const trq_scene_desc* d, int device, trq_scene** out) {
     int rc = check_desc(d, out, "trq_scene_create");
     if (rc != TRQ_OK) return rc;
 
-    trq_scene_info_t info{};
+    PackedTree tree;
     std::vector<uint32_t> ref;
-    uint32_t maxPIndex = 0;
-    rc = plan_layout(d, ref, info, maxPIndex);                 // pure host validation: runs without a GPU
+    rc = plan_layout(d, ref, tree);                            // pure host validation: runs without a GPU
     if (rc != TRQ_OK) return rc;
 
     trq_scene* s = nullptr;
     if ((rc = open_scene(device, &s, "trq_scene_create")) != TRQ_OK) return rc;
+    s->tree = tree;
     DeviceGuard guard(device);
     auto bail = [&](int code) { free_scene(s); return code; };
     if (!guard.ok) return bail(trq::fail(TRQ_ERR_CUDA, "cudaSetDevice(%d) failed", device));
-    s->maxPIndex = maxPIndex;
-
-    if ((rc = upload(&s->d_spheres, d->sphereList, d->nSphere)) != TRQ_OK) return bail(rc);
-    if ((rc = upload(&s->d_squares, d->squareList, d->nSquare)) != TRQ_OK) return bail(rc);
-    if ((rc = upload(&s->d_cubes, d->cubeList, d->nCube)) != TRQ_OK) return bail(rc);
-    if ((rc = upload(&s->d_verts, d->triList, d->nVert)) != TRQ_OK) return bail(rc);
-    if ((rc = upload(&s->d_idx, d->idxList, (size_t)d->nTri * 3)) != TRQ_OK) return bail(rc);
-    if ((rc = upload(&s->d_bvh, d->bvhList, d->nNode)) != TRQ_OK) return bail(rc);
-    if ((rc = upload(&s->d_ref, ref.data(), ref.size())) != TRQ_OK) return bail(rc);
-
-    uint32_t nSqLeaf = 0;
-    for (uint32_t r : ref) if (r != TRQ_REF_DONE_WORD && TRQ_REF_KIND(r) == REF_SQUARE) ++nSqLeaf;
-    const RefBVH* N = (const RefBVH*)d->bvhList;
-    if ((rc = finish_scene(s, d, info, nSqLeaf, ref[0], N[0].bBOX.mini, N[0].bBOX.maxi)) != TRQ_OK) return bail(rc);
+    const cudaMemcpyKind k = cudaMemcpyHostToDevice;
+    if ((rc = open_queues(s)) != TRQ_OK) return bail(rc);
+    if ((rc = upload_records(s->rec, d, k)) != TRQ_OK) return bail(rc);
+    if ((rc = upload(&s->tree.bvh, d->bvhList, d->nNode, k)) != TRQ_OK) return bail(rc);
+    if ((rc = upload(&s->tree.ref, ref.data(), ref.size(), k)) != TRQ_OK) return bail(rc);
+    if ((rc = pack_tree(s->tree, s->rec, device)) != TRQ_OK) return bail(rc);
+    s->defaultCfg = s->tree.autoCfg;
     *out = s;
     return TRQ_OK;
 }
@@ -834,14 +837,13 @@ int trq_scene_create_device(const trq_scene_desc* d, int device, trq_scene** out
     StageTimer tm;
     TRQ_LAP(tm, "open scene");
     const cudaMemcpyKind k = cudaMemcpyDeviceToDevice;
-    if ((rc = upload_from(&s->d_spheres, d->sphereList, d->nSphere, k)) != TRQ_OK) return bail(rc);
-    if ((rc = upload_from(&s->d_squares, d->squareList, d->nSquare, k)) != TRQ_OK) return bail(rc);
-    if ((rc = upload_from(&s->d_cubes, d->cubeList, d->nCube, k)) != TRQ_OK) return bail(rc);
-    if ((rc = upload_from(&s->d_verts, d->triList, d->nVert, k)) != TRQ_OK) return bail(rc);
-    if ((rc = upload_from(&s->d_idx, d->idxList, (size_t)d->nTri * 3, k)) != TRQ_OK) return bail(rc);
-    if ((rc = upload_from(&s->d_bvh, d->bvhList, d->nNode, k)) != TRQ_OK) return bail(rc);
+    if ((rc = open_queues(s)) != TRQ_OK) return bail(rc);
+    if ((rc = upload_records(s->rec, d, k)) != TRQ_OK) return bail(rc);
+    if ((rc = upload(&s->tree.bvh, d->bvhList, d->nNode, k)) != TRQ_OK) return bail(rc);
     TRQ_LAP(tm, "copy six arrays D2D");
-    if ((rc = plan_and_finish(s, d, "trq_scene_create_device")) != TRQ_OK) return bail(rc);
+    if ((rc = plan_tree(s->tree, d->nNode, s->rec, device, "trq_scene_create_device")) != TRQ_OK) return bail(rc);
+    if ((rc = pack_tree(s->tree, s->rec, device)) != TRQ_OK) return bail(rc);
+    s->defaultCfg = s->tree.autoCfg;
     *out = s;
     return TRQ_OK;
 }
@@ -849,7 +851,7 @@ int trq_scene_create_device(const trq_scene_desc* d, int device, trq_scene** out
 // Refit after the vertices moved (animated meshes): the refit with only triList replaced.
 int trq_scene_update_vertices(trq_scene* s, const void* triList, uint32_t nVert, uint32_t flags) {
     if (!s || !triList) return trq::fail(TRQ_ERR_INVALID, "trq_scene_update_vertices: NULL argument");
-    if (nVert != s->nVert) return trq::fail(TRQ_ERR_INVALID, "trq_scene_update_vertices: %u vertices, the scene has %u", nVert, s->nVert);
+    if (nVert != s->rec.nVert) return trq::fail(TRQ_ERR_INVALID, "trq_scene_update_vertices: %u vertices, the scene has %u", nVert, s->rec.nVert);
     if (nVert == 0) return TRQ_OK;                              // (a one-leaf scene is refit too: its leaf is the root)
     trq_scene_desc c{};
     c.triList = triList; c.nVert = nVert;
@@ -865,74 +867,58 @@ int trq_scene_update_primitives(trq_scene* s, const trq_scene_desc* c, uint32_t 
     if ((c->nSphere && !c->sphereList) || (c->nSquare && !c->squareList) || (c->nCube && !c->cubeList) || (c->nVert && !c->triList))
         return trq::fail(TRQ_ERR_INVALID, "%s: NULL array with non-zero count", who);
     const struct { const void* list; uint32_t n, have; const char* what; } kinds[] = {
-        {c->sphereList, c->nSphere, s->listSphere, "spheres"}, {c->squareList, c->nSquare, s->listSquare, "squares"},
-        {c->cubeList, c->nCube, s->listCube, "cubes"}, {c->triList, c->nVert, s->nVert, "vertices"}};
+        {c->sphereList, c->nSphere, s->rec.nSphere, "spheres"}, {c->squareList, c->nSquare, s->rec.nSquare, "squares"},
+        {c->cubeList, c->nCube, s->rec.nCube, "cubes"}, {c->triList, c->nVert, s->rec.nVert, "vertices"}};
     for (const auto& k : kinds)
         if (k.list && k.n != k.have) return trq::fail(TRQ_ERR_INVALID, "%s: %u %s, the scene has %u", who, k.n, k.what, k.have);
     return refit_scene(s, c, flags, who);
 }
 
-// New topology from the current geometry (header: the leaf list, the records and what a rebuild keeps). Everything new is
-// staged in a second trq_scene that borrows the arrays a rebuild keeps (spheres, squares, cubes, indices, queue heads) and
-// goes through the same planning and packing as trq_scene_create_device; the scene itself changes only once that has
-// succeeded, so a failure leaves it as it was.
+// New topology from the current geometry (header: the leaf list, the records and what a rebuild keeps). A new tree is built
+// over the scene's records (with the new vertices, when given), planned and packed like trq_scene_create_device's; only then
+// is it swapped into the scene and the old tree released, so a failure leaves the scene as it was.
 int trq_scene_rebuild(trq_scene* s, const void* triList, uint32_t nVert, uint32_t flags) {
     if (!s) return trq::fail(TRQ_ERR_INVALID, "trq_scene_rebuild: NULL scene");
-    if (triList ? nVert != s->nVert : (nVert != 0 && nVert != s->nVert))
-        return trq::fail(TRQ_ERR_INVALID, "trq_scene_rebuild: %u vertices, the scene has %u", nVert, s->nVert);
+    if (triList ? nVert != s->rec.nVert : (nVert != 0 && nVert != s->rec.nVert))
+        return trq::fail(TRQ_ERR_INVALID, "trq_scene_rebuild: %u vertices, the scene has %u", nVert, s->rec.nVert);
     DeviceGuard guard(s->device);
     if (!guard.ok) return trq::fail(TRQ_ERR_CUDA, "cudaSetDevice(%d) failed", s->device);
     TRQ_CUDA(cudaDeviceSynchronize());                           // traces in flight still read the old arrays
-    trq_scene* t = new (std::nothrow) trq_scene();
-    if (!t) return trq::fail(TRQ_ERR_NOMEM, "trq_scene_rebuild: out of host memory");
-    t->device = s->device; t->numSMs = s->numSMs;
-    t->d_spheres = s->d_spheres; t->d_squares = s->d_squares; t->d_cubes = s->d_cubes; t->d_idx = s->d_idx; t->d_queues = s->d_queues;
-    t->d_verts = s->d_verts;
-    const bool newVerts = triList && nVert;
-    // the arrays a rebuild replaces: the staged ones on failure, the scene's old ones after the commit
-    auto drop = [&] {
-        pool_free(t->d_bvh); pool_free(t->d_ref); pool_free(t->d_nodes); pool_free(t->d_tris); pool_free(t->d_sph); pool_free(t->d_sq);
-        pool_free(t->d_triN); pool_free(t->d_topSoA);
-        if (newVerts) pool_free(t->d_verts);
-        delete t;
-    };
-    auto bail = [&](int code) { drop(); return code; };
+    PackedTree t;
+    RefVertex* newVerts = nullptr;                               // owned here until the commit
+    auto bail = [&](int code) { t.release(); pool_free(newVerts); return code; };
     int rc = TRQ_OK;
-    if (newVerts && (rc = upload_from(&t->d_verts, triList, nVert, (flags & TRQ_HOST_PTRS) ? cudaMemcpyHostToDevice : cudaMemcpyDeviceToDevice)) != TRQ_OK)
+    if (triList && nVert && (rc = upload(&newVerts, triList, nVert, (flags & TRQ_HOST_PTRS) ? cudaMemcpyHostToDevice : cudaMemcpyDeviceToDevice)) != TRQ_OK)
         return bail(rc);
-    const uint32_t n = s->info.nLeaf, nNode = 2 * n - 1;
+    SceneRecords r = s->rec;                                     // the records the new tree is built over (not owned)
+    if (newVerts) r.verts = newVerts;
+    const uint32_t n = s->tree.info.nLeaf, nNode = 2 * n - 1;
     {
         trq::PoolScratch mem(s->device, nullptr);
         RefBVH* leaves = nullptr;
-        if ((rc = trq::reachable_leaves_on_device(s->d_bvh, s->d_ref, s->nNode, n, t->d_verts, s->d_idx, mem, &leaves)) != TRQ_OK) return bail(rc);
-        if (pool_malloc((void**)&t->d_bvh, (size_t)nNode * sizeof(RefBVH)) != cudaSuccess)
+        if ((rc = trq::reachable_leaves_on_device(s->tree.bvh, s->tree.ref, s->tree.info.nNode, n, r.verts, r.idx, mem, &leaves)) != TRQ_OK) return bail(rc);
+        if (pool_malloc((void**)&t.bvh, (size_t)nNode * sizeof(RefBVH)) != cudaSuccess)
             return bail(trq::fail(TRQ_ERR_NOMEM, "trq_scene_rebuild: out of device memory"));
         if (n == 1) {                                            // the lone leaf is the root (BVH.hh:52-54), parent 0
-            cudaError_t e = cudaMemcpyAsync(t->d_bvh, leaves, sizeof(RefBVH), cudaMemcpyDeviceToDevice, nullptr);
+            cudaError_t e = cudaMemcpyAsync(t.bvh, leaves, sizeof(RefBVH), cudaMemcpyDeviceToDevice, nullptr);
             if (e != cudaSuccess) return bail(trq::fail(TRQ_ERR_CUDA, "trq_scene_rebuild: %s", cudaGetErrorString(e)));
         } else {
             uint32_t depth = 0;
-            rc = trq::build_on_device(leaves, n, t->d_bvh, s->device, &depth);
+            rc = trq::build_on_device(leaves, n, t.bvh, s->device, &depth);
             if (rc == TRQ_ERR_DEPTH)
                 return bail(trq::fail(TRQ_ERR_DEPTH, "trq_scene_rebuild: the new tree has interior depth %u, above the 32-bit trail's 31 "
                                                      "(Render.hh:140); the scene is unchanged", depth));
             if (rc != TRQ_OK) return bail(rc);
         }
     }
-    trq_scene_desc d{};                                          // counts of the arrays the scene holds (no pointer is read)
-    d.nSphere = s->listSphere; d.nSquare = s->listSquare; d.nCube = s->listCube; d.nVert = s->nVert; d.nTri = s->listTri; d.nNode = nNode;
-    if ((rc = plan_and_finish(t, &d, "trq_scene_rebuild")) != TRQ_OK) return bail(rc);
+    if ((rc = plan_tree(t, nNode, r, s->device, "trq_scene_rebuild")) != TRQ_OK) return bail(rc);
+    if ((rc = pack_tree(t, r, s->device)) != TRQ_OK) return bail(rc);
 
-    // commit: swap the replaced arrays, take over the derived state
-    std::swap(s->d_verts, t->d_verts); std::swap(s->d_bvh, t->d_bvh); std::swap(s->d_ref, t->d_ref);
-    std::swap(s->d_nodes, t->d_nodes); std::swap(s->d_tris, t->d_tris); std::swap(s->d_sph, t->d_sph); std::swap(s->d_sq, t->d_sq);
-    std::swap(s->d_triN, t->d_triN); std::swap(s->d_topSoA, t->d_topSoA);
-    s->info = t->info; s->dev = t->dev; s->nNode = t->nNode; s->topStride = t->topStride; s->stackDepth = t->stackDepth;
-    s->largeTree = t->largeTree; s->leaves = t->leaves; s->maxPIndex = t->maxPIndex;
-    for (int c = 0; c < kNumCfgs; ++c) s->cfg[c] = t->cfg[c];
-    s->autoCfg = t->autoCfg;
-    if (!(s->userCfg && s->cfg[s->defaultCfg].usable)) { s->defaultCfg = s->autoCfg; s->userCfg = false; }
-    drop();
+    // commit: the new tree (and vertices) in, the old ones out
+    std::swap(s->tree, t);
+    t.release();
+    if (newVerts) { pool_free(s->rec.verts); s->rec.verts = newVerts; }
+    if (!(s->userCfg && s->tree.cfg[s->defaultCfg].usable)) { s->defaultCfg = s->tree.autoCfg; s->userCfg = false; }
     return TRQ_OK;
 }
 
@@ -940,7 +926,7 @@ int trq_scene_copy_bvh(const trq_scene* s, void* out, uint32_t flags) {
     if (!s || !out) return trq::fail(TRQ_ERR_INVALID, "trq_scene_copy_bvh: NULL argument");
     DeviceGuard guard(s->device);
     if (!guard.ok) return trq::fail(TRQ_ERR_CUDA, "cudaSetDevice(%d) failed", s->device);
-    TRQ_CUDA(cudaMemcpy(out, s->d_bvh, (size_t)s->nNode * sizeof(RefBVH), (flags & TRQ_HOST_PTRS) ? cudaMemcpyDeviceToHost : cudaMemcpyDeviceToDevice));
+    TRQ_CUDA(cudaMemcpy(out, s->tree.bvh, (size_t)s->tree.info.nNode * sizeof(RefBVH), (flags & TRQ_HOST_PTRS) ? cudaMemcpyDeviceToHost : cudaMemcpyDeviceToDevice));
     return TRQ_OK;
 }
 
@@ -967,12 +953,12 @@ const char* trq_kernel_config_name(int cfg) { return (cfg >= 0 && cfg < kNumCfgs
 int trq_scene_set_kernel_config(trq_scene* s, int cfg, uint32_t* topNodesStaged) {
     if (!s) return trq::fail(TRQ_ERR_INVALID, "trq_scene_set_kernel_config: NULL scene");
     const bool user = cfg >= 0;
-    if (cfg < 0) cfg = s->autoCfg;
+    if (cfg < 0) cfg = s->tree.autoCfg;
     if (cfg >= kNumCfgs) return trq::fail(TRQ_ERR_INVALID, "trq_scene_set_kernel_config: %d configurations", kNumCfgs);
-    if (!s->cfg[cfg].usable) return trq::fail(TRQ_ERR_INVALID, "trq_scene_set_kernel_config: configuration %s does not fit this scene (stack depth %u)", kCfgs[cfg].name, s->stackDepth);
+    if (!s->tree.cfg[cfg].usable) return trq::fail(TRQ_ERR_INVALID, "trq_scene_set_kernel_config: configuration %s does not fit this scene (stack depth %u)", kCfgs[cfg].name, s->tree.stackDepth);
     s->defaultCfg = cfg;
     s->userCfg = user;
-    if (topNodesStaged) *topNodesStaged = kCfgs[cfg].top ? s->cfg[cfg].topCount : 0;
+    if (topNodesStaged) *topNodesStaged = kCfgs[cfg].top ? s->tree.cfg[cfg].topCount : 0;
     return TRQ_OK;
 }
 
@@ -980,7 +966,7 @@ int trq_scene_kernel_config(const trq_scene* s) { return s ? pick_cfg(s) : -1; }
 
 int trq_scene_info(const trq_scene* s, trq_scene_info_t* info) {
     if (!s || !info) return trq::fail(TRQ_ERR_INVALID, "trq_scene_info: NULL argument");
-    *info = s->info;
+    *info = s->tree.info;
     return TRQ_OK;
 }
 
@@ -1018,8 +1004,8 @@ int trq_trace(trq_scene* s, const trq_ray* rays, uint64_t n, uint32_t flags, voi
     if (!s) return trq::fail(TRQ_ERR_INVALID, "trq_trace: NULL scene");
     if (n == 0) return TRQ_OK;
     if (!rays || !hits) return trq::fail(TRQ_ERR_INVALID, "trq_trace: NULL rays/hits");
-    if ((flags & TRQ_HIT16) && s->maxPIndex >= (1u << 28))
-        return trq::fail(TRQ_ERR_INVALID, "trq_trace: TRQ_HIT16 packs pIndex into 28 bits; this scene has pIndex up to %u", s->maxPIndex);
+    if ((flags & TRQ_HIT16) && s->tree.maxPIndex >= (1u << 28))
+        return trq::fail(TRQ_ERR_INVALID, "trq_trace: TRQ_HIT16 packs pIndex into 28 bits; this scene has pIndex up to %u", s->tree.maxPIndex);
     if (!(flags & TRQ_HOST_PTRS) && ((((uintptr_t)rays) & 31u) || (((uintptr_t)hits) & ((flags & TRQ_HIT16) ? 15u : 31u))))
         return trq::fail(TRQ_ERR_INVALID, "trq_trace: device rays / hits must be aligned to their record size (32 / 32 or 16 bytes: one access per record)");
     DeviceGuard guard(s->device);
@@ -1051,13 +1037,13 @@ int trq_expand_hits(trq_scene* s, const trq_ray* rays, const trq_hit* hits, uint
         if (cudaMalloc((void**)&dq, n * sizeof(trq_hit_record)) != cudaSuccess) { cudaFree(dr); cudaFree(dh); return trq::fail(TRQ_ERR_CUDA, "cudaMalloc failed"); }
         cudaError_t e = cudaMemcpy(dr, rays, n * sizeof(trq_ray), cudaMemcpyHostToDevice);
         if (e == cudaSuccess) e = cudaMemcpy(dh, hits, n * sizeof(trq_hit), cudaMemcpyHostToDevice);
-        if (e == cudaSuccess) { expand_hits_kernel<<<(unsigned)grid, block>>>(s->dev, dr, dh, dq, n); g_launches++; e = cudaGetLastError(); }
+        if (e == cudaSuccess) { expand_hits_kernel<<<(unsigned)grid, block>>>(scene_dev(s), dr, dh, dq, n); g_launches++; e = cudaGetLastError(); }
         if (e == cudaSuccess) e = cudaMemcpy(records, dq, n * sizeof(trq_hit_record), cudaMemcpyDeviceToHost);
         cudaFree(dr); cudaFree(dh); cudaFree(dq);
         if (e != cudaSuccess) return trq::fail(TRQ_ERR_CUDA, "trq_expand_hits: %s", cudaGetErrorString(e));
         return TRQ_OK;
     }
-    expand_hits_kernel<<<(unsigned)grid, block, 0, (cudaStream_t)stream>>>(s->dev, rays, hits, records, n);
+    expand_hits_kernel<<<(unsigned)grid, block, 0, (cudaStream_t)stream>>>(scene_dev(s), rays, hits, records, n);
     g_launches++;
     TRQ_CUDA(cudaGetLastError());
     return TRQ_OK;
@@ -1133,7 +1119,7 @@ int trq_spawn_bounce_rng(trq_scene* s, const trq_ray* rays, const trq_hit* hits,
     cudaStream_t st = (cudaStream_t)stream;
     TRQ_CUDA(cudaMemsetAsync(d_count, 0, sizeof(uint64_t), st));
     if (n == 0) return TRQ_OK;
-    spawn_bounce_kernel<<<(unsigned)((n + 255) / 256), 256, 0, st>>>(s->dev, rays, hits, n, (const unsigned long long*)d_n, seedBase, pixelOf, rngState, out, srcIndex,
+    spawn_bounce_kernel<<<(unsigned)((n + 255) / 256), 256, 0, st>>>(scene_dev(s), rays, hits, n, (const unsigned long long*)d_n, seedBase, pixelOf, rngState, out, srcIndex,
                                                                       (unsigned long long*)d_count);
 
     g_launches++;
@@ -1165,14 +1151,14 @@ int trq_spawn_shadow_rng(trq_scene* s, const trq_ray* rays, const trq_hit* hits,
     if (rc == TRQ_OK && rngState && (((uintptr_t)rngState) & 15u)) rc = trq::fail(TRQ_ERR_INVALID, "trq_spawn_shadow_rng: rngState must be 16-byte aligned");
     if (rc != TRQ_OK) return rc;
     if (n && !out) return trq::fail(TRQ_ERR_INVALID, "trq_spawn_shadow: NULL out");
-    if (lightA >= s->info.nSquare || lightB >= s->info.nSquare)
-        return trq::fail(TRQ_ERR_INVALID, "trq_spawn_shadow: light index out of range (nSquare %u)", s->info.nSquare);
+    if (lightA >= s->tree.info.nSquare || lightB >= s->tree.info.nSquare)
+        return trq::fail(TRQ_ERR_INVALID, "trq_spawn_shadow: light index out of range (nSquare %u)", s->tree.info.nSquare);
     DeviceGuard guard(s->device);
     if (!guard.ok) return trq::fail(TRQ_ERR_CUDA, "cudaSetDevice(%d) failed", s->device);
     cudaStream_t st = (cudaStream_t)stream;
     TRQ_CUDA(cudaMemsetAsync(d_count, 0, sizeof(uint64_t), st));
     if (n == 0) return TRQ_OK;
-    spawn_shadow_kernel<<<(unsigned)((n + 255) / 256), 256, 0, st>>>(s->dev, rays, hits, n, (const unsigned long long*)d_n, seedBase, pixelOf, rngState, lightA, lightB, out, srcIndex,
+    spawn_shadow_kernel<<<(unsigned)((n + 255) / 256), 256, 0, st>>>(scene_dev(s), rays, hits, n, (const unsigned long long*)d_n, seedBase, pixelOf, rngState, lightA, lightB, out, srcIndex,
                                                                       (unsigned long long*)d_count);
     g_launches++;
     TRQ_CUDA(cudaGetLastError());
@@ -1286,7 +1272,7 @@ int trq_trace_gather(trq_scene* s, trq_gather* g, const trq_ray* rays, uint64_t 
     if (n > g->capacity) return trq::fail(TRQ_ERR_INVALID, "trq_trace_gather: %llu rays exceed the capacity %llu", (unsigned long long)n, (unsigned long long)g->capacity);
     if (n && !rays) return trq::fail(TRQ_ERR_INVALID, "trq_trace_gather: NULL rays");
     if (((uintptr_t)rays) & 31u) return trq::fail(TRQ_ERR_INVALID, "trq_trace_gather: rays must be 32-byte aligned");
-    if ((flags & TRQ_HIT16) && s->maxPIndex >= (1u << 28)) return trq::fail(TRQ_ERR_INVALID, "trq_trace_gather: TRQ_HIT16 packs pIndex into 28 bits");
+    if ((flags & TRQ_HIT16) && s->tree.maxPIndex >= (1u << 28)) return trq::fail(TRQ_ERR_INVALID, "trq_trace_gather: TRQ_HIT16 packs pIndex into 28 bits");
     DeviceGuard guard(s->device);
     if (!guard.ok) return trq::fail(TRQ_ERR_CUDA, "cudaSetDevice(%d) failed", s->device);
     const unsigned long long step = ++g->step;
@@ -1331,12 +1317,12 @@ int trq_trace_gather(trq_scene* s, trq_gather* g, const trq_ray* rays, uint64_t 
     // driver sizes the SM's shared-memory carve-out to what the trace needs, rounded up to a supported size; when that leaves
     // less than the reserve (C3's depth: 5 x 39 KB = 195 of 196 KB), ask for the next size for this launch.
     const bool any = (flags & TRQ_TRACE_ANY) != 0, hit16 = (flags & TRQ_HIT16) != 0;
-    const void* fn = kCfgs[0].fn[s->leaves][any ? 1 : 0][hit16 ? 1 : 0];
+    const void* fn = kCfgs[0].fn[s->tree.leaves][any ? 1 : 0][hit16 ? 1 : 0];
     bool bumped = false, useTma = false;
     size_t chosen = 228 * 1024;
     if (n) {
         static const size_t kCarveKB[] = {0, 8, 16, 32, 64, 100, 132, 164, 196, 228};
-        const size_t need = (size_t)s->cfg[0].blocksPerSM[any ? 1 : 0][hit16 ? 1 : 0] * (s->cfg[0].smem + kSmemBlockReserve);
+        const size_t need = (size_t)s->tree.cfg[0].blocksPerSM[any ? 1 : 0][hit16 ? 1 : 0] * (s->tree.cfg[0].smem + kSmemBlockReserve);
         for (size_t kb : kCarveKB) if (kb * 1024 >= need) { chosen = kb * 1024; break; }
         static const int tmaEnv = [] { const char* e = getenv("TRQ_GATHER_TMA"); return e ? atoi(e) : 1; }();
         // the TMA sender stages through 24 KB of shared memory; beside a trace that leaves less than that even at the largest
