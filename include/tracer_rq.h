@@ -152,6 +152,9 @@ typedef struct trq_scene_info_t {
                                        buffers must stay valid (and should be pinned) until trq_host_sync() returns.
                                        Consecutive calls then overlap: the next batch's H2D runs under this one's D2H. */
 
+/* trq_scene_rebuild flags (with TRQ_HOST_PTRS) */
+#define TRQ_BUILD_MORTON     0x80u  /* build the new topology with the Morton builder (trq_bvh_build_tree_morton_device) */
+
 typedef struct trq_scene trq_scene;
 
 int  trq_version(void);
@@ -218,6 +221,8 @@ int  trq_scene_update_primitives(trq_scene* scene, const trq_scene_desc* changes
  *              (maxDepth, topNodes, nNode, bytesReferenceLayout, ...), packed arrays, top-of-tree block, and every launch
  *              configuration's usability and staged node count. A configuration chosen with trq_scene_set_kernel_config
  *              is kept if it is still usable; otherwise the scene uses the automatic choice for the new tree.
+ *   builder    with TRQ_BUILD_MORTON in flags, the tree over the same leaf list is trq_bvh_build_tree_morton_device's
+ *              instead: much faster to build, usually slower to trace, never deeper than 31. Everything else is as above.
  *   failure    TRQ_ERR_DEPTH (new interior depth > 31; the message gives it), TRQ_ERR_NOMEM, TRQ_ERR_INVALID (nVert other
  *              than the scene's): the scene is exactly as before, vertices included.
  * Synchronous: waits for work in flight on the device, returns when the scene is ready for the next trq_trace. Hits traced
@@ -422,6 +427,33 @@ int  trq_bvh_build_tree_gpu(void* bvhList, uint32_t nLeaves, int device, uint32_
  * nodes; the result replaces them): build -> trq_scene_create_device without the tree ever visiting the host.
  * Interior depth above 31 returns TRQ_ERR_DEPTH with the complete tree in d_bvhList and its true depth. */
 int  trq_bvh_build_tree_device(void* d_bvhList, uint32_t nLeaves, int device, uint32_t* nNodeOut, uint32_t* maxDepthOut);
+
+/* The Morton-order (LBVH) builder: a tree in the same node format and layout (root at 0, leaves at 1..nLeaves in list
+ * order, interiors after, parent/left/right final indices), built in a fraction of the SAH builder's time at some cost in
+ * trace speed. It never returns TRQ_ERR_DEPTH: every tree it builds has interior depth <= 31. Its tree, for n leaves:
+ *   centroid   AABB::centroid (AABB.hh:22-25) of each leaf box: mini + (maxi - mini) / 2.
+ *   quantise   per axis, strict fp32: lo / hi = min / max of the FINITE centroid components on that axis. NaN and +inf
+ *              give 2^21 - 1, -inf gives 0. Where the axis has no finite component, or hi - lo is not (finite and > 0),
+ *              every finite component gives 0. Otherwise q = min(2^21 - 1, floor(((c - lo) / (hi - lo)) * 2^21)), each
+ *              operation rounded to nearest, in that order.
+ *   code       63 bits: bit 3i+2 is bit i of qx, bit 3i+1 of qy, bit 3i of qz.
+ *   order      leaves sorted by (code, list position).
+ *   topology   top-down; a node at interior depth d (root 0) over sorted positions [a, b], m = b - a + 1: the left child
+ *              gets floor(m / 2) leaves if code[a] == code[b], else the positions whose code has clear the highest bit in
+ *              which code[a] and code[b] differ. That size is clamped into [m - 2^(31-d), 2^(31-d)] intersected with
+ *              [1, m - 1], which bounds the depth at 31 and changes nothing where the tree is shallow enough already.
+ *   numbering  the interior node splitting between sorted positions g and g + 1 is node n + 1 + g if g is below the root's
+ *              gap, else n + g. n == 1: the lone leaf is node 0 with parent 0.
+ *   fields     axis = dimension of the highest bit in which the node's two end codes differ (0 if equal); pType TRQ_BVH,
+ *              pIndex 0, padding 0; box = union of the child boxes (fminf / fmaxf). Leaves keep every field but parent.
+ * Host restatement: bvhList as for trq_bvh_build_tree (capacity 2*nLeaves-1 nodes). TRQ_ERR_INVALID for an empty list or
+ * more than 0x3fffffff leaves. */
+int  trq_bvh_build_tree_morton(void* bvhList, uint32_t nLeaves, uint32_t* nNodeOut, uint32_t* maxDepthOut);
+
+/* The same tree, byte for byte, built on `device` with the array in DEVICE memory (as trq_bvh_build_tree_device: leaves
+ * in d_bvhList[0..nLeaves), capacity 2*nLeaves-1 nodes, the result replaces them). Synchronous, on the legacy default
+ * stream. TRQ_ERR_INVALID as the host restatement, TRQ_ERR_NO_DEVICE without a GPU. */
+int  trq_bvh_build_tree_morton_device(void* d_bvhList, uint32_t nLeaves, int device, uint32_t* nNodeOut, uint32_t* maxDepthOut);
 
 #ifdef __cplusplus
 }

@@ -13,5 +13,5 @@ mkdir -p $B
 NV="/usr/local/cuda/bin/nvcc -gencode arch=compute_100a,code=sm_100a -O3 -lineinfo -std=c++17 -Xcompiler -fPIC,-ffp-contract=off,-fno-fast-math --expt-relaxed-constexpr $*"
 make -s -C $C >/dev/null
 (cd $C && $NV -c trq_api.cu -o $B/trq_api.o && $NV -c bvh_build_gpu.cu -o $B/bvh_build_gpu.o)
-/usr/local/cuda/bin/nvcc -gencode arch=compute_100a,code=sm_100a -shared -o $OUT/libtracer_rq_$NAME.so $B/trq_api.o $B/bvh_build_gpu.o $C/build/bvh_build.o $C/build/harness.o $C/build/error.o -lpthread
+/usr/local/cuda/bin/nvcc -gencode arch=compute_100a,code=sm_100a -shared -o $OUT/libtracer_rq_$NAME.so $B/trq_api.o $B/bvh_build_gpu.o $C/build/bvh_build.o $C/build/morton_build.o $C/build/harness.o $C/build/error.o -lpthread
 echo built $OUT/libtracer_rq_$NAME.so

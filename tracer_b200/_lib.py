@@ -53,6 +53,7 @@ ABI_SYMBOLS = [
     "trq_kernel_config_count", "trq_kernel_config_name", "trq_scene_set_kernel_config", "trq_scene_kernel_config",
     "trq_trace", "trq_host_sync", "trq_expand_hits", "trq_launch_count", "trq_profile_enable", "trq_profile_read", "trq_probe_bandwidth",
     "trq_bvh_build_node", "trq_bvh_build_nodes_triangles", "trq_bvh_build_nodes_triangles_device", "trq_bvh_build_nodes_device", "trq_bvh_build_tree", "trq_bvh_build_tree_gpu", "trq_bvh_build_tree_device",
+    "trq_bvh_build_tree_morton", "trq_bvh_build_tree_morton_device",
     "trq_cast_rays", "trq_trace_indirect", "trq_spawn_bounce", "trq_spawn_shadow", "trq_spawn_bounce_rng", "trq_spawn_shadow_rng", "trq_rng_frame_begin",
     "trq_mgpu_create", "trq_mgpu_device_count", "trq_mgpu_scene", "trq_mgpu_shard", "trq_mgpu_trace", "trq_mgpu_destroy",
     "trq_gather_create", "trq_gather_connect", "trq_trace_gather", "trq_gather_wait", "trq_gather_status", "trq_gather_destroy",
@@ -117,6 +118,8 @@ lib.trq_bvh_build_nodes_device.argtypes = [_i32, _vp, _u32, _u32, _vp, C.c_int, 
 lib.trq_bvh_build_tree.argtypes = [_vp, _u32, C.POINTER(_u32), C.POINTER(_u32)]
 lib.trq_bvh_build_tree_gpu.argtypes = [_vp, _u32, C.c_int, C.POINTER(_u32), C.POINTER(_u32)]
 lib.trq_bvh_build_tree_device.argtypes = [_vp, _u32, C.c_int, C.POINTER(_u32), C.POINTER(_u32)]
+lib.trq_bvh_build_tree_morton.argtypes = [_vp, _u32, C.POINTER(_u32), C.POINTER(_u32)]
+lib.trq_bvh_build_tree_morton_device.argtypes = [_vp, _u32, C.c_int, C.POINTER(_u32), C.POINTER(_u32)]
 
 lib.trqh_pcg32_fill_f32.argtypes = [_u64, _u64, _u64, _vp]
 lib.trqh_pcg32_fill_f32.restype = None

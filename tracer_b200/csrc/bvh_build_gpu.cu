@@ -1,10 +1,12 @@
 // tracer_b200/csrc/bvh_build_gpu.cu -- BVH::buildTree (BVH.hh:246-269) on the GPU.
 //   trq_bvh_build_tree_device   leaves and result in DEVICE memory (feeds trq_scene_create_device without a host round trip)
 //   trq_bvh_build_tree_gpu      the same build for a HOST array (copy in, build, copy out)
+//   trq_bvh_build_tree_morton_device   the Morton-order builder (kernels/morton_build.cuh), DEVICE memory
 //   trq_bvh_build_nodes_triangles_device / trq_bvh_build_nodes_device   BVH::buildNode per primitive (kernels/leaves.cuh)
 // Orchestrates the level-synchronous kernels of kernels/bvh_build.cuh; same node array as trq_bvh_build_tree.
 #include <cuda_runtime.h>
 
+#include <algorithm>
 #include <cstddef>
 #include <cstdio>
 #include <cstring>
@@ -19,6 +21,9 @@
 #include "host/scratch.h"
 #include "kernels/bvh_build.cuh"
 #include "kernels/leaves.cuh"
+#include "kernels/morton_build.cuh"
+
+#include <cub/device/device_radix_sort.cuh>
 
 using namespace trq;
 using namespace trq::gpubuild;
@@ -146,6 +151,58 @@ int trq::build_on_device(const RefBVH* dLeaves, uint32_t n, RefBVH* dOut, int de
     return TRQ_OK;
 }
 
+// The Morton builder (kernels/morton_build.cuh): bounds, codes, CUB's radix sort of (code, position) -- stable, and the
+// positions enter in order, so ties stay in list order -- 32 split launches whose counts stay on the device, the shared
+// refit, and one read of the depth at the end. Never TRQ_ERR_DEPTH: the depth clamp bounds every tree at 31.
+int trq::build_morton_on_device(const RefBVH* dLeaves, uint32_t n, RefBVH* dOut, int device, uint32_t* maxDepthOut) {
+    using namespace trq::morton;
+    const uint32_t nNode = 2 * n - 1;
+    cudaStream_t st = nullptr;
+    PoolScratch mem(device, st);
+    uint64_t *codeA, *codeB;
+    uint32_t *posA, *posB, *counters, *arrivals;
+    Open *tabA, *tabB;
+    Bounds* bounds;
+    const uint32_t cap = n / 2 + 1;
+    size_t sortBytes = 0;
+    cub::DoubleBuffer<uint64_t> keys(nullptr, nullptr);
+    cub::DoubleBuffer<uint32_t> vals(nullptr, nullptr);
+    BCK(cub::DeviceRadixSort::SortPairs(nullptr, sortBytes, keys, vals, (int)n, 0, 63, st));
+    uint8_t* sortTemp;
+    bool ok = mem.alloc(&codeA, n) && mem.alloc(&codeB, n) && mem.alloc(&posA, n) && mem.alloc(&posB, n) &&
+              mem.alloc(&counters, (size_t)kCounters + nNode) && mem.alloc(&tabA, cap) && mem.alloc(&tabB, cap) &&
+              mem.alloc(&bounds, 1) && mem.alloc(&sortTemp, sortBytes);
+    if (!ok) return trq::fail(TRQ_ERR_NOMEM, "Morton BVH build on the GPU: out of device memory");
+    arrivals = counters + kCounters;
+
+    int sms = 0;
+    BCK(cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, device));
+    const unsigned grid = std::min(blocks(cap, 256), (unsigned)sms * 4u);
+    BCK(cudaMemcpyAsync(dOut + 1, dLeaves, (size_t)n * sizeof(RefBVH), cudaMemcpyDeviceToDevice, st));     // leaves at 1..n
+    BCK(cudaMemsetAsync(counters, 0, ((size_t)kCounters + nNode) * sizeof(uint32_t), st));
+    morton_init_kernel<<<1, 32, 0, st>>>(bounds, tabA, n, counters);
+    morton_bounds_kernel<<<std::min(blocks(n, 256), (unsigned)sms * 8u), 256, 0, st>>>(dLeaves, n, bounds);
+    morton_code_kernel<<<blocks(n, 256), 256, 0, st>>>(dLeaves, n, bounds, codeA, posA);
+    keys = cub::DoubleBuffer<uint64_t>(codeA, codeB);
+    vals = cub::DoubleBuffer<uint32_t>(posA, posB);
+    BCK(cub::DeviceRadixSort::SortPairs(sortTemp, sortBytes, keys, vals, (int)n, 0, 63, st));
+    Open *cur = tabA, *nxt = tabB;
+    for (uint32_t depth = 0; depth < kMaxLevels; ++depth) {
+        morton_level_kernel<<<grid, 256, 0, st>>>(keys.Current(), vals.Current(), n, cur, nxt, cap, counters, depth, dOut);
+        std::swap(cur, nxt);
+    }
+    gpubuild::refit_kernel<<<blocks(n, 256), 256, 0, st>>>(dOut, n, arrivals);
+    // 3 + 32 + 1 launches of ours; CUB's onesweep sort: a histogram, a scan and one launch per 8-bit digit
+    trq::note_launches(36 + 2 + 8);
+    uint32_t tail[2] = {0, 0};                          // deepest level, overflow flag
+    BCK(cudaMemcpyAsync(tail, counters + kMaxDepth, sizeof tail, cudaMemcpyDeviceToHost, st));
+    BCK(cudaStreamSynchronize(st));
+    BCK(cudaGetLastError());
+    if (tail[1]) return trq::fail(TRQ_ERR_LAYOUT, "Morton BVH build on the GPU: internal: level table overflow");
+    if (maxDepthOut) *maxDepthOut = tail[0];
+    return TRQ_OK;
+}
+
 // flag -> exclusive scan (the builder's scan kernels) -> scatter
 int trq::reachable_leaves_on_device(const RefBVH* bvh, const uint32_t* ref, uint32_t nNode, uint32_t nLeaf, const RefVertex* verts,
                                     const uint32_t* idx, PoolScratch& mem, RefBVH** leavesOut) {
@@ -212,6 +269,28 @@ extern "C" int trq_bvh_build_tree_device(void* d_bvhList, uint32_t nLeaves, int 
     if (!mem.alloc(&dLeaves, n)) return trq::fail(TRQ_ERR_NOMEM, "trq_bvh_build_tree_device: out of device memory");
     BCK(cudaMemcpyAsync(dLeaves, d, (size_t)n * sizeof(RefBVH), cudaMemcpyDeviceToDevice, nullptr));
     return build_on_device(dLeaves, n, d, device, maxDepthOut);
+}
+
+extern "C" int trq_bvh_build_tree_morton_device(void* d_bvhList, uint32_t nLeaves, int device, uint32_t* nNodeOut, uint32_t* maxDepthOut) {
+    if (maxDepthOut) *maxDepthOut = 0;
+    if (!d_bvhList || nLeaves == 0) return trq::fail(TRQ_ERR_INVALID, "trq_bvh_build_tree_morton_device: empty leaf list");
+    if (nLeaves > 0x3fffffffu) return trq::fail(TRQ_ERR_INVALID, "trq_bvh_build_tree_morton_device: too many leaves");
+    int rc = check_device(device, "trq_bvh_build_tree_morton_device");
+    if (rc != TRQ_OK) return rc;
+    DeviceScope scope(device);
+    if (!scope.ok) return trq::fail(TRQ_ERR_CUDA, "cudaSetDevice(%d) failed", device);
+    RefBVH* d = (RefBVH*)d_bvhList;
+    const uint32_t n = nLeaves;
+    if (nNodeOut) *nNodeOut = 2 * n - 1;
+    if (n == 1) {                                   // the lone leaf becomes node 0, as trq_bvh_build_tree_device does
+        BCK(cudaMemset(&d[0].parent, 0, sizeof(uint32_t)));
+        return TRQ_OK;
+    }
+    PoolScratch mem(device, nullptr);               // the result overwrites the leaves' slots: build from a copy
+    RefBVH* dLeaves = nullptr;
+    if (!mem.alloc(&dLeaves, n)) return trq::fail(TRQ_ERR_NOMEM, "trq_bvh_build_tree_morton_device: out of device memory");
+    BCK(cudaMemcpyAsync(dLeaves, d, (size_t)n * sizeof(RefBVH), cudaMemcpyDeviceToDevice, nullptr));
+    return build_morton_on_device(dLeaves, n, d, device, maxDepthOut);
 }
 
 extern "C" int trq_bvh_build_tree_gpu(void* bvhList, uint32_t nLeaves, int device, uint32_t* nNodeOut, uint32_t* maxDepthOut) {

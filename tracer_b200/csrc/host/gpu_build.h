@@ -12,6 +12,9 @@ namespace trq {
 // Interior depth above 31 still builds the whole tree and returns TRQ_ERR_DEPTH with its true depth.
 int build_on_device(const RefBVH* dLeaves, uint32_t n, RefBVH* dOut, int device, uint32_t* maxDepthOut);
 
+// The same output layout from the Morton builder (kernels/morton_build.cuh). n >= 2. Interior depth is at most 31.
+int build_morton_on_device(const RefBVH* dLeaves, uint32_t n, RefBVH* dOut, int device, uint32_t* maxDepthOut);
+
 // The leaf list of a rebuild: the nLeaf leaves the root reaches (ref[i] != TRQ_REF_DONE_WORD) in bvhList order, into
 // *leavesOut (allocated from `mem`). Triangle leaves are made again from `verts`; the others keep pType, pIndex and box.
 int reachable_leaves_on_device(const RefBVH* bvh, const uint32_t* ref, uint32_t nNode, uint32_t nLeaf, const RefVertex* verts,

@@ -904,7 +904,8 @@ int trq_scene_rebuild(trq_scene* s, const void* triList, uint32_t nVert, uint32_
             if (e != cudaSuccess) return bail(trq::fail(TRQ_ERR_CUDA, "trq_scene_rebuild: %s", cudaGetErrorString(e)));
         } else {
             uint32_t depth = 0;
-            rc = trq::build_on_device(leaves, n, t.bvh, s->device, &depth);
+            rc = (flags & TRQ_BUILD_MORTON) ? trq::build_morton_on_device(leaves, n, t.bvh, s->device, &depth)
+                                            : trq::build_on_device(leaves, n, t.bvh, s->device, &depth);
             if (rc == TRQ_ERR_DEPTH)
                 return bail(trq::fail(TRQ_ERR_DEPTH, "trq_scene_rebuild: the new tree has interior depth %u, above the 32-bit trail's 31 "
                                                      "(Render.hh:140); the scene is unchanged", depth));

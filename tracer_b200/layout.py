@@ -69,6 +69,7 @@ assert ray_dtype.itemsize == 32 and hit_dtype.itemsize == 32 and hit16_dtype.ite
 
 HIT_FLAG_HIT, HIT_FLAG_FRONT = 1, 2
 TRACE_ANY, HOST_PTRS, KERNEL_REFLAYOUT, SORT_RAYS, HOST_ASYNC, HIT16, NO_SORT = 0x1, 0x2, 0x4, 0x8, 0x10, 0x20, 0x40
+BUILD_MORTON = 0x80                    # trq_scene_rebuild: the Morton builder builds the new topology
 
 FLT_MAX = float(np.finfo(np.float32).max)
 FLT_MIN = float(np.finfo(np.float32).tiny)

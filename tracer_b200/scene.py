@@ -24,6 +24,13 @@ def _ptr(a):
     return None if a is None or a.size == 0 else a.ctypes.data
 
 
+def _morton(method):
+    """True for method="morton" (the Morton-order builder), False for "sah" (the reference's binned-SAH builder)."""
+    if method not in ("sah", "morton"):
+        raise ValueError(f'method must be "sah" or "morton", not {method!r}')
+    return method == "morton"
+
+
 class Primitive:
     """The six arrays of `struct Primitive` (Render.hh:122-130), reference byte layouts."""
 
@@ -83,14 +90,15 @@ class DevicePrimitive:
         return cls(up(prim.sphereList), up(prim.squareList), up(prim.cubeList), up(prim.triList), up(prim.idxList), up(prim.bvhList))
 
     @classmethod
-    def build(cls, sphereList=None, squareList=None, cubeList=None, triList=None, idxList=None, device=0):
+    def build(cls, sphereList=None, squareList=None, cubeList=None, triList=None, idxList=None, device=0, method="sah"):
         """BVH::buildNode + BVH::buildTree without leaving the GPU: the leaves are made on `device` in the order of
         harness.build_primitive (AAPLRenderer.mm:454-468,546-591) -- spheres, cubes, squares, then triangles, each kind
         numbered from pIndex 0 -- by trq_bvh_build_nodes_device / trq_bvh_build_nodes_triangles_device, and the tree by
-        trq_bvh_build_tree_device. Arguments are torch uint8 CUDA tensors (or None) on `device` in the reference layouts.
-        Returns the DevicePrimitive, ready for Scene(...)."""
+        trq_bvh_build_tree_device (method="morton": trq_bvh_build_tree_morton_device). Arguments are torch uint8 CUDA tensors
+        (or None) on `device` in the reference layouts. Returns the DevicePrimitive, ready for Scene(...)."""
         import torch
         from . import layout as L
+        morton = _morton(method)
         prim = cls(sphereList, squareList, cubeList, triList, idxList)
         dev = torch.device(f"cuda:{int(device)}")
         for k, t in prim.arrays.items():
@@ -116,7 +124,8 @@ class DevicePrimitive:
                                                            C.c_void_p(stream.cuda_stream)), "trq_bvh_build_nodes_triangles_device")
         stream.synchronize()                     # the tree build runs on the legacy default stream
         nNode, depth = C.c_uint32(0), C.c_uint32(0)
-        check(lib.trq_bvh_build_tree_device(bvh.data_ptr(), n, int(device), C.byref(nNode), C.byref(depth)), "trq_bvh_build_tree_device")
+        fn = lib.trq_bvh_build_tree_morton_device if morton else lib.trq_bvh_build_tree_device
+        check(fn(bvh.data_ptr(), n, int(device), C.byref(nNode), C.byref(depth)), fn.__name__)
         prim.arrays["bvhList"] = bvh
         prim.maxDepth = depth.value
         return prim
@@ -164,8 +173,13 @@ class BVHBuilder:
                                                     nodes.ctypes.data), "trq_bvh_build_nodes_triangles")
         self._chunks.append(nodes)
 
-    def buildTree(self, gpu=None):
-        """BVH::buildTree. gpu=None: host builder; gpu=<device index>: the same tree built on that GPU."""
+    def buildTree(self, gpu=None, method="sah"):
+        """BVH::buildTree. gpu=None: host builder; gpu=<device index>: the same tree built on that GPU.
+        method="morton": the Morton-order builder's tree instead (trq_bvh_build_tree_morton on the host; on a GPU,
+        trq_bvh_build_tree_morton_device through a device copy)."""
+        if _morton(method) and gpu is not None:
+            d = self.buildTreeDevice(gpu, method)
+            return d.cpu().numpy().view(L.bvh_dtype)
         leaves = np.concatenate(self._chunks) if self._chunks else np.zeros(0, dtype=L.bvh_dtype)
         n = leaves.size
         if n == 0:
@@ -173,17 +187,21 @@ class BVHBuilder:
         nodes = np.zeros(2 * n - 1, dtype=L.bvh_dtype)
         nodes[:n] = leaves
         nNode, depth = C.c_uint32(0), C.c_uint32(0)
-        if gpu is None:
+        if method == "morton":
+            check(lib.trq_bvh_build_tree_morton(nodes.ctypes.data, n, C.byref(nNode), C.byref(depth)), "trq_bvh_build_tree_morton")
+        elif gpu is None:
             check(lib.trq_bvh_build_tree(nodes.ctypes.data, n, C.byref(nNode), C.byref(depth)), "trq_bvh_build_tree")
         else:
             check(lib.trq_bvh_build_tree_gpu(nodes.ctypes.data, n, int(gpu), C.byref(nNode), C.byref(depth)), "trq_bvh_build_tree_gpu")
         self.maxDepth = depth.value
         return nodes[: nNode.value]
 
-    def buildTreeDevice(self, device=0):
-        """BVH::buildTree with the node array left ON the GPU (trq_bvh_build_tree_device): returns a torch uint8 CUDA
-        tensor holding the 2n-1 64-byte nodes, ready for DevicePrimitive(bvhList=...)."""
+    def buildTreeDevice(self, device=0, method="sah"):
+        """BVH::buildTree with the node array left ON the GPU (trq_bvh_build_tree_device; method="morton":
+        trq_bvh_build_tree_morton_device): returns a torch uint8 CUDA tensor holding the 2n-1 64-byte nodes, ready for
+        DevicePrimitive(bvhList=...)."""
         import torch
+        morton = _morton(method)
         leaves = np.concatenate(self._chunks) if self._chunks else np.zeros(0, dtype=L.bvh_dtype)
         n = leaves.size
         if n == 0:
@@ -191,7 +209,8 @@ class BVHBuilder:
         d = torch.zeros((2 * n - 1) * L.bvh_dtype.itemsize, dtype=torch.uint8, device=f"cuda:{device}")
         d[: n * L.bvh_dtype.itemsize] = torch.from_numpy(leaves.view(np.uint8).reshape(-1)).to(d.device)
         nNode, depth = C.c_uint32(0), C.c_uint32(0)
-        check(lib.trq_bvh_build_tree_device(d.data_ptr(), n, int(device), C.byref(nNode), C.byref(depth)), "trq_bvh_build_tree_device")
+        fn = lib.trq_bvh_build_tree_morton_device if morton else lib.trq_bvh_build_tree_device
+        check(fn(d.data_ptr(), n, int(device), C.byref(nNode), C.byref(depth)), fn.__name__)
         self.maxDepth = depth.value
         return d
 
@@ -289,18 +308,20 @@ class Scene:
                 setattr(d, _COUNT[k], prim.count(k))
             check(lib.trq_scene_update_primitives(self._h, C.byref(d), 0), "trq_scene_update_primitives")
 
-    def rebuild(self, triList=None):
+    def rebuild(self, triList=None, method="sah"):
         """New topology from the current geometry (trq_scene_rebuild), optionally after moving the vertices: numpy
         `vertex_dtype` array or a torch uint8 CUDA tensor holding all of the scene's vertices; None keeps them. Triangle leaf
-        boxes follow the vertices, other leaves keep theirs. Refreshes `info`; on failure the scene is unchanged."""
+        boxes follow the vertices, other leaves keep theirs. method="morton": the Morton-order builder builds the tree
+        (TRQ_BUILD_MORTON), for a rebuild every frame. Refreshes `info`; on failure the scene is unchanged."""
+        flags = L.BUILD_MORTON if _morton(method) else 0
         if triList is None:
-            check(lib.trq_scene_rebuild(self._h, None, 0, 0), "trq_scene_rebuild")
+            check(lib.trq_scene_rebuild(self._h, None, 0, flags), "trq_scene_rebuild")
         elif isinstance(triList, np.ndarray):
             a = np.ascontiguousarray(triList)
-            check(lib.trq_scene_rebuild(self._h, a.ctypes.data, a.size, L.HOST_PTRS), "trq_scene_rebuild")
+            check(lib.trq_scene_rebuild(self._h, a.ctypes.data, a.size, flags | L.HOST_PTRS), "trq_scene_rebuild")
         else:
             n = triList.numel() * triList.element_size() // L.vertex_dtype.itemsize
-            check(lib.trq_scene_rebuild(self._h, triList.data_ptr(), n, 0), "trq_scene_rebuild")
+            check(lib.trq_scene_rebuild(self._h, triList.data_ptr(), n, flags), "trq_scene_rebuild")
         self._read_info()
 
     def bvh(self):
