@@ -275,7 +275,10 @@ int  trq_expand_hits(trq_scene* scene, const trq_ray* rays, const trq_hit* hits,
 /* ---- wavefront callers (the producers either side of the query; device pointers only) ----------------------
  * With these a cast -> trace -> spawn -> trace ... wavefront stays on the GPU: spawn compacts the surviving rays
  * into `out` with one atomic per warp and leaves their number in device memory (*d_count), which
- * trq_trace_indirect and the next spawn read on the device (no host round trip). */
+ * trq_trace_indirect and the next spawn read on the device (no host round trip).
+ * Overlap: the outputs of a call must not share memory with its inputs. A spawn zeroes *d_count on the stream before its
+ * kernel reads *d_n, so d_count == d_n spawns nothing; out / srcIndex overlapping rays / hits (or trq_trace_indirect's
+ * hits overlapping rays / d_count) is a race whose result is undefined. */
 
 /* Arguments of MakeCamera (RT_Metal/Tracer/Tracer.mm:87-125); vfov in radians, as the reference passes it. */
 typedef struct trq_camera {

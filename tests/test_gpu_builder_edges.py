@@ -262,13 +262,14 @@ def trace_both(port, tri, idx, tree, want_tree, box, seed, where, t_only=False):
     rays = H.random_rays(4000, seed=seed, lo=box[0], hi=box[1])
     for any_hit in (False, True):
         got = gpu_trace(scene, rays, any_hit)
-        want = port.trace(Primitive(triList=tri, idxList=idx, bvhList=want_tree), rays, any=any_hit, nthreads=8)["hits"]
+        want = port.trace(Primitive(triList=tri, idxList=idx, bvhList=want_tree), rays, any=any_hit, records=True, nthreads=8)
+        want, recs = want["hits"], want["records"]
         if t_only:
             assert np.array_equal(got["flags"] & 1, want["flags"] & 1), f"{where} any={any_hit}: hit flags differ"
             if not any_hit:
                 assert np.array_equal(got["t"].view(np.uint32), want["t"].view(np.uint32)), f"{where}: closest t differs"
         else:
-            assert_hits_equal(got, want, f"{where} any={any_hit}")
+            assert_hits_equal(got, want, f"{where} any={any_hit}", recs)
     scene.close()
 
 

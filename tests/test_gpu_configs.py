@@ -9,7 +9,7 @@ import pytest
 
 from tracer_b200 import layout as L
 
-from .test_gpu_parity import _torch, assert_hits_equal, gpu_trace
+from .test_gpu_parity import _torch, assert_hits_equal, assert_like_oracle, gpu_trace, oracle
 
 pytestmark = pytest.mark.gpu
 
@@ -29,7 +29,7 @@ def test_every_configuration_matches_the_oracle(built, port):
     cases = [(soup, H.random_rays(300000, seed=2), False), (soup, H.random_rays(100000, seed=3), True),
              (mixed, H.cornell_camera_rays(320, 180), False),
              (mixed, H.random_rays(100000, seed=5, lo=(-245, 0, 0), hi=(800, 555, 555)), True)]
-    wants = [port.trace(p, r, any=a, nthreads=8)["hits"] for p, r, a in cases]
+    wants = [oracle(port, p, r, a) for p, r, a in cases]
     staged_any = False
     for prim in (soup, mixed):
         scene = Scene(prim, 0)
@@ -43,7 +43,7 @@ def test_every_configuration_matches_the_oracle(built, port):
             staged_any |= staged > 0
             for (p, rays, any_hit), want in zip(cases, wants):
                 if p is prim:
-                    assert_hits_equal(gpu_trace(scene, rays, any_hit), want, f"cfg {name}")
+                    assert_hits_equal(gpu_trace(scene, rays, any_hit), want[0], f"cfg {name}", want[1])
         scene.close()
     assert staged_any
     # the library's own choice: staging only for trees that fit into the staged block whole
@@ -127,8 +127,8 @@ def test_automatic_ray_ordering(built, port):
                 assert torch.equal(auto.view(torch.int32), ref.view(torch.int32))
                 assert torch.equal(hinted.view(torch.int32), ref.view(torch.int32))
             sub = np.arange(0, rays.size, 97)
-            want = port.trace(prim, np.ascontiguousarray(rays[sub]), nthreads=8)["hits"]
-            assert_hits_equal(plain.cpu().numpy().view(L.hit_dtype).reshape(-1)[sub], want, "auto ordering")
+            assert_like_oracle(plain.cpu().numpy().view(L.hit_dtype).reshape(-1)[sub], port, prim, np.ascontiguousarray(rays[sub]),
+                               False, "auto ordering")
     finally:
         del os.environ["TRQ_AUTO_SORT"]
     scene.close()

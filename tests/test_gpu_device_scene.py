@@ -14,7 +14,7 @@ import pytest
 
 from tracer_b200 import layout as L
 
-from .test_gpu_parity import _torch, assert_hits_equal, gpu_trace
+from .test_gpu_parity import _torch, assert_like_oracle, gpu_trace
 from .util import refit_on_host
 
 pytestmark = pytest.mark.gpu
@@ -55,10 +55,9 @@ def test_scene_created_on_the_device_equals_scene_created_from_the_host(built, p
         for rays, any_hit in ((rays_a, False), (rays_b, True)):
             if rays is None:
                 continue
-            want = port.trace(prim, rays, any=any_hit, nthreads=8)["hits"]
             a, b = gpu_trace(host, rays, any_hit), gpu_trace(dev, rays, any_hit)
             assert np.array_equal(a.view(np.uint8), b.view(np.uint8)), "device-planned scene answers differently"
-            assert_hits_equal(b, want, "device-created scene")
+            assert_like_oracle(b, port, prim, rays, any_hit, "device-created scene")
         for c in range(len(Scene.kernel_configs())):           # the staged top-of-tree block must be the same block
             try:
                 host.set_kernel_config(c); dev.set_kernel_config(c)
@@ -118,7 +117,7 @@ def test_build_and_create_without_leaving_the_gpu(built, port):
             scene.close()
     assert np.array_equal(nodes.cpu().numpy().view(L.bvh_dtype).reshape(-1).view(np.uint8), prim.bvhList.view(np.uint8))
     rays = H.random_rays(200000, seed=2)
-    assert_hits_equal(gpu_trace(scene, rays), port.trace(prim, rays, nthreads=8)["hits"], "built + created on the device")
+    assert_like_oracle(gpu_trace(scene, rays), port, prim, rays, False, "built + created on the device")
     scene.close()
 
 
@@ -135,15 +134,14 @@ def test_refit_after_the_vertices_moved(built, port):
         for how in ("host", "device"):
             scene.update_vertices(verts if how == "host" else torch.from_numpy(verts.view(np.uint8).reshape(-1).copy()).cuda())
             for any_hit in (False, True):
-                want = port.trace(moved, rays, any=any_hit, nthreads=8)["hits"]
-                assert_hits_equal(gpu_trace(scene, rays, any_hit), want, f"refit ({how})")
+                assert_like_oracle(gpu_trace(scene, rays, any_hit), port, moved, rays, any_hit, f"refit ({how})")
             for c in range(len(Scene.kernel_configs())):
                 try:
                     scene.set_kernel_config(c)
                 except Exception:
                     continue
-                assert_hits_equal(gpu_trace(scene, rays), port.trace(moved, rays, nthreads=8)["hits"], f"refit cfg {c}")
+                assert_like_oracle(gpu_trace(scene, rays), port, moved, rays, False, f"refit cfg {c}")
             scene.set_kernel_config(-1)
         scene.update_vertices(prim.triList)                     # and back: the original answers return
-        assert_hits_equal(gpu_trace(scene, rays), port.trace(prim, rays, nthreads=8)["hits"], "refit back")
+        assert_like_oracle(gpu_trace(scene, rays), port, prim, rays, False, "refit back")
         scene.close()

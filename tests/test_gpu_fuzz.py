@@ -128,9 +128,9 @@ def test_adversarial_parity(built, port, seed):
         rays = adversarial_rays(rng, prim, 40000)
         d = rays_to_torch(rays, "cuda:0")
         for any_hit in (False, True):
-            want = port.trace(prim, rays, any=any_hit, counters=True, records=not any_hit, nthreads=8)
+            want = port.trace(prim, rays, any=any_hit, counters=True, records=True, nthreads=8)
             got = gpu_trace(scene, rays, any_hit, True)
-            assert_hits_equal(got, want["hits"], f"{name} seed={seed} any={any_hit} reflayout")
+            assert_hits_equal(got, want["hits"], f"{name} seed={seed} any={any_hit} reflayout", want["records"])
             for c in range(ncfg):
                 try:
                     scene.set_kernel_config(c)
@@ -139,7 +139,7 @@ def test_adversarial_parity(built, port, seed):
                 where = f"{name} seed={seed} any={any_hit} cfg={c}"
                 h = scene.hit(d, any=any_hit)
                 got = h.cpu().numpy().view(L.hit_dtype).reshape(-1)
-                assert_hits_equal(got, want["hits"], where)
+                assert_hits_equal(got, want["hits"], where, want["records"])
                 h16 = scene.hit(d, any=any_hit, hit16=True).cpu().numpy().view(L.hit16_dtype).reshape(-1)
                 assert np.array_equal(h16.view(np.uint8), L.pack_hit16(got).view(np.uint8)), where + " hit16"
                 if not any_hit and c == 0:

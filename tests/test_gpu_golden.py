@@ -33,7 +33,7 @@ def test_gpu_matches_reference_golden(built, name, reflayout):
     assert np.array_equal(hits["material"][hit], want["material"][hit])
     assert np.array_equal(((hits["flags"] >> 1) & 1)[hit], want["front"][hit])
     recs = scene.expand(d, h).cpu().numpy().view(L.record_dtype).reshape(-1)
-    assert_records_match_reference(recs, want, hits=hits, sphere_uv_atol=1e-5, where=name)
+    assert_records_match_reference(recs, want, hits=hits, where=name)
     scene.close()
 
 
@@ -209,24 +209,23 @@ def test_c4_any_hit_full_scene(built, port):
     assert bool((c["t"][occluded] <= got["t"][occluded]).all())
 
 
-def test_c1_sphere_scene_full_batch(built, port):
-    """BASELINE C1: the 485-sphere randomScene as Sphere leaves, all 921,600 primary rays against the oracle."""
+def test_c1_sphere_scene_full_batch(built, port, capsys):
+    """BASELINE C1: the 485-sphere randomScene as Sphere leaves, all 921,600 primary rays against the oracle: ids and t bit
+    for bit, sphere uv (atan2f / asinf) inside CUDA's documented error of the float64 value (assert_sphere_uv), the
+    oracle's bits at the poles -- where rounding pushes |gn.y| above 1 on the r = 1000 ground sphere, both sides give NaN."""
     _torch()
     from tracer_b200 import Scene, harness as H, hits_to_numpy, rays_to_torch
+    from .test_gpu_parity import assert_hits_equal
+    from .test_special_rays_cpu import sphere_uv_error
     prim = H.scene_c1()
     scene = Scene(prim, 0)
     rays = H.camera_rays((13, 2, 3), (0, 0, 0), np.float32(20 * np.pi / 180), 1280, 720)
     assert rays.size == 921_600
     got = hits_to_numpy(scene.hit(rays_to_torch(rays, "cuda:0")))
-    want = port.trace(prim, rays, nthreads=8)["hits"]
-    for k in ("flags", "pType", "pIndex", "leafNode", "material"):
-        assert np.array_equal(got[k], want[k]), k
-    assert np.array_equal(bits(got["t"]), bits(want["t"]))
-    hit = (want["flags"] & 1) == 1
-    for k in ("u", "v"):                                         # sphere uv: atan2f / asinf, libm vs CUDA (ulps apart)
-        g, w = got[k][hit], want[k][hit]
-        # asin(gn.y) is NaN on both sides where rounding pushes |gn.y| above 1 (top of the r = 1000 ground sphere)
-        assert np.array_equal(np.isnan(g), np.isnan(w)), f"{k}: NaN pattern differs"
-        ok = ~np.isnan(w)
-        err = np.abs(g[ok] - w[ok])
-        assert err.max() <= 1e-5, f"{k}: max |diff| {err.max()} at {np.argmax(err)}"
+    want = port.trace(prim, rays, records=True, nthreads=8)
+    assert_hits_equal(got, want["hits"], "c1", want["records"])
+    sph = (want["hits"]["flags"] & 1) == 1
+    assert (want["hits"]["pType"][sph] == L.SPHERE).all() and sph.sum() > 500_000
+    eu, ev = sphere_uv_error(got["u"][sph], got["v"][sph], want["records"]["gn"][sph])
+    with capsys.disabled():
+        print(f"\nC1 full batch, sphere uv: largest error of phi (atan2f) {eu} ulp, of theta (asinf) {ev} ulp")

@@ -16,7 +16,7 @@ from tracer_b200._lib import ERR_DEPTH, ERR_INVALID, TrqError, check, lib
 from .morton_util import (chain_points, check_morton_structure, host_morton, mixed_leaves, morton_codes, morton_rebuild_on_host,
                           point_leaves, rebuild_leaves, reference_cornell_leaves)
 from .test_gpu_builder_edges import COMBS, EXACT, LARGE, soup
-from .test_gpu_parity import assert_hits_equal, gpu_trace
+from .test_gpu_parity import assert_hits_equal, assert_like_oracle, gpu_trace, oracle
 from .test_gpu_tree_shapes import (_check_configurations, _leaf_items, _trace_everything, comb_rays, refit_case, tree_rays,
                                    with_finite_tmax)
 from .update_util import update_on_host
@@ -207,7 +207,7 @@ def test_morton_rebuild_after_motion(built, port, how, source):
     refit = refit_on_host(want, again)
     assert scene.bvh().tobytes() == refit.bvhList.tobytes()
     for any_hit in (False, True):
-        assert_hits_equal(gpu_trace(scene, rays, any_hit), port.trace(refit, rays, any=any_hit, nthreads=8)["hits"], f"refit any={any_hit}")
+        assert_like_oracle(gpu_trace(scene, rays, any_hit), port, refit, rays, any_hit, f"refit any={any_hit}")
     scene.rebuild(method="sah")                             # and the SAH builder takes it back
     from .rebuild_util import rebuild_on_host
     assert scene.bvh().tobytes() == rebuild_on_host(refit).bvhList.tobytes()
@@ -234,14 +234,11 @@ def test_morton_rebuild_then_update_primitives(built, port):
     assert scene.bvh().tobytes() == moved.bvhList.tobytes()
     rays = H.cornell_camera_rays(160, 90)
     for any_hit in (False, True):
-        got, ref = gpu_trace(scene, rays, any_hit), port.trace(moved, rays, any=any_hit, nthreads=8)["hits"]
-        sph = ref["pType"] == L.SPHERE
-        for k in ref.dtype.names:
-            if k in ("u", "v"):
-                assert np.allclose(got[k][sph], ref[k][sph], rtol=0, atol=1e-5), k      # sphereUV: CUDA vs libm
-                assert np.array_equal(got[k][~sph].view(np.uint32), ref[k][~sph].view(np.uint32)), k
-            else:
-                assert np.array_equal(got[k].view(np.uint32), ref[k].view(np.uint32)), (k, any_hit)
+        got, (want, recs) = gpu_trace(scene, rays, any_hit), oracle(port, moved, rays, any_hit)
+        assert_hits_equal(got, want, f"moved any={any_hit}", recs)
+        miss = (want["flags"] & 1) == 0                          # and the u / v bytes of the misses
+        for k in ("u", "v"):
+            assert np.array_equal(got[k][miss].view(np.uint32), want[k][miss].view(np.uint32)), (k, any_hit)
     scene.close()
 
 

@@ -62,7 +62,7 @@ def test_spawn_bounce_and_shadow_match_host(cornell):
         assert np.array_equal(src.cpu().numpy()[:n].astype(np.uint32)[order], wsrc)
         assert np.array_equal(bits(got["o"]), bits(want["o"])), "offset_ray origins must be bit-exact"
         if kind == "shadow":
-            assert np.allclose(got["tmax"], want["tmax"], rtol=1e-6)
+            assert np.array_equal(bits(got["tmax"]), bits(want["tmax"])), "shadow lengths: strict fp32 sqrtf, bit-exact"
             assert np.array_equal(bits(got["d"]), bits(want["d"])), "shadow directions use no libm: bit-exact"
         else:
             assert (got["tmax"] == np.float32(L.FLT_MAX)).all()

@@ -14,7 +14,7 @@ from tracer_b200 import harness as H, layout as L
 from tracer_b200._lib import ERR_DEPTH, ERR_INVALID, TrqError, check, lib
 
 from .test_gpu_builder_edges import COMBS
-from .test_gpu_parity import assert_hits_equal, gpu_trace
+from .test_gpu_parity import assert_like_oracle, gpu_trace
 from .test_gpu_tree_shapes import (_check_configurations, _leaf_items, _trace_everything, expected_staging, refit_case, tree_case, tree_rays,
                                    with_finite_tmax)
 from .rebuild_util import reachable, rebuild_on_host
@@ -182,7 +182,7 @@ def _answers(scene, rays):
 
 def _assert_oracle(port, prim, scene, rays, where):
     for any_hit, got in zip((False, True), _answers(scene, rays)):
-        assert_hits_equal(got, port.trace(prim, rays, any=any_hit, nthreads=8)["hits"], f"{where} any={any_hit}")
+        assert_like_oracle(got, port, prim, rays, any_hit, f"{where} any={any_hit}")
 
 
 @pytest.mark.parametrize("name", ["c1", "c2", "reference_cornell", "soup300k"])

@@ -14,9 +14,8 @@ from tracer_b200 import layout as L
 
 from .test_gpu_fuzz import _assert_records
 from .test_gpu_parity import _torch, gpu_trace
-from .test_special_rays_cpu import (ULP_ASINF, ULP_ATAN2F, _nan_aware_equal, aimed_rays, bounce_direction_candidates, comb_right, degenerate_scene,
-                                    flat_cube_scene, nan_origin_rays, one_leaf, pole_spheres_scene, special_rays,
-                                    sphere_uv_interval)
+from .test_special_rays_cpu import (_nan_aware_equal, _seen, aimed_rays, assert_sphere_uv, bounce_direction_candidates, comb_right,
+                                    degenerate_scene, flat_cube_scene, nan_origin_rays, one_leaf, pole_spheres_scene, special_rays)
 from .util import bits
 
 pytestmark = pytest.mark.gpu
@@ -24,39 +23,9 @@ pytestmark = pytest.mark.gpu
 f32 = np.float32
 
 
-_seen = {"u": 0, "v": 0}
-
-
-def assert_sphere_uv(u, v, gn, want_u, want_v, where):
-    """Sphere uv of hits with oracle shading normal gn. Where atan2 (u) or asin (v) is at a special point -- gn.x or gn.z
-    at +-0, |gn.y| >= 1, a non-finite component -- the oracle's bits (NaN-aware); elsewhere inside the interval of
-    sphere_uv_interval."""
-    fin = np.isfinite(gn).all(axis=1)
-    with np.errstate(invalid="ignore"):
-        su = ~fin | (gn[:, 0] == 0) | (gn[:, 2] == 0)
-        sv = ~fin | (np.abs(gn[:, 1]) >= 1)
-    assert _nan_aware_equal(u[su], want_u[su]), f"{where}: sphere u on the seam: {u[su][:3]} want {want_u[su][:3]}"
-    assert _nan_aware_equal(v[sv], want_v[sv]), f"{where}: sphere v at a pole: {v[sv][:3]} want {want_v[sv][:3]}"
-    gf = np.where(fin[:, None], gn, f32(0))
-    ulo, uhi, vlo, vhi, _, _ = sphere_uv_interval(gf)
-    for name, x, lo, hi, special in (("u", u, ulo, uhi, su), ("v", v, vlo, vhi, sv)):
-        bad = ~special & ~((x >= lo) & (x <= hi))
-        assert not bad.any(), f"{where}: sphere {name} outside [{lo[bad][:3]}, {hi[bad][:3]}]: {x[bad][:3]}, gn {gn[bad][:3]}"
-    for k in range(max(ULP_ATAN2F, ULP_ASINF) + 1):                  # the largest error of atan2f / asinf actually seen
-        ulo, uhi, vlo, vhi, _, _ = sphere_uv_interval(gf, k, k)
-        if ((u >= ulo) & (u <= uhi) | su).all():
-            _seen["u"] = max(_seen["u"], k)
-            break
-    for k in range(max(ULP_ATAN2F, ULP_ASINF) + 1):
-        ulo, uhi, vlo, vhi, _, _ = sphere_uv_interval(gf, k, k)
-        if ((v >= vlo) & (v <= vhi) | sv).all():
-            _seen["v"] = max(_seen["v"], k)
-            break
-
-
 def assert_hits_exact(got, want, where, records=None):
     """trq_hit against the oracle: ids and flags equal, t bit for bit, u / v bit for bit except sphere hits (NaN-aware);
-    sphere uv by assert_sphere_uv when the oracle's records are given."""
+    sphere uv by assert_sphere_uv against the oracle's records, which are required when the oracle reports a sphere hit."""
     assert got.size == want.size
     for k in ("flags", "pType", "pIndex", "leafNode", "material"):
         bad = np.nonzero(got[k] != want[k])[0]
@@ -66,7 +35,9 @@ def assert_hits_exact(got, want, where, records=None):
     sph = hit & (want["pType"] == L.SPHERE)
     for k in ("u", "v"):
         assert _nan_aware_equal(got[k][hit & ~sph], want[k][hit & ~sph]), f"{where}: {k}"
-    if records is not None and sph.any():
+    if sph.any():
+        assert records is not None, f"{where}: {int(sph.sum())} sphere hits: pass the oracle's records to check their uv"
+        assert records.size == want.size, f"{where}: records of other rays"
         assert_sphere_uv(got["u"][sph], got["v"][sph], records["gn"][sph], want["u"][sph], want["v"][sph], where)
 
 

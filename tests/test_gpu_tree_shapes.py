@@ -557,15 +557,15 @@ def _trace_everything(port, prim, scene, rays, rays_any, where, cfgs):
     out = []
     level = 0
     for any_hit, r in ((False, rays), (True, rays_any)):
-        want = port.trace(prim, r, any=any_hit, records=not any_hit, counters=True, nthreads=8)
-        assert_hits_equal(gpu_trace(scene, r, any_hit, reflayout=True), want["hits"], f"{where} any={any_hit} reflayout")
+        want = port.trace(prim, r, any=any_hit, records=True, counters=True, nthreads=8)
+        assert_hits_equal(gpu_trace(scene, r, any_hit, reflayout=True), want["hits"], f"{where} any={any_hit} reflayout", want["records"])
         d = rays_to_torch(r, f"cuda:{scene.device}")
         for c in cfgs:
             scene.set_kernel_config(c)
             at = f"{where} any={any_hit} cfg={c}"
             h = scene.hit(d, any=any_hit)
             got = h.cpu().numpy().view(L.hit_dtype).reshape(-1)
-            assert_hits_equal(got, want["hits"], at)
+            assert_hits_equal(got, want["hits"], at, want["records"])
             h16 = scene.hit(d, any=any_hit, hit16=True).cpu().numpy().view(L.hit16_dtype).reshape(-1)
             assert np.array_equal(h16.view(np.uint8), L.pack_hit16(got).view(np.uint8)), at + " hit16"
             if not any_hit and c == cfgs[0]:
@@ -740,7 +740,7 @@ def test_refit_of_caller_built_trees(built, port, name):
     host and from a device vertex source; then the original vertices back."""
     torch = _torch()
     from tracer_b200 import Scene
-    from .test_gpu_parity import assert_hits_equal, gpu_trace
+    from .test_gpu_parity import assert_like_oracle, gpu_trace
     prim, verts = refit_case(name)
     moved = refit_on_host(prim, verts)
     rng = np.random.default_rng(7)
@@ -761,6 +761,5 @@ def test_refit_of_caller_built_trees(built, port, name):
             assert level == MAX_DEPTH
         scene.update_vertices(prim.triList)                    # and back: the original geometry's answers return
         for any_hit in (False, True):
-            want = port.trace(back, old_rays, any=any_hit, nthreads=8)["hits"]
-            assert_hits_equal(gpu_trace(scene, old_rays, any_hit), want, f"refit {name} back ({how})")
+            assert_like_oracle(gpu_trace(scene, old_rays, any_hit), port, back, old_rays, any_hit, f"refit {name} back ({how})")
     scene.close()

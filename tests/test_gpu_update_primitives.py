@@ -62,53 +62,6 @@ def _same_except_boxes(a, b, where):
             assert a[k].tobytes() == b[k].tobytes(), f"{where}: {k}"
 
 
-def _uv_comparable(port, prim, rays, rays_any):
-    """Mask of the rays whose sphere uv test_gpu_parity.assert_hits_equal can compare (atol 1e-5) between CUDA's asinf /
-    atan2f and libm's. Not comparable: a sphere hit with a NaN u or v (a normal rounded just past a pole), and, on a sphere
-    of radius below 100, a hit within about 1 % of a pole in v or on the u seam, where an ulp of the normal moves uv by
-    more than the tolerance. (C1's ground sphere, radius 1000, is hit near its pole everywhere, well inside it.) The other
-    rays' fields are still compared, by _assert_hits_except_uv."""
-    keep = np.ones(rays.size, dtype=bool)
-    if prim.sphereList.size == 0:
-        return keep
-    for r, any_hit in ((rays, False), (rays_any, True)):
-        h = port.trace(prim, r, any=any_hit, nthreads=8)["hits"]
-        sph = ((h["flags"] & 1) == 1) & (h["pType"] == L.SPHERE)
-        small = prim.sphereList["radius"][np.where(sph, h["pIndex"], 0)] < f32(100)
-        cos_lat = np.sin(np.pi * h["v"].astype(np.float64))
-        seam = np.minimum(h["u"], 1 - h["u"]) < 1e-4
-        nan = ~(np.isfinite(h["u"]) & np.isfinite(h["v"]))
-        keep &= ~(sph & (nan | (small & ((cos_lat < 0.04) | seam))))
-    assert keep.mean() > 0.8
-    return keep
-
-
-def _assert_hits_except_uv(port, prim, scene, rays, rays_any, cfgs, where):
-    """Every hit field but u and v against the oracle: the reference-layout kernel and the packed kernel in each of cfgs."""
-    from .test_gpu_parity import gpu_trace
-    for any_hit, r in ((False, rays), (True, rays_any)):
-        if r.size == 0:
-            continue
-        want = port.trace(prim, r, any=any_hit, nthreads=8)["hits"]
-        got = [("reflayout", gpu_trace(scene, r, any_hit, reflayout=True))]
-        for c in cfgs:
-            scene.set_kernel_config(c)
-            got.append((f"cfg={c}", gpu_trace(scene, r, any_hit)))
-        scene.set_kernel_config(-1)
-        for how, g in got:
-            at = f"{where} any={any_hit} {how} (uv not comparable)"
-            for k in ("flags", "pType", "pIndex", "leafNode", "material"):
-                assert np.array_equal(g[k], want[k]), f"{at}: {k}"
-            assert np.array_equal(g["t"].view(np.uint32), want["t"].view(np.uint32)), f"{at}: t"
-
-
-def _assert_like_oracle(port, prim, scene, rays, where):
-    """test_gpu_rebuild._assert_oracle, with the rays whose sphere uv cannot be compared checked on every other field."""
-    keep = _uv_comparable(port, prim, rays, rays)
-    _assert_oracle(port, prim, scene, rays[keep], where)
-    _assert_hits_except_uv(port, prim, scene, rays[~keep], rays[~keep], _cfgs(scene), where)
-
-
 def _check(port, scene, want, info, rays, rays_any, where, exact=True):
     """The updated scene against the restatement `want`. exact=False (non-finite records): leaves byte for byte, interior
     boxes by value (+-0 equal, NaN equal), every other field byte for byte; the traces then run on the scene's own tree and
@@ -128,9 +81,7 @@ def _check(port, scene, want, info, rays, rays_any, where, exact=True):
     assert _info(scene) == info, where
     cfgs = _cfgs(scene)
     if exact:
-        keep = _uv_comparable(port, want, rays, rays_any)
-        _trace_everything(port, want, scene, rays[keep], rays_any[keep], where, cfgs)
-        _assert_hits_except_uv(port, want, scene, rays[~keep], rays_any[~keep], cfgs, where)
+        _trace_everything(port, want, scene, rays, rays_any, where, cfgs)
     fresh = Scene(want, 0)
     for a, b in zip(_hits(scene, rays, rays_any, cfgs), _hits(fresh, rays, rays_any, cfgs)):
         assert a.tobytes() == b.tobytes(), f"{where}: a scene created from the new lists traces differently"
@@ -415,7 +366,7 @@ def test_c4_spheres_and_lights_move(built, port):
     assert np.array_equal(src.cpu().numpy()[:n].astype(np.uint32)[order], wsrc)
     assert np.array_equal(got["o"].view(np.uint32), want_rays["o"].view(np.uint32))
     assert np.array_equal(got["d"].view(np.uint32), want_rays["d"].view(np.uint32)), "shadow directions use no libm: bit-exact"
-    assert np.allclose(got["tmax"], want_rays["tmax"], rtol=1e-6)
+    assert np.array_equal(got["tmax"].view(np.uint32), want_rays["tmax"].view(np.uint32)), "shadow lengths: strict fp32 sqrtf, bit-exact"
     assert not np.array_equal(want_rays["d"], old_rays["d"])
     torch.cuda.synchronize()
     scene.close()
@@ -453,7 +404,7 @@ def test_update_then_rebuild(built, port, name):
     assert scene.bvh().tobytes() == want.bvhList.tobytes(), name
     assert scene.bvh().tobytes() != prim.bvhList.tobytes(), name
     rays = _c1_rays(rng)[0] if name == "c1" else H.cornell_camera_rays(160, 90)
-    _assert_like_oracle(port, want, scene, rays, f"{name} update then rebuild")
+    _assert_oracle(port, want, scene, rays, f"{name} update then rebuild")
     scene.close()
 
 
@@ -487,7 +438,7 @@ def test_failed_update_leaves_the_scene_intact(built, port):
     for a, b in zip(before, _hits(scene, rays, rays_any, _cfgs(scene))):
         assert a.tobytes() == b.tobytes()
     assert scene.expand(d, scene.hit(d)).cpu().numpy().tobytes() == recs.tobytes()
-    _assert_like_oracle(port, prim, scene, rays, "after failed updates")
+    _assert_oracle(port, prim, scene, rays, "after failed updates")
     scene.close()
 
 

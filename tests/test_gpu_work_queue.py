@@ -23,7 +23,7 @@ import pytest
 from tracer_b200 import layout as L
 
 from .test_gpu_fuzz import adversarial_rays
-from .test_gpu_parity import _torch, assert_hits_equal, gpu_trace
+from .test_gpu_parity import _torch, assert_hits_equal, assert_like_oracle, gpu_trace, oracle
 from .test_gpu_tree_shapes import MAX_DEPTH, comb_prim, comb_rays
 
 pytestmark = pytest.mark.gpu
@@ -93,7 +93,7 @@ def test_graphs_captured_4096_launches_apart_replay_concurrently(soup, port):
     for rays, want, where in ((A, wantA, "A"), (B, wantB, "B")):
         sub = np.unique(np.concatenate([np.arange(0, rays.size, 997), np.arange(rays.size - 40, rays.size)]))
         got = want.cpu().numpy().view(L.hit_dtype).reshape(-1)[sub]
-        assert_hits_equal(got, port.trace(prim, np.ascontiguousarray(rays[sub]), nthreads=8)["hits"], f"eager {where}")
+        assert_like_oracle(got, port, prim, np.ascontiguousarray(rays[sub]), False, f"eager {where}")
 
     scene = Scene(prim, 0)
     outA, outB = torch.empty_like(wantA), torch.empty_like(wantB)
@@ -302,14 +302,14 @@ def test_every_scheduler_setting_gives_the_default_bytes(built, port, variants, 
         for rname, rays, count in cases[sname]:
             live = rays if count is None else rays[:count]
             for a in (False, True):
-                want = port.trace(prim, np.ascontiguousarray(live), any=a, nthreads=8)["hits"]
+                want, recs = oracle(port, prim, np.ascontiguousarray(live), a)
                 for c in (0, 1):
                     if f"{sname}/cfg{c}/staged" not in default:
                         continue
                     key = f"{sname}/{rname}/cfg{c}/any{int(a)}"
                     h32 = default[key + "/h32"].view(L.hit_dtype)
                     h16 = default[key + "/h16"].view(L.hit16_dtype)
-                    assert_hits_equal(h32[:live.size], want, key)
+                    assert_hits_equal(h32[:live.size], want, key, recs)
                     assert np.array_equal(h16[:live.size].view(np.uint8), L.pack_hit16(h32[:live.size]).view(np.uint8)), key + " hit16"
                     if count is not None:
                         assert (h32[count:].view(np.uint8) == 0xFF).all() and (h16[count:].view(np.uint8) == 0xFF).all(), \
@@ -353,7 +353,7 @@ def test_every_staged_prefix_size_matches_the_oracle(soup, port):
     rays = np.ascontiguousarray(np.concatenate([H.random_rays(60000, seed=71), adversarial_rays(rng, prim, 8000)]))
     short = rays.copy()
     short["tmax"] = f32(0.05)
-    want = {False: port.trace(prim, rays, nthreads=8)["hits"], True: port.trace(prim, short, any=True, nthreads=8)["hits"]}
+    want = {False: oracle(port, prim, rays), True: oracle(port, prim, short, True)}
     for value in (0, 1, 2, 3, 7, 100, 2046, 2047):
         os.environ["TRQ_TOP_NODES"] = str(value)
         try:
@@ -365,8 +365,8 @@ def test_every_staged_prefix_size_matches_the_oracle(soup, port):
                 scene.set_kernel_config(1)
         else:
             assert scene.set_kernel_config(1) == min(value, fits), value
-            assert_hits_equal(gpu_trace(scene, rays, False), want[False], f"TRQ_TOP_NODES={value} closest")
-            assert_hits_equal(gpu_trace(scene, short, True), want[True], f"TRQ_TOP_NODES={value} any")
+            assert_hits_equal(gpu_trace(scene, rays, False), want[False][0], f"TRQ_TOP_NODES={value} closest", want[False][1])
+            assert_hits_equal(gpu_trace(scene, short, True), want[True][0], f"TRQ_TOP_NODES={value} any", want[True][1])
         scene.close()
 
 
@@ -409,7 +409,7 @@ def test_batches_past_the_launch_limit_are_split(built, port, variants, tmp_path
     scene.close()
     assert want["launches"].tolist() == [1, 1]
     sub = np.arange(0, SPLIT_N, 61)
-    assert_hits_equal(want["closest"].view(L.hit_dtype)[sub], port.trace(prim, np.ascontiguousarray(rays[sub]), nthreads=8)["hits"], "product")
+    assert_like_oracle(want["closest"].view(L.hit_dtype)[sub], port, prim, np.ascontiguousarray(rays[sub]), False, "product")
     out = tmp_path / "split.npz"
     _run_worker("split", tmp_path / "unused", out, {"TRQ_LIB": variants["maxrays16"]})
     got = np.load(out)
@@ -461,8 +461,8 @@ def test_more_than_2_31_rays(built, port):
     want16 = scene.hit(base, hit16=True, sort=False)
     want32 = scene.hit(base, sort=False)
     sub = np.concatenate([np.arange(0, M, 101), [M - 1]])
-    assert_hits_equal(want32.cpu().numpy().view(L.hit_dtype).reshape(-1)[sub],
-                      port.trace(prim, np.ascontiguousarray(base_h[sub]), nthreads=8)["hits"], "base")
+    assert_like_oracle(want32.cpu().numpy().view(L.hit_dtype).reshape(-1)[sub], port, prim, np.ascontiguousarray(base_h[sub]),
+                       False, "base")
     chunk = 1 << 26
     rays = torch.empty((n, 8), dtype=torch.float32, device="cuda:0")
     for lo in range(0, n, chunk):

@@ -270,6 +270,49 @@ def _nan_aware_equal(a, b):
     return np.array_equal(na, nb) and np.array_equal(bits(a)[~na], bits(b)[~nb])
 
 
+_seen = {"u": 0, "v": 0}                                              # largest atan2f / asinf error seen, in ulps
+
+
+def assert_sphere_uv(u, v, gn, want_u, want_v, where):
+    """Sphere uv of hits with oracle shading normal gn. Where atan2 (u) or asin (v) is at a special point -- gn.x or gn.z
+    at +-0, |gn.y| >= 1, a non-finite component -- the oracle's bits (NaN-aware); elsewhere inside the interval of
+    sphere_uv_interval."""
+    fin = np.isfinite(gn).all(axis=1)
+    with np.errstate(invalid="ignore"):
+        su = ~fin | (gn[:, 0] == 0) | (gn[:, 2] == 0)
+        sv = ~fin | (np.abs(gn[:, 1]) >= 1)
+    assert _nan_aware_equal(u[su], want_u[su]), f"{where}: sphere u on the seam: {u[su][:3]} want {want_u[su][:3]}"
+    assert _nan_aware_equal(v[sv], want_v[sv]), f"{where}: sphere v at a pole: {v[sv][:3]} want {want_v[sv][:3]}"
+    gf = np.where(fin[:, None], gn, f32(0))
+    ulo, uhi, vlo, vhi, _, _ = sphere_uv_interval(gf)
+    for name, x, lo, hi, special in (("u", u, ulo, uhi, su), ("v", v, vlo, vhi, sv)):
+        bad = ~special & ~((x >= lo) & (x <= hi))
+        assert not bad.any(), f"{where}: sphere {name} outside [{lo[bad][:3]}, {hi[bad][:3]}]: {x[bad][:3]}, gn {gn[bad][:3]}"
+    eu, ev = sphere_uv_error(u, v, gn)
+    _seen["u"], _seen["v"] = max(_seen["u"], eu), max(_seen["v"], ev)
+
+
+def sphere_uv_error(u, v, gn):
+    """-> (atan2f ulps, asinf ulps): the smallest k for which sphere_uv_interval(gn, k, k) holds every u / v off the
+    special points (as assert_sphere_uv), None when none up to the documented bound does; for reporting."""
+    fin = np.isfinite(gn).all(axis=1)
+    with np.errstate(invalid="ignore"):
+        su = ~fin | (gn[:, 0] == 0) | (gn[:, 2] == 0)
+        sv = ~fin | (np.abs(gn[:, 1]) >= 1)
+    gf = np.where(fin[:, None], gn, f32(0))
+    out = []
+    for name, x, special in (("u", u, su), ("v", v, sv)):
+        for k in range(max(ULP_ATAN2F, ULP_ASINF) + 1):
+            ulo, uhi, vlo, vhi, _, _ = sphere_uv_interval(gf, k, k)
+            lo, hi = (ulo, uhi) if name == "u" else (vlo, vhi)
+            if ((x >= lo) & (x <= hi) | special).all():
+                out.append(k)
+                break
+        else:
+            out.append(None)
+    return tuple(out)
+
+
 def bounce_direction_candidates(sn, u0, u1):
     """Every direction spawn_bounce can give for shading normal sn and draws (u0, u1) when cosf / sinf return any float32
     within their ulp bounds of cos / sin (float64) at the float32 theta: concentric_sample_disk, z, coordinate_system,

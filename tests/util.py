@@ -61,15 +61,20 @@ def refit_on_host(prim, verts):
                      idxList=prim.idxList, bvhList=nodes)
 
 
-def assert_records_match_reference(recs, want, hits=None, sphere_uv_atol=None, where=""):
-    """Bit-exact comparison of HitRecord dumps on the rays the reference reports as hit."""
+def assert_records_match_reference(recs, want, hits=None, where=""):
+    """Bit-exact comparison of HitRecord dumps on the rays the reference reports as hit. hits: the trq_hit rows of a GPU
+    trace of the same rays; their sphere hits' uv comes from CUDA's atan2f / asinf, and is held to
+    test_special_rays_cpu.assert_sphere_uv against the reference's shading normals instead."""
     assert np.array_equal(recs["hit"], want["hit"]), f"{where}: hit flags differ"
     m = want["hit"] == 1
     for k in ("t", "p", "gn", "sn", "front", "material"):
         assert np.array_equal(bits(recs[k][m]), bits(want[k][m])), f"{where}: {k} differs"
-    if sphere_uv_atol is None or hits is None:
+    if hits is None:
         assert np.array_equal(bits(recs["uv"][m]), bits(want["uv"][m])), f"{where}: uv differs"
     else:
-        sph = hits["pType"] == L.SPHERE
+        from .test_special_rays_cpu import assert_sphere_uv
+        sph = m & (hits["pType"] == L.SPHERE)
         assert np.array_equal(bits(recs["uv"][m & ~sph]), bits(want["uv"][m & ~sph])), f"{where}: uv differs"
-        assert np.allclose(recs["uv"][m & sph], want["uv"][m & sph], rtol=0, atol=sphere_uv_atol), f"{where}: sphere uv"
+        if sph.any():
+            assert_sphere_uv(recs["uv"][sph, 0], recs["uv"][sph, 1], want["gn"][sph], want["uv"][sph, 0], want["uv"][sph, 1],
+                             f"{where}: sphere uv")

@@ -24,6 +24,41 @@ def _ptr(a):
     return None if a is None or a.size == 0 else a.ctypes.data
 
 
+def _device_arg(t, name, dtype, device, width=None, at_least=None, exactly=None):
+    """Refuses a tensor the C-ABI would misread, before anything is launched: TypeError unless `t` is a contiguous CUDA
+    tensor of `dtype` with shape (rows, width) (width None: one dimension); ValueError unless it is on cuda:`device` and has
+    at least `at_least` (or exactly `exactly`) rows."""
+    import torch
+    if not isinstance(t, torch.Tensor) or not t.is_cuda:
+        raise TypeError(f"{name} must be a CUDA tensor")
+    if t.dtype != dtype:
+        raise TypeError(f"{name} must be {dtype}, not {t.dtype}")
+    if not t.is_contiguous():
+        raise TypeError(f"{name} must be contiguous")
+    if (t.dim() != 1) if width is None else (t.dim() != 2 or t.shape[1] != width):
+        raise TypeError(f"{name} must have shape {'(n,)' if width is None else f'(n, {width})'}, not {tuple(t.shape)}")
+    if t.device.index != device:
+        raise ValueError(f"{name} is on {t.device}, the scene on cuda:{device}")
+    if at_least is not None and t.shape[0] < at_least:
+        raise ValueError(f"{name} has {t.shape[0]} rows, needs at least {at_least}")
+    if exactly is not None and t.shape[0] != exactly:
+        raise ValueError(f"{name} has {t.shape[0]} rows, needs exactly {exactly}")
+    return t
+
+
+def _disjoint(outputs, inputs):
+    """ValueError if an output shares a byte of memory with an input or with another output (dicts name -> tensor, None:
+    absent): the kernels read the one while writing the other, and the spawns zero `count` on the stream before they read
+    `count_in`. Inputs may share memory with each other: reading a buffer twice is harmless."""
+    def spans(d):
+        return [(k, t.data_ptr(), t.data_ptr() + t.numel() * t.element_size()) for k, t in d.items() if t is not None and t.numel()]
+    outs, ins = spans(outputs), spans(inputs)
+    for i, (a, lo, hi) in enumerate(outs):
+        for b, lo2, hi2 in outs[i + 1:] + ins:
+            if lo < hi2 and lo2 < hi:
+                raise ValueError(f"{a} and {b} share memory")
+
+
 def _morton(method):
     """True for method="morton" (the Morton-order builder), False for "sah" (the reference's binned-SAH builder)."""
     if method not in ("sah", "morton"):
@@ -257,11 +292,11 @@ class Scene:
             check(lib.trq_trace(self._h, rays.ctypes.data, rays.size, flags | L.HOST_PTRS, hits.ctypes.data, None), "trq_trace")
             return hits
         import torch
-        if not (rays.is_cuda and rays.dtype == torch.float32 and rays.dim() == 2 and rays.shape[1] == 8 and rays.is_contiguous()):
-            raise TypeError("device rays must be a contiguous CUDA float32 tensor of shape (n, 8)")
-        if rays.device.index != self.device:
-            raise ValueError("rays are on a different device than the scene")
+        _device_arg(rays, "rays", torch.float32, self.device, 8)
         n = rays.shape[0]
+        if out is not None:
+            _device_arg(out, "out", torch.float32, self.device, width, at_least=n)
+            _disjoint(dict(out=out), dict(rays=rays))
         hits = out if out is not None else torch.empty((n, width), dtype=torch.float32, device=rays.device)
         st = stream if stream is not None else torch.cuda.current_stream(rays.device).cuda_stream
         check(lib.trq_trace(self._h, rays.data_ptr(), n, flags, hits.data_ptr(), C.c_void_p(st)), "trq_trace")
@@ -273,8 +308,15 @@ class Scene:
             a = np.ascontiguousarray(triList)
             check(lib.trq_scene_update_vertices(self._h, a.ctypes.data, a.size, L.HOST_PTRS), "trq_scene_update_vertices")
         else:
-            n = triList.numel() * triList.element_size() // L.vertex_dtype.itemsize
+            n = self._device_vertices(triList, "update_vertices")
             check(lib.trq_scene_update_vertices(self._h, triList.data_ptr(), n, 0), "trq_scene_update_vertices")
+
+    def _device_vertices(self, triList, who):
+        """-> the vertex count of a device vertex list, after the checks DevicePrimitive and update_primitives make."""
+        DevicePrimitive(triList=triList)
+        if triList.device.index != self.device:
+            raise ValueError(f"{who}: triList is on {triList.device}, the scene on cuda:{self.device}")
+        return triList.numel() * triList.element_size() // L.vertex_dtype.itemsize
 
     def update_primitives(self, spheres=None, squares=None, cubes=None, triList=None):
         """Refit after primitives moved (trq_scene_update_primitives, same topology): each argument given replaces that list
@@ -320,7 +362,7 @@ class Scene:
             a = np.ascontiguousarray(triList)
             check(lib.trq_scene_rebuild(self._h, a.ctypes.data, a.size, flags | L.HOST_PTRS), "trq_scene_rebuild")
         else:
-            n = triList.numel() * triList.element_size() // L.vertex_dtype.itemsize
+            n = self._device_vertices(triList, "rebuild")
             check(lib.trq_scene_rebuild(self._h, triList.data_ptr(), n, flags), "trq_scene_rebuild")
         self._read_info()
 
@@ -362,9 +404,13 @@ class Scene:
     def cast_rays(self, look_from, look_at, view_up, vfov, W, H, aperture=0.0, focus_dist=10.0, out=None, stream=None):
         """castRay for every pixel (Camera.hh:59-69, Render.metal:523-527) -> (W*H, 8) CUDA tensor of trq_ray."""
         import torch
+        if out is not None:
+            _device_arg(out, "out", torch.float32, self.device, 8, at_least=W * H)
         cam = Camera()
         cam.lookFrom[:], cam.lookAt[:], cam.viewUp[:] = look_from, look_at, view_up
-        cam.vfov, cam.aspect, cam.aperture, cam.focus_dist = float(vfov), float(np.float32(W) / np.float32(H)), aperture, focus_dist
+        with np.errstate(divide="ignore", invalid="ignore"):             # H = 0 casts nothing
+            aspect = float(np.float32(W) / np.float32(H))
+        cam.vfov, cam.aspect, cam.aperture, cam.focus_dist = float(vfov), aspect, aperture, focus_dist
         rays = out if out is not None else torch.empty((W * H, 8), dtype=torch.float32, device=f"cuda:{self.device}")
         check(lib.trq_cast_rays(self._h, C.byref(cam), W, H, rays.data_ptr(), self._stream(stream)), "trq_cast_rays")
         return rays
@@ -372,6 +418,11 @@ class Scene:
     def hit_indirect(self, rays, count, any=False, out=None, sort=False, stream=None, hit16=False):
         """Scene::hit over min(*count, len(rays)) rays; `count` is a 1-element int64 CUDA tensor written by spawn_*."""
         import torch
+        _device_arg(rays, "rays", torch.float32, self.device, 8)
+        _device_arg(count, "count", torch.int64, self.device, exactly=1)
+        if out is not None:
+            _device_arg(out, "out", torch.float32, self.device, 4 if hit16 else 8, at_least=rays.shape[0])
+        _disjoint(dict(out=out), dict(rays=rays, count=count))
         flags = (L.TRACE_ANY if any else 0) | (L.SORT_RAYS if sort else 0) | (L.HIT16 if hit16 else 0)
         hits = out if out is not None else torch.empty((rays.shape[0], 4 if hit16 else 8), dtype=torch.float32, device=rays.device)
         check(lib.trq_trace_indirect(self._h, rays.data_ptr(), count.data_ptr(), rays.shape[0], flags, hits.data_ptr(),
@@ -380,7 +431,16 @@ class Scene:
 
     def _spawn(self, fn, rays, hits, count_in, seed_base, pixel_of, rng_state, extra, out, src, count, stream):
         import torch
+        _device_arg(rays, "rays", torch.float32, self.device, 8)
         n = rays.shape[0]
+        _device_arg(hits, "hits", torch.float32, self.device, 8, at_least=n)          # trq_hit rows; trq_hit16 is refused
+        for name, t, dtype, width, rows in (("count_in", count_in, torch.int64, None, None), ("pixel_of", pixel_of, torch.int32, None, n),
+                                            ("rng_state", rng_state, torch.int32, 4, n if pixel_of is None else None),
+                                            ("out", out, torch.float32, 8, n), ("src", src, torch.int32, None, n),
+                                            ("count", count, torch.int64, None, None)):
+            if t is not None:
+                _device_arg(t, name, dtype, self.device, width, at_least=rows, exactly=1 if name.startswith("count") else None)
+        _disjoint(dict(rng_state=rng_state, out=out, src=src, count=count), dict(rays=rays, hits=hits, count_in=count_in, pixel_of=pixel_of))
         dev = rays.device
         out = out if out is not None else torch.empty((n, 8), dtype=torch.float32, device=dev)
         src = src if src is not None else torch.empty(n, dtype=torch.int32, device=dev)
@@ -393,6 +453,8 @@ class Scene:
 
     def rng_frame_begin(self, rng_state, stream=None):
         """Once per frame, before the first wave: the reference's toRNG entry conversion (halves of every texel swap)."""
+        import torch
+        _device_arg(rng_state, "rng_state", torch.int32, self.device, 4)
         check(lib.trq_rng_frame_begin(self._h, rng_state.data_ptr(), rng_state.shape[0], self._stream(stream)), "trq_rng_frame_begin")
 
     def spawn_bounce(self, rays, hits, seed_base=0, count_in=None, out=None, src=None, count=None, stream=None,
@@ -425,7 +487,12 @@ class Scene:
                                       recs.ctypes.data, None), "trq_expand_hits")
             return recs
         import torch
+        _device_arg(rays, "rays", torch.float32, self.device, 8)
         n = rays.shape[0]
+        _device_arg(hits, "hits", torch.float32, self.device, 8, at_least=n)
+        if out is not None:
+            _device_arg(out, "out", torch.float32, self.device, 16, at_least=n)
+        _disjoint(dict(out=out), dict(rays=rays, hits=hits))
         recs = out if out is not None else torch.empty((n, 16), dtype=torch.float32, device=rays.device)
         st = stream if stream is not None else torch.cuda.current_stream(rays.device).cuda_stream
         check(lib.trq_expand_hits(self._h, rays.data_ptr(), hits.data_ptr(), n, 0, recs.data_ptr(), C.c_void_p(st)),
