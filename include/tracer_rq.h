@@ -373,8 +373,12 @@ int  trq_gather_destroy(trq_gather* g);
 /* Per-kernel timing for roofline reports: when enabled, every device-pointer trq_trace records CUDA
  * events (on the caller's stream) around the traversal kernel (with its ordering passes, if any) and
  * around what follows it -- the resolve pass of TRQ_KERNEL_REFLAYOUT; the packed kernel finishes its own
- * records, so resolveKernelMs is 0 for it. trq_profile_read waits for the events and returns the SUMS over
- * the launches since the last read (at most the 64 most recent) and resets. Not for TRQ_HOST_PTRS calls. */
+ * records, so resolveKernelMs is 0 for it. A trace that follows another trace of the same tree on its stream
+ * starts under that one's tail (programmatic dependent launch), and an event between the two would make it wait:
+ * such a launch is timed by the kernel itself (%globaltimer at its first CTA's start and its last CTA's exit), and
+ * these launches count with the time during which at least one of them ran. trq_profile_read waits for the
+ * launches and returns the SUMS over the launches since the last read (at most the 64 most recent) and resets.
+ * Not for TRQ_HOST_PTRS calls. */
 int  trq_profile_enable(trq_scene* scene, int on);
 int  trq_profile_read(trq_scene* scene, uint32_t* nLaunches, float* traceKernelMs, float* resolveKernelMs);
 

@@ -2,6 +2,8 @@
 # Developer tool: build an instrumented copy of the library into tools/variants/ (git-ignored, travels with gpurun).
 #   tools/build_variant.sh tl -DTRQ_STAGE_TIMELINE        ->  tools/variants/libtracer_rq_tl.so   (use with TRQ_LIB=...)
 #   tools/build_variant.sh stats -DTRQ_STATS
+#   tools/build_variant.sh tail -DTRQ_TAIL_TIMELINE       ->  per-CTA start / queue-exhausted / exit stamps (tools/tail_probe.py)
+#   tools/build_variant.sh nopdl -DTRQ_NO_PDL             ->  every trace waits for the previous kernel (tools/pdl_ab.py)
 # TRQ_VARIANT_DIR=<dir> puts the library (and its objects) there instead.
 set -e
 NAME=$1; shift

@@ -287,7 +287,20 @@ struct TraceParams {
     uint32_t       refillMin;      // refill when at least this many lanes of a warp are idle
     uint32_t       leafBatch;      // leave the interior phase when this many lanes wait at a leaf
     uint32_t       topCount;       // interior nodes [0, topCount) are staged in shared memory (TOP kernels), else 0
-    uint32_t       pad0, pad1;
+    // 1: launched as a programmatic dependent of the previous kernel on its stream, so its CTAs may start while that
+    // kernel's last rays are still being traced. Until a warp has passed griddepcontrol.wait (gate() in the kernel) it
+    // stores nothing but into `park`, and it checks every ray it read before the wait again after it.
+    uint32_t       early;
+    uint32_t       tailSlot;       // TRQ_TAIL_TIMELINE builds: the launch record of g_tail this launch fills
+    // trq_profile_enable on an early launch: {start of CTA 0, end of the last CTA} in %globaltimer ns. NULL otherwise.
+    unsigned long long* timing;
+    // an early launch's scratch for records finished before its wait: [grid warps][TRQ_PARK_ROWS][4][32] float4s, owned by
+    // this launch until it ends. NULL: the warps wait after the rays they drew first.
+    float4*             park;
+    // with park: this launch's word, 0 while it runs (its last CTA sets 1), and the previous launch's on the stream. Warps park
+    // only while the previous launch still runs; once it has ended they wait at once (griddepcontrol.wait returns).
+    volatile uint32_t*  parkRunning;
+    const volatile uint32_t* prevRunning;
     const uint32_t* order;         // optional queue order (TRQ_SORT_RAYS): queue slot -> ray index; NULL = identity
     const uint32_t* orderFlag;     // optional (automatic mode): the probe's counters; `order` applies only if batch_is_incoherent()
     const unsigned long long* nPtr;    // optional device-resident batch size (trq_trace_indirect); n is then the capacity
@@ -309,6 +322,33 @@ __device__ __forceinline__ unsigned long long ld_acquire_sys(const unsigned long
 __device__ __forceinline__ void stg4(void* p, const float4& a) {
     asm volatile("st.global.v4.f32 [%0], {%1,%2,%3,%4};" :: "l"(p), "f"(a.x), "f"(a.y), "f"(a.z), "f"(a.w) : "memory");
 }
+// 256-bit load cached in L2 only. An early launch reads its rays with it: an L1 line filled before griddepcontrol.wait
+// may hold what the previous kernel had not yet written, and a later ray of the same line would be read from it.
+__device__ __forceinline__ void ldcg8(const float4* p, float4& a, float4& b) {
+    asm volatile("ld.global.cg.v8.f32 {%0,%1,%2,%3,%4,%5,%6,%7}, [%8];"
+                 : "=f"(a.x), "=f"(a.y), "=f"(a.z), "=f"(a.w), "=f"(b.x), "=f"(b.y), "=f"(b.z), "=f"(b.w)
+                 : "l"(p) : "memory");
+}
+__device__ __forceinline__ unsigned long long global_ns() {
+    unsigned long long t;
+    asm volatile("mov.u64 %0, %%globaltimer;" : "=l"(t));
+    return t;
+}
+// Programmatic dependent launch (sm_90+). Both are no-ops in a grid that has no programmatic dependency / dependent.
+__device__ __forceinline__ void griddep_wait() { asm volatile("griddepcontrol.wait;" ::: "memory"); }
+__device__ __forceinline__ void griddep_launch_dependents() { asm volatile("griddepcontrol.launch_dependents;" ::: "memory"); }
+
+// Scratch rows per warp for the records an early launch finishes before its wait (2 KB each). A B200 warp refills about
+// every 10-20 us; the previous launch's tail is up to ~200 us (C3, profiles/r07_pdl.txt).
+#define TRQ_PARK_ROWS 8u
+
+#ifdef TRQ_TAIL_TIMELINE
+// developer instrumentation (tools/build_variant.sh <name> -DTRQ_TAIL_TIMELINE, read by tools/tail_probe.py): per CTA of
+// the last TRQ_TAIL_LAUNCHES launches, %globaltimer at {start, ~(first warp to find the queue exhausted), exit}
+#define TRQ_TAIL_LAUNCHES 8
+#define TRQ_TAIL_MAX_CTAS 4096
+__device__ unsigned long long g_tail[TRQ_TAIL_LAUNCHES][TRQ_TAIL_MAX_CTAS][3];
+#endif
 
 // trq_hit (two float4) -> trq_hit16 {t, id, u, v}; id = 0xffffffff on a miss, else front << 31 | pType << 28 | pIndex
 __device__ __forceinline__ float4 pack_hit16(const float4& o0, const float4& o1) {
@@ -430,6 +470,18 @@ trace_packed_kernel(const SceneDev S, const TraceParams P) {
     constexpr int TAG = ((((BLOCK * 8 + MINB) * 2 + (ANY ? 1 : 0)) * 2 + OUT) * 2 + (TOP ? 1 : 0)) * 4 + LEAVES;
     constexpr bool TRIS = LEAVES == LEAVES_TRI, SQCUBE = LEAVES == LEAVES_ALL;
 
+    // The next trace on this stream may start as this grid's CTAs retire. An early grid lets its own dependent start only
+    // once its predecessor has finished (in gate()), so that at most two traces overlap: the queue heads of the ring
+    // stay one launch's each.
+    bool gated = P.early != 0;                       // this warp has not passed griddepcontrol.wait yet
+    bool drew = false;                               // this warp has drawn its first rays
+    if (!gated) griddep_launch_dependents();
+    if (P.timing && blockIdx.x == 0 && threadIdx.x == 0) P.timing[0] = global_ns();
+    if (P.park && blockIdx.x == 0 && threadIdx.x == 0) { *P.parkRunning = 1u; __threadfence(); }
+#ifdef TRQ_TAIL_TIMELINE
+    unsigned long long* const tail = blockIdx.x < TRQ_TAIL_MAX_CTAS ? g_tail[P.tailSlot % TRQ_TAIL_LAUNCHES][blockIdx.x] : nullptr;
+    if (tail && threadIdx.x == 0) tail[0] = global_ns();
+#endif
     if (TOP) packed::stage_top_of_tree(reinterpret_cast<float4*>(smem_u32), S.topSoA, P.topCount, S.topStride, &topBarrier);
 
     const uint64_t N = live_count(P.n, P.nPtr);
@@ -445,11 +497,10 @@ trace_packed_kernel(const SceneDev S, const TraceParams P) {
     // registers (ro, range_y) stay untouched between finish() and flush().
     bool pending = false;
     auto finish = [&]() { active = false; pending = true; };
-    auto flush = [&]() {
-        if (pending) {
+    auto record = [&](float4& o0, float4& o1) {                       // the finished ray's record
             const uint32_t best = cold[COLD_BEST * BLOCK];
             const bool hit = (range_y < coldf[COLD_TEST_T * BLOCK]) && best != 0xffffffffu;   // Render.hh:251
-            float4 o0 = make_float4(0.f, 0.f, 0.f, 0.f), o1 = o0;
+            o0 = make_float4(0.f, 0.f, 0.f, 0.f); o1 = o0;
             if (hit) {
                 const float u = coldf[COLD_U * BLOCK], v = coldf[COLD_V * BLOCK];
                 const f3 d = make_f3(coldf[COLD_DX * BLOCK], coldf[COLD_DY * BLOCK], coldf[COLD_DZ * BLOCK]);
@@ -469,9 +520,36 @@ trace_packed_kernel(const SceneDev S, const TraceParams P) {
                     o0 = o[0]; o1 = o[1];
                 }
             }
+    };
+    auto flush = [&]() {
+        if (pending) {
+            float4 o0, o1;
+            record(o0, o1);
             emit_record<OUT>(P, cold[COLD_RAY * BLOCK], o0, o1);
             pending = false;
         }
+    };
+    // Before its wait an early warp may store nothing where the caller can see it: the previous kernel may still read or
+    // write those buffers. It parks the records of its finished rays instead, one row of 32 per refill, in this launch's own
+    // scratch (P.park): [warp][row][quarter][lane] float4s = {ox, oy, oz, tmax}, {dx, dy, dz, bits(ray index)}, the record's
+    // two halves; ray index ~0: no ray. After the wait, gate() stores each parked record whose ray is still what was traced.
+    const uint64_t parkWarp = ((uint64_t)blockIdx.x * (BLOCK / 32) + (threadIdx.x >> 5)) * TRQ_PARK_ROWS;
+    uint32_t parked = 0;                             // rows this warp has parked
+    uint32_t redo = 0;                               // this lane's parked rows whose ray changed: traced again after the wait
+    auto park = [&]() {
+        float4* const row = P.park + (parkWarp + parked) * 128u + lane;
+        float4 q1 = make_float4(0.f, 0.f, 0.f, __uint_as_float(0xffffffffu));
+        if (pending) {
+            float4 o0, o1;
+            record(o0, o1);
+            stg4(row, make_float4(ro.x, ro.y, ro.z, coldf[COLD_TEST_T * BLOCK]));
+            q1 = make_float4(coldf[COLD_DX * BLOCK], coldf[COLD_DY * BLOCK], coldf[COLD_DZ * BLOCK], __uint_as_float(cold[COLD_RAY * BLOCK]));
+            stg4(row + 64, o0);
+            stg4(row + 96, o1);
+            pending = false;
+        }
+        stg4(row + 32, q1);
+        ++parked;
     };
     auto push = [&](uint32_t ref) { stk[sp * BLOCK] = ref; ++sp; };
     auto pop = [&]() {
@@ -486,43 +564,117 @@ trace_packed_kernel(const SceneDev S, const TraceParams P) {
         unsigned long long base = 0;
         if (lane == 0) base = atomicAdd(&P.queue->head, (unsigned long long)want);
         base = __shfl_sync(0xffffffffu, base, 0);
-        if (base + (unsigned long long)want >= N) exhausted = true;
+        if (base + (unsigned long long)want >= N) {
+#ifdef TRQ_TAIL_TIMELINE
+            if (tail && lane == 0 && !exhausted) atomicMax(&tail[1], ~global_ns());     // stored inverted: 0 = never
+#endif
+            exhausted = true;
+        }
         const uint64_t slot = base + (uint64_t)__popc(mask & ((1u << lane) - 1u));
         if (!((mask >> lane) & 1u) || slot >= N) return ~0ull;
         return useOrder ? (uint64_t)__ldg(P.order + slot) : slot;
     };
+    // Gives this lane ray `idx` (r0, r1: its trq_ray). A ray that misses the root is finished at once: its (all-zero)
+    // record is stored now, or -- `defer`, in an early launch -- left pending for flush(), like any finished ray.
+    auto start = [&](uint32_t idx, const float4& r0, const float4& r1, bool defer) {
+        const RayCtx ray = make_ray_ctx(r0.x, r0.y, r0.z, r1.x, r1.y, r1.z);
+        ro = ray.o; rinv = ray.inv;
+        range_y = r0.w;                                                // Render.hh:143  range_t = (FLT_MIN, test_t)
+        sp = 0;
+        const f3 rootMin = make_f3(S.rootMin[0], S.rootMin[1], S.rootMin[2]);
+        const f3 rootMax = make_f3(S.rootMax[0], S.rootMax[1], S.rootMax[2]);
+        const bool root = box_hit(rootMin, rootMax, ray, FLT_MIN, range_y);    // :145
+        if (root || defer) {
+            coldf[COLD_TEST_T * BLOCK] = r0.w;
+            cold[COLD_BEST * BLOCK] = 0xffffffffu;
+            coldf[COLD_U * BLOCK] = 0.0f; coldf[COLD_V * BLOCK] = 0.0f;
+            cold[COLD_AUX * BLOCK] = 0u;
+            cold[COLD_RAY * BLOCK] = idx;
+            coldf[COLD_DX * BLOCK] = r1.x; coldf[COLD_DY * BLOCK] = r1.y; coldf[COLD_DZ * BLOCK] = r1.z;
+        }
+        if (root) { cur = S.rootRef; active = true; }
+        else if (defer) pending = true;
+        else {
+            const float4 z = make_float4(0.f, 0.f, 0.f, 0.f);
+            emit_record<OUT>(P, idx, z, z);
+        }
+    };
+    // An early warp's wait for the previous kernel on the stream (it returns once that grid has finished and its stores
+    // are visible). The rays this warp drew before it may have been read before the previous kernel wrote them (a caller's
+    // kernel that rewrites the batch, or a batch that is the previous trace's output): every lane reads its ray again and
+    // starts it over if any of the seven words the traversal uses (flags is reserved) has changed.
+    auto gate = [&]() {
+        griddep_wait();
+        griddep_launch_dependents();
+        gated = false;
+        for (uint32_t r = 0; r < parked; ++r) {
+            const float4* const row = P.park + (parkWarp + r) * 128u + lane;
+            const float4 q1 = __ldcg(row + 32);
+            const uint32_t idx = __float_as_uint(q1.w);
+            if (idx == 0xffffffffu) continue;
+            const float4 q0 = __ldcg(row);
+            float4 r0, r1;
+            ldcg8(reinterpret_cast<const float4*>(P.rays + idx), r0, r1);
+            const bool same = __float_as_uint(r0.x) == __float_as_uint(q0.x) && __float_as_uint(r0.y) == __float_as_uint(q0.y) &&
+                              __float_as_uint(r0.z) == __float_as_uint(q0.z) && __float_as_uint(r0.w) == __float_as_uint(q0.w) &&
+                              __float_as_uint(r1.x) == __float_as_uint(q1.x) && __float_as_uint(r1.y) == __float_as_uint(q1.y) &&
+                              __float_as_uint(r1.z) == __float_as_uint(q1.z);
+            if (same) emit_record<OUT>(P, idx, __ldcg(row + 64), __ldcg(row + 96));
+            else      redo |= 1u << r;
+        }
+        if (active || pending) {
+            const uint32_t idx = cold[COLD_RAY * BLOCK];
+            float4 r0, r1;
+            ldcg8(reinterpret_cast<const float4*>(P.rays + idx), r0, r1);
+            const bool same = __float_as_uint(r0.x) == __float_as_uint(ro.x) && __float_as_uint(r0.y) == __float_as_uint(ro.y) &&
+                              __float_as_uint(r0.z) == __float_as_uint(ro.z) && __float_as_uint(r0.w) == cold[COLD_TEST_T * BLOCK] &&
+                              __float_as_uint(r1.x) == cold[COLD_DX * BLOCK] && __float_as_uint(r1.y) == cold[COLD_DY * BLOCK] &&
+                              __float_as_uint(r1.z) == cold[COLD_DZ * BLOCK];
+            if (!same) { active = false; pending = false; start(idx, r0, r1, true); }
+        }
+    };
 
     for (;;) {
         // ---- refill idle lanes from the global queue: one atomic per warp ----
-        const unsigned idleMask = __ballot_sync(0xffffffffu, !active);
-        if (!exhausted && (idleMask == 0xffffffffu || __popc(idleMask) >= (int)P.refillMin)) {
-            const uint64_t idx = draw(idleMask);
-            flush();
+        unsigned idleMask = __ballot_sync(0xffffffffu, !active);
+        bool more = !exhausted || __any_sync(0xffffffffu, redo != 0u);
+        bool refill = more && (idleMask == 0xffffffffu || __popc(idleMask) >= (int)P.refillMin);
+        // an early warp parks its finished rays' records while it has scratch rows left, then waits
+        if (refill && gated && drew &&
+            (P.park == nullptr || parked == TRQ_PARK_ROWS || __shfl_sync(0xffffffffu, lane == 0 ? *P.prevRunning : 0u, 0) == 0u)) {
+            gate();
+            idleMask = __ballot_sync(0xffffffffu, !active);
+            more = !exhausted || __any_sync(0xffffffffu, redo != 0u);
+            refill = more && (idleMask == 0xffffffffu || __popc(idleMask) >= (int)P.refillMin);
+        }
+        if (refill) {
+            drew = true;
+            const bool again = !active && redo != 0u;          // an idle lane with a parked ray that changed traces it first
+            const unsigned drawMask = idleMask & ~__ballot_sync(0xffffffffu, again);
+            uint64_t idx = ~0ull;
+            if (drawMask != 0u && !exhausted) idx = draw(drawMask);
+            if (gated) { if (__any_sync(0xffffffffu, pending)) park(); }
+            else flush();
+            if (again) {
+                const uint32_t r = (uint32_t)__ffs(redo) - 1u;
+                redo &= redo - 1u;
+                idx = __float_as_uint(__ldcg(P.park + (parkWarp + r) * 128u + 32u + lane).w);
+            }
             if (idx != ~0ull) {
-                float4 r0, r1;
-                ldg8(reinterpret_cast<const float4*>(P.rays + idx), r0, r1);          // trq_ray is one 32-byte record
-                const RayCtx ray = make_ray_ctx(r0.x, r0.y, r0.z, r1.x, r1.y, r1.z);
-                ro = ray.o; rinv = ray.inv;
-                range_y = r0.w;                                        // Render.hh:143  range_t = (FLT_MIN, test_t)
-                sp = 0;
-                const f3 rootMin = make_f3(S.rootMin[0], S.rootMin[1], S.rootMin[2]);
-                const f3 rootMax = make_f3(S.rootMax[0], S.rootMax[1], S.rootMax[2]);
-                if (box_hit(rootMin, rootMax, ray, FLT_MIN, range_y)) {            // :145
-                    coldf[COLD_TEST_T * BLOCK] = r0.w;
-                    cold[COLD_BEST * BLOCK] = 0xffffffffu;
-                    coldf[COLD_U * BLOCK] = 0.0f; coldf[COLD_V * BLOCK] = 0.0f;
-                    cold[COLD_AUX * BLOCK] = 0u;
-                    cold[COLD_RAY * BLOCK] = (uint32_t)idx;
-                    coldf[COLD_DX * BLOCK] = r1.x; coldf[COLD_DY * BLOCK] = r1.y; coldf[COLD_DZ * BLOCK] = r1.z;
-                    cur = S.rootRef; active = true;
-                } else {
-                    const float4 z = make_float4(0.f, 0.f, 0.f, 0.f);
-                    emit_record<OUT>(P, (uint32_t)idx, z, z);
-                }
+                float4 r0, r1;                                         // trq_ray is one 32-byte record
+                if (P.early) ldcg8(reinterpret_cast<const float4*>(P.rays + idx), r0, r1);
+                else         ldg8(reinterpret_cast<const float4*>(P.rays + idx), r0, r1);
+                start((uint32_t)idx, r0, r1, gated);
             }
         }
         const unsigned actMask = __ballot_sync(0xffffffffu, active);
-        if (actMask == 0u) { if (exhausted) { flush(); break; } else continue; }
+        if (actMask == 0u) {
+            if (!exhausted) continue;
+            if (gated) gate();
+            if (__any_sync(0xffffffffu, active || redo != 0u)) continue;   // rays that changed start over
+            flush();
+            break;
+        }
 
         // ---- traverse until enough lanes have retired to make a refill worthwhile ----
         // Two phases per round so that the (rarer) leaf code is not issued on every interior step:
@@ -618,14 +770,19 @@ trace_packed_kernel(const SceneDev S, const TraceParams P) {
         } while (__popc(__ballot_sync(0xffffffffu, active)) > keepGoing);
     }
 
-    // ---- epilogue: the last CTA to leave re-arms the queue head for the next launch that draws it
+    // ---- epilogue (every warp has passed gate()): the last CTA to leave re-arms the queue head for the next launch that draws it
     __syncthreads();
     if (threadIdx.x == 0) {
         const unsigned int prev = atomicAdd(&P.queue->done, 1u);
         if (prev == gridDim.x - 1) {
+            if (P.timing) P.timing[1] = global_ns();
+            if (P.park) *P.parkRunning = 0u;
             P.queue->head = 0ull;
             P.queue->done = 0u;
         }
+#ifdef TRQ_TAIL_TIMELINE
+        if (tail) tail[2] = global_ns();
+#endif
     }
 }
 

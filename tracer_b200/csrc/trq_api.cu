@@ -8,6 +8,7 @@
 
 #include <cuda_runtime.h>
 
+#include <algorithm>
 #include <atomic>
 #include <chrono>
 #include <cstdio>
@@ -176,11 +177,28 @@ struct trq_scene {
     cudaStream_t stageStream[kStageBufs] = {};   // one stream per staging buffer: copy in, trace, copy out in stream order
     bool stageReady = false;
     uint64_t stageSeq = 0;        // chunks ever staged (ring position)
-    // optional per-kernel timing (trq_profile_enable): events around the trace and resolve kernels
+    // optional per-kernel timing (trq_profile_enable): events around the trace and resolve kernels; an early launch (below)
+    // is timed by the kernel itself instead, since an event recorded between two kernels makes the second wait for the first
     std::mutex profMutex;
     bool profile = false;
     cudaEvent_t evProf[kProfRing][3] = {};
+    unsigned long long* d_profStamps = nullptr;   // [kProfRing][2]: {start, end} of an early launch (TraceParams::timing)
+    bool profByKernel[kProfRing] = {};
     uint32_t profHead = 0, profCount = 0;
+    // A trace has been launched on the tree as it now is (cleared by a refit or a rebuild): the next trace may be an early
+    // launch, one whose CTAs start while the previous kernel on its stream is still running (launch_trace).
+    std::atomic<bool> treeTraced{false};
+    uint32_t tailSeq = 0;         // TRQ_TAIL_TIMELINE builds: launches since trq_debug_tail's reset
+    // Scratch in which early launches park the records they finish before their wait (TraceParams::park): two halves, taken
+    // in turn by the early launches on one stream (the first that asks). Two launches that overlap are consecutive on their
+    // stream, so they never share a half; early launches on other streams do without.
+    std::mutex parkMutex;
+    float4* d_park = nullptr;
+    uint32_t* d_parkRunning = nullptr;   // [2]: one word per half (TraceParams::parkRunning)
+    size_t parkHalf = 0;
+    cudaStream_t parkStream = nullptr;
+    bool parkBound = false;
+    uint32_t parkSeq = 0;
 };
 
 namespace {
@@ -207,6 +225,9 @@ void free_scene(trq_scene* s) {
     }
     for (int k = 0; k < kProfRing; ++k)
         for (int j = 0; j < 3; ++j) if (s->evProf[k][j]) cudaEventDestroy(s->evProf[k][j]);
+    cudaFree(s->d_profStamps);
+    cudaFree(s->d_park);
+    cudaFree(s->d_parkRunning);
     delete s;
 }
 
@@ -350,11 +371,41 @@ int launch_trace(trq_scene* s, const trq_ray* d_rays, uint64_t n, uint32_t flags
     }
     const bool any = (flags & TRQ_TRACE_ANY) != 0;
     const SceneDev dev = scene_dev(s);
+    // TRQ_SORT_RAYS: counting sort of ray indices by (origin cell, direction octant); stream-ordered scratch. The flag is the
+    // caller's word that the batch is incoherent. Without it, scenes whose packed tree is more than twice the L2 (where an
+    // incoherent batch runs at DRAM latency: C5 400 vs 990 Mrays/s) get the AUTOMATIC mode for batches of >= 1 M rays: a
+    // probe over 64 K sampled rays measures how many neighbouring rays share a key, and the queue is ordered only if fewer
+    // than half do -- decided on the device, no host round trip. TRQ_NO_SORT opts out; TRQ_SORT_RAYS=0/1 in the environment overrides
+    // both (experiments), TRQ_AUTO_SORT=1 treats every scene as large (tests).
+    static const int sortEnv = [] { const char* e = getenv("TRQ_SORT_RAYS"); return e ? atoi(e) : -1; }();
+    const char* autoStr = getenv("TRQ_AUTO_SORT");               // read per call: the tests switch it inside one process
+    const int autoEnv = autoStr ? atoi(autoStr) : -1;
+    const bool sortRays = sortEnv >= 0 ? (sortEnv != 0) : ((flags & TRQ_SORT_RAYS) != 0);
+    const bool autoSort = !sortRays && sortEnv < 0 && !(flags & TRQ_NO_SORT) && !tileDone && n >= (1ull << 20) &&
+                          (autoEnv >= 0 ? autoEnv != 0 : s->tree.largeTree);
+    const bool ordered = (sortRays && n >= 65536) || autoSort;
+    cudaStreamCaptureStatus capture = cudaStreamCaptureStatusNone;
+    TRQ_CUDA(cudaStreamIsCapturing(st, &capture));
+    // Early launch (programmatic dependent launch): the packed kernel's CTAs may take the SMs that the previous kernel on
+    // this stream leaves as its last, longest rays finish, instead of waiting for its last CTA (profiles/r07_pdl.txt).
+    // Only for a plain eager launch of the packed kernel on a tree that has been traced as it is: not under capture (a graph
+    // replay may run beside anything), not for the ordered, indirect or gather paths (their inputs are written by the kernels
+    // just before them) and not right after a refit or rebuild.
+    bool early = false;
+#ifndef TRQ_NO_PDL
+    early = !(flags & TRQ_KERNEL_REFLAYOUT) && !ordered && !nPtr && !tileDone && capture == cudaStreamCaptureStatusNone &&
+            s->treeTraced.load();
+#endif
+    s->treeTraced.store(true);
     cudaEvent_t* prof = nullptr;
+    unsigned long long* stamps = nullptr;
     if (s->profile) {
         std::lock_guard<std::mutex> lock(s->profMutex);
         if (s->profile) {
-            prof = s->evProf[s->profHead % kProfRing];
+            const uint32_t slot = s->profHead % kProfRing;
+            prof = s->evProf[slot];
+            s->profByKernel[slot] = early;
+            if (early) { stamps = s->d_profStamps + 2 * slot; prof = nullptr; }
             s->profHead++; if (s->profCount < kProfRing) s->profCount++;
         }
     }
@@ -397,8 +448,6 @@ int launch_trace(trq_scene* s, const trq_ray* d_rays, uint64_t n, uint32_t flags
         // last CTA re-arms the one it used). A launch captured into a CUDA graph is fixed in the graph and may be replayed at
         // any later time, beside any other launch: it gets a head of its own, allocated, zeroed and freed in stream order
         // around the kernel at every replay. (A per-launch memset for eager launches too costs ~1 % on C1 / C2.)
-        cudaStreamCaptureStatus capture = cudaStreamCaptureStatusNone;
-        TRQ_CUDA(cudaStreamIsCapturing(st, &capture));
         QueueHead* ownHead = nullptr;
         if (capture != cudaStreamCaptureStatusNone) {
             TRQ_CUDA(cudaMallocFromPoolAsync((void**)&ownHead, sizeof(QueueHead), s->scratchPool, st));
@@ -409,20 +458,12 @@ int launch_trace(trq_scene* s, const trq_ray* d_rays, uint64_t n, uint32_t flags
         P.topCount = K.top ? cs.topCount : 0;
         P.order = nullptr; P.nPtr = nPtr;
         P.tileDone = tileDone; P.tileShift = tileShift;
-        // TRQ_SORT_RAYS: counting sort of ray indices by (origin cell, direction octant); stream-ordered scratch. The flag is the
-        // caller's word that the batch is incoherent. Without it, scenes whose packed tree is more than twice the L2 (where an
-        // incoherent batch runs at DRAM latency: C5 400 vs 990 Mrays/s) get the AUTOMATIC mode for batches of >= 1 M rays: a
-        // probe over 64 K sampled rays measures how many neighbouring rays share a key, and the queue is ordered only if fewer
-        // than half do -- decided on the device, no host round trip. TRQ_NO_SORT opts out; TRQ_SORT_RAYS=0/1 in the environment overrides
-        // both (experiments), TRQ_AUTO_SORT=1 treats every scene as large (tests).
-        static const int sortEnv = [] { const char* e = getenv("TRQ_SORT_RAYS"); return e ? atoi(e) : -1; }();
-        const char* autoStr = getenv("TRQ_AUTO_SORT");           // read per call: the tests switch it inside one process
-        const int autoEnv = autoStr ? atoi(autoStr) : -1;
-        const bool sortRays = sortEnv >= 0 ? (sortEnv != 0) : ((flags & TRQ_SORT_RAYS) != 0);
-        const bool autoSort = !sortRays && sortEnv < 0 && !(flags & TRQ_NO_SORT) && !tileDone && n >= (1ull << 20) &&
-                              (autoEnv >= 0 ? autoEnv != 0 : s->tree.largeTree);
+        P.early = early ? 1u : 0u; P.timing = stamps;
+#ifdef TRQ_TAIL_TIMELINE
+        P.tailSlot = s->tailSeq++;
+#endif
         uint32_t* scratch = nullptr;
-        if ((sortRays && n >= 65536) || autoSort) {
+        if (ordered) {
             const size_t words = (size_t)TRQ_SORT_BINS + 4 + 2 * (size_t)n;      // hist | ctrl | keys | order
             TRQ_CUDA(cudaMallocFromPoolAsync((void**)&scratch, words * sizeof(uint32_t), s->scratchPool, st));
             uint32_t* hist = scratch; uint32_t* ctrl = scratch + TRQ_SORT_BINS; uint32_t* keys = ctrl + 4; uint32_t* order = keys + n;
@@ -439,7 +480,43 @@ int launch_trace(trq_scene* s, const trq_ray* d_rays, uint64_t n, uint32_t flags
             P.orderFlag = decide;
         }
         void* args[2] = {(void*)&dev, (void*)&P};
-        TRQ_CUDA(cudaLaunchKernel(K.fn[s->tree.leaves][any ? 1 : 0][hit16 ? 1 : 0], dim3((unsigned)grid), dim3((unsigned)K.block), args, cs.smem, st));
+        const void* fn = K.fn[s->tree.leaves][any ? 1 : 0][hit16 ? 1 : 0];
+        std::unique_lock<std::mutex> parkLock;                  // held until the launch: halves alternate in stream order
+        if (early) {
+            parkLock = std::unique_lock<std::mutex>(s->parkMutex);
+            if (!s->parkBound && cudaMalloc((void**)&s->d_parkRunning, 2 * sizeof(uint32_t)) == cudaSuccess &&
+                cudaMemset(s->d_parkRunning, 0, 2 * sizeof(uint32_t)) == cudaSuccess) {
+                s->parkStream = st; s->parkBound = true;
+            }
+            cudaGetLastError();
+            const size_t half = (size_t)grid * (K.block / 32) * TRQ_PARK_ROWS * 128u * sizeof(float4);
+            if (s->parkBound && s->parkStream == st && half > s->parkHalf) {
+                if (s->d_park) {                                // the launches that use the old halves are on this stream
+                    TRQ_CUDA(cudaStreamSynchronize(st));
+                    TRQ_CUDA(cudaFree(s->d_park));
+                    s->d_park = nullptr; s->parkHalf = 0;
+                }
+                if (cudaMalloc((void**)&s->d_park, 2 * half) == cudaSuccess) s->parkHalf = half;
+                else { cudaGetLastError(); s->d_park = nullptr; }   // without scratch the warps wait after their first rays
+            }
+            if (s->parkBound && s->parkStream == st && s->d_park) {
+                const uint32_t h = s->parkSeq++ & 1u;
+                P.park = reinterpret_cast<float4*>(reinterpret_cast<uint8_t*>(s->d_park) + h * s->parkHalf);
+                P.parkRunning = s->d_parkRunning + h;
+                P.prevRunning = s->d_parkRunning + (h ^ 1u);
+            }
+        }
+        if (early) {
+            cudaLaunchAttribute attr[1];
+            attr[0].id = cudaLaunchAttributeProgrammaticStreamSerialization;
+            attr[0].val.programmaticStreamSerializationAllowed = 1;
+            cudaLaunchConfig_t lc = {};
+            lc.gridDim = dim3((unsigned)grid); lc.blockDim = dim3((unsigned)K.block); lc.dynamicSmemBytes = cs.smem; lc.stream = st;
+            lc.attrs = attr; lc.numAttrs = 1;
+            TRQ_CUDA(cudaLaunchKernelExC(&lc, fn, args));
+        } else {
+            TRQ_CUDA(cudaLaunchKernel(fn, dim3((unsigned)grid), dim3((unsigned)K.block), args, cs.smem, st));
+        }
         g_launches++;
         if (ownHead) TRQ_CUDA(cudaFreeAsync(ownHead, st));
         if (scratch) TRQ_CUDA(cudaFreeAsync(scratch, st));
@@ -566,6 +643,23 @@ int trq_device_count(void) {
 }
 
 uint64_t trq_launch_count(void) { return g_launches.load(); }
+
+#ifdef TRQ_TAIL_TIMELINE
+// tools/tail_probe.py: out <- the stamps of the last TRQ_TAIL_LAUNCHES packed-kernel launches ([launch % 8][CTA][start,
+// ~first exhausted, exit]); reset: clear them and number this scene's launches from 0 again
+int trq_debug_tail(trq_scene* s, unsigned long long* out, int reset) {
+    TRQ_CUDA(cudaDeviceSynchronize());
+    if (out) TRQ_CUDA(cudaMemcpyFromSymbol(out, trq::g_tail, sizeof(trq::g_tail)));
+    if (reset) {
+        void* p = nullptr;
+        TRQ_CUDA(cudaGetSymbolAddress(&p, trq::g_tail));
+        TRQ_CUDA(cudaMemset(p, 0, sizeof(trq::g_tail)));
+        TRQ_CUDA(cudaDeviceSynchronize());
+        s->tailSeq = 0;
+    }
+    return TRQ_OK;
+}
+#endif
 
 #ifdef TRQ_STATS
 void trq_debug_stats(unsigned long long* out, int reset) {
@@ -763,6 +857,7 @@ int refit_scene(trq_scene* s, const trq_scene_desc* c, uint32_t flags, const cha
     DeviceGuard guard(s->device);
     if (!guard.ok) return trq::fail(TRQ_ERR_CUDA, "cudaSetDevice(%d) failed", s->device);
     TRQ_CUDA(cudaDeviceSynchronize());                           // traces in flight still read the old boxes and records
+    s->treeTraced.store(false);                                  // the next trace reads the new tree: no early launch
     PackedTree& t = s->tree;
     const SceneRecords& r = s->rec;
     const uint32_t n = t.info.nNode;
@@ -916,6 +1011,7 @@ int trq_scene_rebuild(trq_scene* s, const void* triList, uint32_t nVert, uint32_
     if ((rc = pack_tree(t, r, s->device)) != TRQ_OK) return bail(rc);
 
     // commit: the new tree (and vertices) in, the old ones out
+    s->treeTraced.store(false);
     std::swap(s->tree, t);
     t.release();
     if (newVerts) { pool_free(s->rec.verts); s->rec.verts = newVerts; }
@@ -977,6 +1073,7 @@ int trq_profile_enable(trq_scene* s, int on) {
     if (on && !s->evProf[0][0]) {
         for (int k = 0; k < kProfRing; ++k)
             for (int j = 0; j < 3; ++j) TRQ_CUDA(cudaEventCreate(&s->evProf[k][j]));
+        TRQ_CUDA(cudaMalloc((void**)&s->d_profStamps, 2 * kProfRing * sizeof(unsigned long long)));
     }
     std::lock_guard<std::mutex> lock(s->profMutex);
     s->profile = on != 0;
@@ -989,7 +1086,31 @@ int trq_profile_read(trq_scene* s, uint32_t* nLaunches, float* traceMs, float* r
     DeviceGuard guard(s->device);
     std::lock_guard<std::mutex> lock(s->profMutex);
     *nLaunches = 0; *traceMs = 0.0f; *resolveMs = 0.0f;
+    // early launches: the time during which at least one of them ran (they overlap their predecessors by design)
+    std::vector<std::pair<unsigned long long, unsigned long long>> spans;
     for (uint32_t k = 0; k < s->profCount; ++k) {
+        if (!s->profByKernel[(s->profHead - 1 - k) % kProfRing]) continue;
+        if (spans.empty()) {
+            TRQ_CUDA(cudaDeviceSynchronize());
+            std::vector<unsigned long long> h(2 * kProfRing);
+            TRQ_CUDA(cudaMemcpy(h.data(), s->d_profStamps, h.size() * sizeof(unsigned long long), cudaMemcpyDeviceToHost));
+            for (uint32_t j = 0; j < s->profCount; ++j) {
+                const uint32_t slot = (s->profHead - 1 - j) % kProfRing;
+                if (s->profByKernel[slot]) spans.emplace_back(h[2 * slot], h[2 * slot + 1]);
+            }
+            std::sort(spans.begin(), spans.end());
+            unsigned long long covered = 0, reach = 0;
+            for (const auto& sp : spans) {
+                const unsigned long long from = sp.first > reach ? sp.first : reach;
+                if (sp.second > from) covered += sp.second - from;
+                if (sp.second > reach) reach = sp.second;
+            }
+            *traceMs += (float)(covered * 1e-6);
+        }
+        (*nLaunches)++;
+    }
+    for (uint32_t k = 0; k < s->profCount; ++k) {
+        if (s->profByKernel[(s->profHead - 1 - k) % kProfRing]) continue;
         cudaEvent_t* ev = s->evProf[(s->profHead - 1 - k) % kProfRing];
         TRQ_CUDA(cudaEventSynchronize(ev[2]));
         float a = 0.0f, b = 0.0f;
